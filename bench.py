@@ -16,6 +16,7 @@ The line also carries the dominant kernel's roofline (HBM-write as BASELINE asks
 that actually binds it) and the reference CPU tools timed on this box's cores (cpu_baseline).
 """
 import argparse
+import atexit
 import json
 import os
 import pathlib
@@ -133,6 +134,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "50",
                                           "-i", ",".join(str(g) for g in self.gpus)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
             threading.Thread(target=self._read, daemon=True).start()
+            atexit.register(self.proc.terminate)          # the sampler loops until stopped: not past an early exit
         except OSError:
             self.proc = None
 
@@ -238,6 +240,18 @@ def bind_near_gpu(index):
         return {"bound": False, "why": type(e).__name__}
 
 
+def sample_streams(buf, ns, k, seed):
+    """A fixed, seeded choice of k streams of a dense batch (stream i at i * max(ns), as vs_synth_batch lays it out without
+    offsets): {"pcm": their samples one after the other as float32, "streams": their indices, "nsamples": their lengths}."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(seed).choice(len(ns), size=min(k, len(ns)), replace=False))
+    stride = int(ns.max())
+    t = torch.as_tensor(buf)
+    pcm = torch.cat([t[int(i) * stride: int(i) * stride + int(ns[i])] for i in idx]).float().cpu().numpy()
+    return {"pcm": pcm, "streams": idx.astype(np.float64), "nsamples": ns[idx].astype(np.float64)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -247,7 +261,12 @@ def main():
     ap.add_argument("--ref-streams", type=int, default=1024, help="streams per step of the reference arm")
     ap.add_argument("--cpu-sample", type=int, default=2048, help="streams of the cpu_baseline sample (0 = skip)")
     ap.add_argument("--no-other", action="store_true", help="skip the cfg3 / cfg5 workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the PCM of the last timed step of each workload (a seeded sample of its streams, float32) "
+                         "to DIR/<workload>_{pcm,streams,nsamples}.npy; rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -322,6 +341,10 @@ def main():
     e1.record(stream)
     barrier()
     dev_ms = e0.elapsed_time(e1) / args.steps
+    # taken before any later leg reuses the output buffers; 56 MB in all with the cfg3 and cfg5 samples below
+    dumps = {}
+    if args.dump_outputs:
+        dumps["cfg2"] = sample_streams(dev_out, ns, 256, seed=0)
     t = ctx.timing()
     launches += t["launches"] * args.steps
     warm = t["warmup_samples"]
@@ -409,6 +432,8 @@ def main():
         ms3 = e0.elapsed_time(e1) / k3
         t3 = ctx.timing()
         launches += t3["launches"] * (k3 + 5)
+        if args.dump_outputs:
+            dumps["cfg3"] = sample_streams(out3, api.flow_nsamples(p3), 128, seed=0)
         del out3
         # configs[4]: 1 M utterances x 1 s, 131 072 per GPU, PCM streamed to pinned host memory: eight calls of
         # 16 384 utterances alternate between two pinned buffers, PCIe inside the timed region
@@ -429,6 +454,8 @@ def main():
         sweep()
         ms5 = (time.perf_counter() - t0) * 1e3
         barrier()
+        if args.dump_outputs:                # the sweep's last call: parts[-1] into ring[(nsub - 1) & 1]
+            dumps["cfg5"] = sample_streams(ring[(nsub - 1) & 1], api.flow_nsamples(parts[-1][0]), 128, seed=0)
         t5 = ctx.timing()
         launches += t5["launches"] * nsub * 2
         ctx.set_option(api.OPT_ASYNC_HOST, 0)
@@ -474,6 +501,12 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        out_dir = pathlib.Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for w, arrays in dumps.items():
+            for name, a in arrays.items():
+                np.save(out_dir / f"{w}_{name}.npy", a)
 
     total_samples = samples_per_step * world
     value = total_samples / (dev_ms * 1e-3) / 1e6
