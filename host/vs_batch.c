@@ -5,7 +5,12 @@
  * Each manifest line describes one voice with the reference tools' own flags:
  *   <out.wav> <vowel> <seed> [flowgen_shimmer flags, e.g. -d 1 -f 120 -j 1 -s 3] [-V gain] [-P pre]
  * which is what   VS_SEED=<seed> flowgen_shimmer -o tmp.wav <flags>; vowel -i tmp.wav -o <out.wav> -v <vowel>
- * would produce, without the intermediate file. */
+ * would produce, without the intermediate file.
+ *
+ * <vowel> is a preset key ('a','i','u','1'..'7') or a formant tract  f:F1/B1,F2/B2,...  (Hz, 1 to 11 formants),
+ * built at the voice's own sampling rate (-r) by vs_tract_from_formants.  A slab with formant voices renders through
+ * vs_synth_batch_tract (presets become tracts, identical (spec, rate) pairs share one entry, at most VS_MAX_TRACTS
+ * distinct tracts per slab); a slab without any takes vs_synth_batch. */
 #include <pthread.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -17,6 +22,28 @@
 #include "vs_wav.h"
 
 #define MAXTOK 64
+#define MAXFORMANTS 11
+
+/* "f:F1/B1,F2/B2,..." -> den; 0, or -1 for a malformed spec, or the VS_E* code of vs_tract_from_formants */
+static int formant_tract(const char *spec, int32_t fs, double den[23])
+{
+    float F[MAXFORMANTS + 1], B[MAXFORMANTS + 1];
+    int k = 0;
+    const char *c = spec + 2;
+    while (*c) {
+        char *e;
+        if (k > MAXFORMANTS) return -1;
+        F[k] = strtof(c, &e);
+        if (e == c || *e != '/') return -1;
+        c = e + 1;
+        B[k] = strtof(c, &e);
+        if (e == c || (*e != ',' && *e != 0)) return -1;
+        k++;
+        c = *e ? e + 1 : e;
+    }
+    if (k == 0) return -1;
+    return vs_tract_from_formants(F, B, k, fs, den) ? -2 : 0;
+}
 
 /* ---- writer pool: a slab of voices is handed over as one job; the threads pull voices off it ---------- */
 typedef struct {
@@ -126,10 +153,13 @@ int main(int argc, char **argv)
     vs_cli_flow *rows = NULL;
     char **outs = NULL;
     uint8_t *preset = NULL;
+    char **spec = NULL;              /* formant spec of a voice, NULL for a preset voice */
+    size_t *lineno = NULL, nline = 0, nformant = 0;
     uint32_t *seed = NULL;
     float *gain = NULL, *pre = NULL;
     char line[4096];
     while (fgets(line, sizeof line, mf)) {
+        nline++;
         char *tok[MAXTOK];
         int nt = 0;
         for (char *t = strtok(line, " \t\r\n"); t && nt < MAXTOK; t = strtok(NULL, " \t\r\n")) tok[nt++] = t;
@@ -139,10 +169,15 @@ int main(int argc, char **argv)
             cap = cap ? cap * 2 : 1024;
             rows = realloc(rows, cap * sizeof *rows); outs = realloc(outs, cap * sizeof *outs);
             preset = realloc(preset, cap); seed = realloc(seed, cap * sizeof *seed);
+            spec = realloc(spec, cap * sizeof *spec); lineno = realloc(lineno, cap * sizeof *lineno);
             gain = realloc(gain, cap * sizeof *gain); pre = realloc(pre, cap * sizeof *pre);
         }
         outs[n] = strdup(tok[0]);
-        preset[n] = (uint8_t)tok[1][0];
+        const int is_formant = !strncmp(tok[1], "f:", 2);
+        preset[n] = is_formant ? (uint8_t)'a' : (uint8_t)tok[1][0];
+        spec[n] = is_formant ? strdup(tok[1]) : NULL;
+        lineno[n] = nline;
+        nformant += is_formant;
         seed[n] = (uint32_t)strtoul(tok[2], NULL, 10);
         gain[n] = 10.0f; pre[n] = 1.0f;
         /* split our two extra flags from the flowgen flags */
@@ -156,6 +191,15 @@ int main(int argc, char **argv)
         }
         if (fargc == 1) { fargv[fargc++] = "-d"; fargv[fargc++] = "1"; }
         if (vs_cli_parse_flow(fargc, fargv, 0, &rows[n])) { fprintf(stderr, "vs_batch: line %zu: bad flowgen flags\n", n + 1); return 1; }
+        if (is_formant) {
+            double den[23];
+            const int frc = formant_tract(spec[n], rows[n].fs, den);
+            if (frc) {
+                fprintf(stderr, "vs_batch: line %zu: %s formant tract '%s' (want f:F1/B1,F2/B2,... with 1 to %d formants, 0 < F < fs/2 = %d/2, B > 0)\n",
+                        nline, frc == -1 ? "malformed" : "out-of-range", spec[n], MAXFORMANTS, (int)rows[n].fs);
+                return 1;
+            }
+        }
         n++;
     }
     fclose(mf);
@@ -194,6 +238,13 @@ int main(int argc, char **argv)
         for (size_t i = a0; i < n && i < a0 + slab; i++) { offs[i] = tot; tot += (ns[i] + 7) & ~7ull; }   /* 16-byte aligned rows */
         if (tot > buf_samples) buf_samples = tot;
     }
+    /* the tract table of a slab with formant voices: presets and (spec, rate) pairs, each once */
+    double *tden = NULL;
+    uint8_t *tidx = NULL;
+    if (nformant) {
+        tden = malloc(sizeof(double) * 23 * VS_MAX_TRACTS);
+        tidx = malloc(slab);
+    }
     int16_t *buf[2];
     for (int k = 0; k < 2; k++) {
         buf[k] = vs_host_alloc(buf_samples * sizeof(int16_t));
@@ -212,8 +263,38 @@ int main(int argc, char **argv)
         pool_wait(&pool, k & 1);                                   /* slab k-2 is on disk */
         vs_flow_params ps = {dur + a0, jit + a0, shm + a0, cq + a0, K + a0, Kv + a0, F0 + a0, DC + a0, noise + a0,
                              amp + a0, fs + a0, flags + a0, seed + a0};
-        vs_filter_params fs_ = {preset + a0, gain + a0, pre + a0};
-        rc = vs_synth_batch(ctx, &ps, &fs_, cnt, pcm, offs + a0, NULL);
+        int any_formant = 0;
+        for (size_t i = a0; i < a0 + cnt && !any_formant; i++) any_formant = spec[i] != NULL;
+        if (!any_formant) {
+            vs_filter_params fs_ = {preset + a0, gain + a0, pre + a0};
+            rc = vs_synth_batch(ctx, &ps, &fs_, cnt, pcm, offs + a0, NULL);
+        } else {
+            /* entry t: a preset (key_spec[t] NULL, key_p[t] its key) or a formant spec at rate key_fs[t] */
+            const char *key_spec[VS_MAX_TRACTS];
+            int key_p[VS_MAX_TRACTS];
+            int32_t key_fs[VS_MAX_TRACTS];
+            uint32_t nt = 0;
+            for (size_t i = a0; i < a0 + cnt; i++) {
+                uint32_t t = 0;
+                for (; t < nt; t++) {
+                    if (spec[i] ? (key_spec[t] && key_fs[t] == fs[i] && !strcmp(key_spec[t], spec[i])) : (!key_spec[t] && key_p[t] == preset[i])) break;
+                }
+                if (t == nt) {
+                    if (nt == VS_MAX_TRACTS) {
+                        fprintf(stderr, "vs_batch: line %zu: more than %d distinct vocal tracts in one slab of %zu voices (lower -S)\n",
+                                lineno[i], VS_MAX_TRACTS, slab);
+                        return 1;
+                    }
+                    key_spec[nt] = spec[i]; key_p[nt] = preset[i]; key_fs[nt] = fs[i];
+                    const int trc = spec[i] ? formant_tract(spec[i], fs[i], tden + 23 * nt) : vs_tract_from_preset(preset[i], tden + 23 * nt);
+                    if (trc) { fprintf(stderr, "vs_batch: line %zu: bad vowel '%s'\n", lineno[i], spec[i] ? spec[i] : "?"); return 1; }
+                    nt++;
+                }
+                tidx[i - a0] = (uint8_t)t;
+            }
+            vs_tract_params tp = {tden, nt, tidx, gain + a0, pre + a0};
+            rc = vs_synth_batch_tract(ctx, &ps, &tp, cnt, pcm, offs + a0, NULL);
+        }
         if (!rc) rc = vs_sync(ctx);
         if (rc) { fprintf(stderr, "vs_batch: %s (%s)\n", vs_strerror(rc), vs_last_error(ctx)); return 1; }
         vs_timing t;

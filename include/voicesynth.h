@@ -114,7 +114,8 @@ typedef struct vs_timing {
     uint64_t h2d_bytes;       /* host->device bytes the call copied (descriptors, tables, flow_in) */
     uint64_t d2h_bytes;       /* device->host bytes the call copied (PCM, raw, period log)         */
     uint32_t render_path;     /* which render kernel ran (last launch): bit 0 = branch-free generator, bit 1 = glottal-noise
-                                 variant, bits 2-3 = filter arithmetic (0 integer pre-emphasis, 1 FMA, 2 exact)       */
+                                 variant, bits 2-3 = filter arithmetic (0 integer pre-emphasis, 1 FMA, 2 exact),
+                                 bit 6 = caller-defined tract coefficients (vs_*_batch_tract)                          */
     uint32_t reserved;
 } vs_timing;
 
@@ -210,6 +211,42 @@ int vs_vowel_noise_batch(vs_ctx *ctx, int16_t *pcm, const uint64_t *offsets, con
 /* n voices, flow generation fused with the filter: only the final PCM is written. */
 int vs_synth_batch(vs_ctx *ctx, const vs_flow_params *p, const vs_filter_params *f, size_t n,
                    int16_t *pcm_out, const uint64_t *offsets, double *raw_out);
+
+/* ---- caller-defined vocal tracts ------------------------------------------------------------ */
+/* The same filter as the presets (vowel_new.c:266-289: gain, the all-pole recurrence 1/A(z) of order <= 22,
+ * pre-emphasis), with the denominator supplied by the caller instead of one of the ten tables.  A tract holding a
+ * preset's table (vs_tract_from_preset) computes exactly what the preset does.
+ *
+ * Validation, per call:
+ *   n_tracts 0 or above VS_MAX_TRACTS, a stream's tract index >= n_tracts             -> VS_EINVAL
+ *   a coefficient not finite, A[0] != 1, or a carry warm-up (vs_filter_warmup at the ctx's VS_OPT_CARRY_TOL) above
+ *   16384 samples: unstable filters and nearly marginal ones (pole radius above ~0.998)  -> VS_ERANGE
+ * The warm-up of a tract is computed once per context (a few ms) and remembered, keyed by its coefficients. */
+#define VS_MAX_TRACTS 128
+typedef struct vs_tract_params {
+    const double  *den;       /* [n_tracts][23]: A[0..22] of 1/A(z); A[0] must be 1.0; lower orders end in zeros */
+    uint32_t       n_tracts;  /* 1..VS_MAX_TRACTS                                                                 */
+    const uint8_t *tract;     /* [n] index into den per stream (NULL: 0 for every stream)                        */
+    const float   *gain;      /* NULL: 10.0f  (same meaning as vs_filter_params)                                 */
+    const float   *pre;       /* NULL: 1.0f                                                                       */
+} vs_tract_params;
+
+/* vs_synth_batch / vs_vowel_filter_batch with caller-defined tracts: same buffers, offsets, raw output, options
+ * and arithmetic contract. */
+int vs_synth_batch_tract(vs_ctx *ctx, const vs_flow_params *p, const vs_tract_params *t, size_t n,
+                         int16_t *pcm_out, const uint64_t *offsets, double *raw_out);
+int vs_vowel_filter_batch_tract(vs_ctx *ctx, const int16_t *flow_in, const uint64_t *in_offsets, const uint64_t *nsamp,
+                                const vs_tract_params *t, size_t n, int16_t *pcm_out, const uint64_t *out_offsets,
+                                double *raw_out);
+
+/* host-only helpers, no GPU needed.
+ * vs_tract_from_formants: den = the product, in the order given, of  1 - 2 r_k cos(th_k) z^-1 + r_k^2 z^-2  with
+ * r_k = exp(-pi B_k / fs), th_k = 2 pi F_k / fs, in double; orders above 2*n_formants are zero.  n_formants is
+ * 1..11 (else VS_EINVAL); a formant is refused (VS_ERANGE) unless 0 < F_k < fs/2 and B_k > 0 (fs > 0).
+ * vs_tract_from_preset: the preset's table ('a','i','u','1'..'7'), for mixing presets and custom tracts in one
+ * call; an unknown key gives VS_EPRESET. */
+int vs_tract_from_formants(const float *freq_hz, const float *bw_hz, int n_formants, int32_t fs, double den[23]);
+int vs_tract_from_preset(int preset_key, double den[23]);
 
 #ifdef __cplusplus
 }

@@ -7,7 +7,8 @@ LIB_PATH = pathlib.Path(__file__).resolve().parent / "lib" / "libvoicesynth_cuda
 EXPORTS = ["vs_abi_version", "vs_device_count", "vs_strerror", "vs_last_error", "vs_ctx_create", "vs_ctx_destroy",
            "vs_ctx_set_option", "vs_ctx_set_stream", "vs_sync", "vs_get_timing", "vs_measure_fp64_peak", "vs_host_alloc", "vs_host_free",
            "vs_flow_nsamples", "vs_flow_max_periods", "vs_flow_validate", "vs_filter_warmup",
-           "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch"]
+           "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch",
+           "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset"]
 
 
 class FlowParamsC(C.Structure):
@@ -17,6 +18,10 @@ class FlowParamsC(C.Structure):
 
 class FilterParamsC(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("preset", "gain", "pre")]
+
+
+class TractParamsC(C.Structure):
+    _fields_ = [("den", C.c_void_p), ("n_tracts", C.c_uint32), ("tract", C.c_void_p), ("gain", C.c_void_p), ("pre", C.c_void_p)]
 
 
 class PeriodLogC(C.Structure):
@@ -71,5 +76,11 @@ def load():
                                  C.c_void_p, C.c_void_p, C.c_void_p]
     L.vs_flow_analyze_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_size_t, C.c_void_p]
+    L.vs_synth_batch_tract.argtypes = [C.c_void_p, C.POINTER(FlowParamsC), C.POINTER(TractParamsC), C.c_size_t,
+                                       C.c_void_p, C.c_void_p, C.c_void_p]
+    L.vs_vowel_filter_batch_tract.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(TractParamsC),
+                                              C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.vs_tract_from_formants.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int32, C.c_void_p]
+    L.vs_tract_from_preset.argtypes = [C.c_int, C.c_void_p]
     _lib = L
     return L

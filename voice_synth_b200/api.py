@@ -11,7 +11,7 @@ import re
 import numpy as np
 
 from . import _lib
-from ._lib import FilterParamsC, FlowParamsC, PeriodLogC, TimingC
+from ._lib import FilterParamsC, FlowParamsC, PeriodLogC, TimingC, TractParamsC
 
 VS_F_JITTER, VS_F_SHIMMER, VS_F_NOISE = 1, 2, 4
 VS_OK, VS_EINVAL, VS_ERANGE, VS_EPRESET, VS_ENOMEM, VS_ECUDA, VS_ENODEV, VS_EOVERLAP = 0, -1, -2, -3, -4, -5, -6, -7
@@ -206,6 +206,55 @@ class FilterParams:
         return c
 
 
+class TractParams:
+    """Caller-defined vocal tracts (vs_tract_params): den is [n_tracts][23] (A[0..22] of 1/A(z), A[0] = 1), tract the
+    per-stream index into it (None: 0 for every stream); gain and pre as in FilterParams."""
+
+    def __init__(self, n, den, tract=None, gain=10.0, pre=1.0):
+        self.n = n
+        self.den = np.ascontiguousarray(np.atleast_2d(np.asarray(den, dtype=np.float64)))
+        if self.den.shape[1] != 23:
+            raise ValueError(f"den must be [n_tracts][23], got {self.den.shape}")
+        self.tract = np.zeros(n, dtype=np.uint8)
+        if tract is not None:
+            self.tract[...] = tract
+        self.gain = np.full(n, gain, dtype=np.float32)
+        self.pre = np.full(n, pre, dtype=np.float32)
+
+    def select(self, idx):
+        q = TractParams(len(idx), self.den)
+        q.tract[...] = self.tract[idx]
+        q.gain[...] = self.gain[idx]
+        q.pre[...] = self.pre[idx]
+        return q
+
+    def _c(self):
+        return TractParamsC(self.den.ctypes.data, self.den.shape[0], self.tract.ctypes.data, self.gain.ctypes.data,
+                            self.pre.ctypes.data)
+
+
+def _den_or_raise(rc, den):
+    if rc:
+        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
+    return den
+
+
+def tract_from_formants(freqs, bws, fs):
+    """den[23] of the cascade of formant resonators (F_k, B_k in Hz) at sampling rate fs (vs_tract_from_formants)."""
+    f = np.ascontiguousarray(freqs, dtype=np.float32)
+    b = np.ascontiguousarray(bws, dtype=np.float32)
+    if f.shape != b.shape:
+        raise ValueError("freqs and bws differ in length")
+    den = np.zeros(23, dtype=np.float64)
+    return _den_or_raise(_lib.load().vs_tract_from_formants(f.ctypes.data, b.ctypes.data, f.size, int(fs), den.ctypes.data), den)
+
+
+def tract_from_preset(key):
+    """den[23] of a vowel preset ('a','i','u','1'..'7'), for mixing presets and custom tracts in one call."""
+    den = np.zeros(23, dtype=np.float64)
+    return _den_or_raise(_lib.load().vs_tract_from_preset(ord(key), den.ctypes.data), den)
+
+
 def flow_validate(p):
     """(VS_OK, None) or (error code, index of the first offending stream): the checks vs_*_batch apply up front."""
     bad = C.c_size_t(0)
@@ -317,8 +366,9 @@ class Context:
         if out is None:
             out = np.zeros(total, dtype=np.int16)
         raw = np.zeros(total, dtype=np.float64) if want_raw is True else (want_raw if want_raw is not False else None)
-        self._check(self.L.vs_vowel_filter_batch(self.h, _ptr(flow), _ptr(in_arg), ns.ctypes.data, C.byref(f._c()),
-                                                 len(ns), _ptr(out), _ptr(out_arg), _ptr(raw)))
+        call = self.L.vs_vowel_filter_batch_tract if isinstance(f, TractParams) else self.L.vs_vowel_filter_batch
+        self._check(call(self.h, _ptr(flow), _ptr(in_arg), ns.ctypes.data, C.byref(f._c()), len(ns), _ptr(out), _ptr(out_arg),
+                         _ptr(raw)))
         return (out, offs, raw) if want_raw is not False else (out, offs)
 
     def vowel_noise_batch(self, pcm, nsamp, snr_db, seeds, offsets=None, fs=None):
@@ -349,15 +399,16 @@ class Context:
         return stats
 
     def synth_batch(self, p, f, out=None, offsets=None, want_raw=False):
+        """f: FilterParams (the presets) or TractParams (caller-defined tracts, vs_synth_batch_tract)."""
+        call = self.L.vs_synth_batch_tract if isinstance(f, TractParams) else self.L.vs_synth_batch
         if out is not None and offsets is None and want_raw is False:
             # fast path for repeated calls into a caller-owned dense buffer: nothing to size or return
-            self._check(self.L.vs_synth_batch(self.h, C.byref(p._c()), C.byref(f._c()), p.n, _ptr(out), None, None))
+            self._check(call(self.h, C.byref(p._c()), C.byref(f._c()), p.n, _ptr(out), None, None))
             return out, None, None
         ns = flow_nsamples(p)
         offs_arg, offs, total = self._layout(ns, offsets)
         if out is None:
             out = np.zeros(total, dtype=np.int16)
         raw = np.zeros(total, dtype=np.float64) if want_raw is True else (want_raw if want_raw is not False else None)
-        self._check(self.L.vs_synth_batch(self.h, C.byref(p._c()), C.byref(f._c()), p.n, _ptr(out), _ptr(offs_arg),
-                                          _ptr(raw)))
+        self._check(call(self.h, C.byref(p._c()), C.byref(f._c()), p.n, _ptr(out), _ptr(offs_arg), _ptr(raw)))
         return (out, offs, ns, raw) if want_raw is not False else (out, offs, ns)

@@ -21,6 +21,7 @@
 #include <chrono>
 #include <map>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/voicesynth.h"
@@ -31,7 +32,9 @@ enum { VS_MODE_FLOW = 0, VS_MODE_SYNTH = 1, VS_MODE_FILTER = 2 };
 enum { VS_GEN_FAST = 0, VS_GEN_SIMPLE = 1 };
 enum { VS_FILT_INT = 0, VS_FILT_FMA = 1, VS_FILT_EXACT = 2 };
 cudaError_t vs_launch_plan(const VsPlanArgs &a, bool want_log, bool need_pulse, bool warp_per_stream, cudaStream_t s);
-cudaError_t vs_launch_render(const VsRenderArgs &a, int mode, int gen, bool noise, int filt, cudaStream_t s);
+cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s);
+static_assert(VS_MAX_TRACTS == VS_MAX_TRACTS_I, "tract count");
+static_assert(VS_MAX_TRACTS <= 256, "a stream's tract index is a uint8_t");
 cudaError_t vs_render_init_device();
 int vs_render_window(int mode);
 int vs_render_tiles(int mode);
@@ -87,7 +90,7 @@ struct Slot {
     std::vector<VsChunk> plan_chunks;
     std::vector<uint32_t> plan_order, plan_nch;
     struct PlanGeom {                                /* per slab: what the render launch needs besides the rows */
-        uint32_t cta_end[VS_NUM_PRESETS];
+        uint32_t cta_end[VS_MAX_TRACTS_I];           /* group ends: presets in blocks of 32 rows, tracts in CTAs  */
         uint32_t cache_doubles;                      /* pulse-table cache a warp needs (fast generator)        */
     };
     std::vector<PlanGeom> plan_geom;
@@ -120,6 +123,7 @@ struct vs_ctx {
     uint32_t pulse_last_off = 0;
     int warm[VS_NUM_PRESETS];    /* warm-up samples per preset at opt_tol (gain-independent part) */
     double l1gain[VS_NUM_PRESETS]; /* sum |h[n]| of each preset: |y| <= l1gain * gain * max|x| */
+    std::unordered_map<std::string, int> tract_warm;   /* warm-up at opt_tol of every tract seen, keyed by its 23 coefficients' bytes */
     std::string err;
     vs_timing timing;
     bool timing_pending = false;
@@ -133,6 +137,8 @@ struct vs_ctx {
         bool any_noise = false, any_kvar = false, int_filter = true, amp_fits = true, noise_simple = true;
         int t_min = 0x7fffffff, t_max = 0, t2_min = 0x7fffffff;
     } in_facts;
+    std::vector<int> in_warm;      /* warm-up per filter group of the inputs: per preset, or per tract of a _tract call */
+    std::vector<double> in_ncoef;  /* [n_tracts][VS_ORDER] = -A[1..22] of the inputs' tracts (tract calls) */
     uint64_t in_version = 0;     /* bumped whenever in_hs changes */
     bool env_profile_host = false, env_sync_plan = false;
 };
@@ -299,7 +305,7 @@ int preset_index(int key)
 
 /* Samples after which the free response of an arbitrary unit-bounded initial state has decayed below
  * tol: W = 1 + last n with sum_j |(Phi^n)[0][j]| >= tol, Phi the companion matrix of the preset. */
-int warmup_for(const double *A, double tol)
+int warmup_for(const double *A, double tol, int limit = 60000)
 {
     const int N = VS_ORDER;
     /* column j holds the free response state started from unit vector e_j */
@@ -318,7 +324,7 @@ int warmup_for(const double *A, double tol)
             s[0] = y0;
             g += std::fabs(y0);
         }
-        if (g >= tol) { last = n + 1; quiet = 0; }
+        if (!(g < tol)) { last = n + 1; quiet = 0; if (last >= limit) break; }    /* (a response that overflowed: not decayed) */
         else if (++quiet > 4096) break;
     }
     return last + 1;
@@ -443,6 +449,7 @@ struct Batch {
     size_t n;
     const vs_flow_params *fp;
     const vs_filter_params *ff;
+    const vs_tract_params *ft;     /* _tract calls: caller-defined tracts instead of ff */
     const int16_t *flow_in;
     const uint64_t *in_offsets;
     const uint64_t *nsamp;
@@ -516,7 +523,7 @@ uint32_t choose_chunk(vs_ctx *ctx, const Slot &slot, int mode, size_t n_streams,
  * chunk length  L_s = budget - W_s  and pick the smallest budget whose rows fit in `waves` waves;
  * take the wave count with the smallest  waves * budget. */
 void plan_filter_chunks(vs_ctx *ctx, const Slot &slot, const std::vector<VsStream> &hs, size_t a0, size_t a1,
-                        std::vector<uint32_t> &nchunks, int plan_nt)
+                        std::vector<uint32_t> &nchunks, int plan_nt, const int *warm, bool tracts)
 {
     const size_t ns = a1 - a0;
     nchunks.assign(ns, 1u);
@@ -543,12 +550,22 @@ void plan_filter_chunks(vs_ctx *ctx, const Slot &slot, const std::vector<VsStrea
     /* the first chunk of a stream needs no warm-up, so it emits `budget` samples, the others budget - W */
     auto chunks_of = [&](uint32_t n, uint8_t preset, double budget) -> uint32_t {
         if ((double)n <= budget) return 1u;
-        const double L = std::max(512.0, budget - (double)ctx->warm[preset]);
+        const double L = std::max(512.0, budget - (double)warm[preset]);
         return 1u + (uint32_t)std::ceil(((double)n - budget) / L);
     };
+    /* presets: groups padded to blocks of 32 rows, a 3 % allowance covers that; tracts: groups padded to whole CTAs,
+     * counted exactly */
+    const double fill = tracts ? 1.0 : 0.97;
     auto rows_for = [&](double budget) -> double {
+        if (!tracts) {
+            double rows = 0;
+            for (const auto &kv : classes) rows += (double)kv.second * chunks_of(kv.first.first, kv.first.second, budget);
+            return rows;
+        }
+        double per[VS_MAX_TRACTS_I] = {0.0};
+        for (const auto &kv : classes) per[kv.first.second] += (double)kv.second * chunks_of(kv.first.first, kv.first.second, budget);
         double rows = 0;
-        for (const auto &kv : classes) rows += (double)kv.second * chunks_of(kv.first.first, kv.first.second, budget);
+        for (int t = 0; t < VS_MAX_TRACTS_I; t++) rows += std::ceil(per[t] / VS_NT) * VS_NT;
         return rows;
     };
     double best_cost = 1e300, best_budget = (double)nmax;
@@ -557,12 +574,25 @@ void plan_filter_chunks(vs_ctx *ctx, const Slot &slot, const std::vector<VsStrea
         double lo = 512.0, hi = (double)nmax;                                  /* smallest budget that fits */
         for (int it = 0; it < 30; it++) {
             const double mid = 0.5 * (lo + hi);
-            if (rows_for(mid) <= waves * cap * 0.97) hi = mid; else lo = mid;  /* 3 % room for preset padding */
+            if (rows_for(mid) <= waves * cap * fill) hi = mid; else lo = mid;
         }
         const double cost = waves * hi;
         if (cost < best_cost * 0.98) { best_cost = cost; best_budget = hi; }
     }
     for (size_t i = 0; i < ns; i++) nchunks[i] = chunks_of(hs[a0 + i].n, hs[a0 + i].preset, best_budget);
+}
+
+/* a tract's warm-up at the ctx's tolerance, computed once per context; -1 if it is not acceptable */
+#define VS_TRACT_MAX_WARMUP 16384
+int tract_warmup(vs_ctx *ctx, const double *A)
+{
+    const std::string key(reinterpret_cast<const char *>(A), (VS_ORDER + 1) * sizeof(double));
+    auto it = ctx->tract_warm.find(key);
+    if (it != ctx->tract_warm.end()) return it->second;
+    const int w = warmup_for(A, ctx->opt_tol, VS_TRACT_MAX_WARMUP + 1);
+    if (ctx->tract_warm.size() >= (1u << 16)) ctx->tract_warm.clear();   /* a bound on what a stream of one-off tracts leaves behind */
+    ctx->tract_warm.emplace(key, w);
+    return w;
 }
 
 struct HostProf {
@@ -599,6 +629,12 @@ void snapshot_inputs(const Batch &b, bool want_log, const void *extra, size_t ex
         arr(b.fp->F0, 4); arr(b.fp->DC, 4); arr(b.fp->noise, 4); arr(b.fp->amp, 4); arr(b.fp->fs, 4); arr(b.fp->flags, 1); arr(b.fp->seed, 4);
     }
     if (b.ff) { arr(b.ff->preset, 1); arr(b.ff->gain, 4); arr(b.ff->pre, 4); }
+    if (b.ft) {
+        const uint64_t nt = b.ft->n_tracts;
+        put(&nt, sizeof nt);
+        if (b.ft->den && nt <= VS_MAX_TRACTS) put(b.ft->den, nt * (VS_ORDER + 1) * sizeof(double));
+        arr(b.ft->tract, 1); arr(b.ft->gain, 4); arr(b.ft->pre, 4);
+    }
     arr(b.nsamp, 8); arr(b.in_offsets, 8); arr(b.offsets, 8);
     if (want_log) put(b.log->rec_offsets, 8 * (b.n + 1));
 }
@@ -630,7 +666,8 @@ int run_batch(vs_ctx *ctx, const Batch &b)
     const PtrKind out_kind = classify(b.pcm_out, &odev);
     {   /* what the chunk plan depends on besides the parameter arrays */
         const double key[10] = {ctx->opt_chunk, ctx->opt_tol, (double)ctx->opt_exact, (double)ctx->opt_slab, ctx->opt_warps, (double)ctx->opt_simple_gen,
-                                (double)(out_kind == PK_DEVICE), (double)(reinterpret_cast<uintptr_t>(b.pcm_out) & 127), (double)ctx->slots.size(), 0.0};
+                                (double)(out_kind == PK_DEVICE), (double)(reinterpret_cast<uintptr_t>(b.pcm_out) & 127), (double)ctx->slots.size(),
+                                b.ft ? 1.0 : 0.0};
         snapshot_inputs(b, want_log, key, sizeof key, blob);
     }
     const bool same_inputs = blob.size() == ctx->in_blob.size() && memcmp(blob.data(), ctx->in_blob.data(), blob.size()) == 0;
@@ -645,6 +682,25 @@ int run_batch(vs_ctx *ctx, const Batch &b)
     int t2_min = 0x7fffffff;             /* shortest half open phase */
     bool amp_fits = true;            /* no amplitude can pass 32767 (fast generator) */
     bool noise_simple = true;        /* every noisy stream has DC <= 1 (then T4 == 0) and T2 >= 16: 16-byte period entries do */
+    /* filter groups: the ten presets, or the caller's tracts (validated, warm-ups from the ctx's cache) */
+    ctx->in_warm.assign(ctx->warm, ctx->warm + VS_NUM_PRESETS);
+    ctx->in_ncoef.clear();
+    if (b.ft) {
+        const uint32_t nt = b.ft->n_tracts;
+        if (!b.ft->den || nt == 0 || nt > VS_MAX_TRACTS) return fail(ctx, VS_EINVAL, "n_tracts %u outside 1..%d (or den is NULL)", nt, VS_MAX_TRACTS);
+        ctx->in_warm.assign(nt, 0);
+        ctx->in_ncoef.assign((size_t)nt * VS_ORDER, 0.0);
+        for (uint32_t t = 0; t < nt; t++) {
+            const double *A = b.ft->den + (size_t)t * (VS_ORDER + 1);
+            for (int j = 0; j <= VS_ORDER; j++)
+                if (!std::isfinite(A[j])) return fail(ctx, VS_ERANGE, "tract %u: coefficient %d is not finite", t, j);
+            if (A[0] != 1.0) return fail(ctx, VS_ERANGE, "tract %u: A[0] = %g, must be 1", t, A[0]);
+            const int w = tract_warmup(ctx, A);
+            if (w > VS_TRACT_MAX_WARMUP) return fail(ctx, VS_ERANGE, "tract %u: unstable or nearly marginal (carry warm-up above %d samples)", t, VS_TRACT_MAX_WARMUP);
+            ctx->in_warm[t] = w;
+            for (int j = 1; j <= VS_ORDER; j++) ctx->in_ncoef[(size_t)t * VS_ORDER + j - 1] = -A[j];
+        }
+    }
     for (size_t i = 0; i < n; i++) {
         VsStream &s = hs[i];
         memset(&s, 0, sizeof s);
@@ -678,13 +734,21 @@ int run_batch(vs_ctx *ctx, const Batch &b)
                 if ((r.flags & VS_F_SHIMMER) && r.shimmer != 0.0f ? 1.8f * (float)r.amp > 32767.0f : r.amp > 32767) amp_fits = false;
             }
         }
-        if (b.mode != VS_MODE_FLOW) {
+        if (b.mode != VS_MODE_FLOW && b.ft) {
+            const uint32_t t = b.ft->tract ? b.ft->tract[i] : 0u;
+            if (t >= b.ft->n_tracts) return fail(ctx, VS_EINVAL, "stream %zu: tract index %u >= n_tracts %u", i, t, b.ft->n_tracts);
+            s.preset = (uint8_t)t;                                      /* the filter group: here a tract */
+            s.gain = b.ft->gain ? b.ft->gain[i] : 10.0f;
+            s.pre = b.ft->pre ? b.ft->pre[i] : 1.0f;
+        } else if (b.mode != VS_MODE_FLOW) {
             const int key = b.ff && b.ff->preset ? b.ff->preset[i] : 'a';
             const int pi = preset_index(key);
             if (pi < 0) return fail(ctx, VS_EPRESET, "stream %zu: unknown vowel preset 0x%02x", i, key);
             s.preset = (uint8_t)pi;
             s.gain = b.ff && b.ff->gain ? b.ff->gain[i] : 10.0f;
             s.pre = b.ff && b.ff->pre ? b.ff->pre[i] : 1.0f;
+        }
+        if (b.mode != VS_MODE_FLOW) {
             if (!std::isfinite(s.gain) || !std::isfinite(s.pre)) return fail(ctx, VS_ERANGE, "stream %zu: gain/pre not finite", i);
             if (!(s.gain == std::floor(s.gain) && std::fabs(s.gain) <= 32767.0f && (s.pre == 0.0f || s.pre == 1.0f))) int_filter = false;
         }
@@ -728,6 +792,10 @@ int run_batch(vs_ctx *ctx, const Batch &b)
     const vs_ctx::Facts &fc = ctx->in_facts;
     const bool any_noise = fc.any_noise, any_kvar = fc.any_kvar, int_filter = fc.int_filter, amp_fits = fc.amp_fits, noise_simple = fc.noise_simple;
     const int t_min = fc.t_min, t_max = fc.t_max;
+    const bool tracts = b.ft != nullptr;
+    const int *gwarm = ctx->in_warm.data();          /* warm-up per filter group (preset or tract) */
+    const int n_groups = tracts ? VS_MAX_TRACTS_I : VS_NUM_PRESETS;
+    const size_t group_rows = tracts ? VS_NT : 32;   /* groups are padded to whole CTAs (tracts) or blocks of 32 rows (presets) */
 
     prof.mark("stream descriptors");
     /* ---- 2. where do the buffers live ------------------------------------------------------- */
@@ -790,7 +858,7 @@ int run_batch(vs_ctx *ctx, const Batch &b)
         double warm_sum = 0.0;
         for (size_t i = s0; i < s1; i++) {
             total += hs[i].n;
-            if (b.mode != VS_MODE_FLOW) warm_sum += ctx->warm[hs[i].preset];
+            if (b.mode != VS_MODE_FLOW) warm_sum += gwarm[hs[i].preset];
         }
         /* slabs: groups of consecutive streams that are launched and copied together */
         size_t slab_streams = ns;
@@ -816,6 +884,8 @@ int run_batch(vs_ctx *ctx, const Batch &b)
         sig.push_back(((uint64_t)b.mode << 48) ^ ((uint64_t)n_slabs << 24) ^ (uint64_t)slab_streams ^ ((uint64_t)plan_nt << 52));
         sig.push_back((uint64_t)(int64_t)ctx->opt_chunk ^ ((uint64_t)ctx->opt_exact << 62) ^ ((uint64_t)sl.sm_count << 40));
         { double t = ctx->opt_tol, w = ctx->opt_warps; uint64_t u; memcpy(&u, &t, 8); sig.push_back(u); memcpy(&u, &w, 8); sig.push_back(u); }
+        sig.push_back((uint64_t)tracts);
+        if (tracts) for (int w : ctx->in_warm) sig.push_back((uint64_t)w);   /* the chunk plan depends on the tracts' warm-ups */
         for (size_t i = s0; i < s1; i++) {
             const uint64_t base_addr = out_dev ? (reinterpret_cast<uintptr_t>(b.pcm_out) >> 1) + hs[i].out_off : hs[i].out_off;
             sig.push_back((uint64_t)hs[i].n | ((uint64_t)hs[i].preset << 32) | ((base_addr & ph_mask) << 40));
@@ -838,7 +908,7 @@ int run_batch(vs_ctx *ctx, const Batch &b)
             for (size_t i = a0; i < a1; i++) tot += hs[i].n;
             const uint32_t Lflow = b.mode == VS_MODE_FLOW ? choose_chunk(ctx, sl, b.mode, a1 - a0, tot, 0.0, flow_rows) : 0u;
             std::vector<uint32_t> nch;
-            if (b.mode != VS_MODE_FLOW) plan_filter_chunks(ctx, sl, hs, a0, a1, nch, plan_nt);
+            if (b.mode != VS_MODE_FLOW) plan_filter_chunks(ctx, sl, hs, a0, a1, nch, plan_nt, gwarm, tracts);
             slab_c0[k] = hc.size();
             for (size_t i = a0; i < a1; i++) {
                 VsStream &s = hs[i];
@@ -846,7 +916,7 @@ int run_batch(vs_ctx *ctx, const Batch &b)
                 /* host outputs are mirrored on the device at the same offsets relative to a 16-byte
                  * aligned slab base, so the phase of a row is its sample offset mod 8 either way */
                 const uint32_t ph = (uint32_t)(base_addr & ph_mask);
-                const uint32_t W = (b.mode == VS_MODE_FLOW) ? 0u : (uint32_t)ctx->warm[s.preset];
+                const uint32_t W = (b.mode == VS_MODE_FLOW) ? 0u : (uint32_t)gwarm[s.preset];
                 /* chunk c > 0 emits [L0 + (c-1)*L - ph, L0 + c*L - ph); L0 and L are multiples of 8 (of 256 for the
                  * lanes-along-the-row flow kernel, whose steps then never straddle two chunks) */
                 uint32_t C, L, L0;
@@ -906,7 +976,7 @@ int run_batch(vs_ctx *ctx, const Batch &b)
                     const uint32_t id = (uint32_t)(slab_c0[k] + c);
                     /* (flow-only chunks are all about one length: keep rows that share a pulse table together instead) */
                     const uint32_t work = b.mode == VS_MODE_FLOW ? 0u : (hc[id].emit_hi - hc[id].gen_target) >> 6;
-                    keyed[c] = {((uint64_t)preset_of(id) << 60) | ((uint64_t)(0x0fffffffu - std::min(work, 0x0fffffffu)) << 32) |
+                    keyed[c] = {((uint64_t)preset_of(id) << 57) | ((uint64_t)(0x01ffffffu - std::min(work, 0x01ffffffu)) << 32) |
                                     (uint64_t)hs[s0 + hc[id].stream].pulse_off, id};
                 }
                 std::sort(keyed.begin(), keyed.end());
@@ -920,12 +990,12 @@ int run_batch(vs_ctx *ctx, const Batch &b)
                 size_t i1 = i0;
                 const int pr = preset_of(ids[i0]);
                 while (i1 < ids.size() && preset_of(ids[i1]) == pr) i1++;
-                for (; pr_done < pr; pr_done++) gm.cta_end[pr_done] = (uint32_t)((order.size() - r_first) / 32);
+                for (; pr_done < pr; pr_done++) gm.cta_end[pr_done] = (uint32_t)((order.size() - r_first) / group_rows);
                 for (size_t i = i0; i < i1; i++) order.push_back(ids[i]);
-                while ((order.size() - r_first) % 32) order.push_back(VS_NO_CHUNK);
+                while ((order.size() - r_first) % group_rows) order.push_back(VS_NO_CHUNK);
                 i0 = i1;
             }
-            for (; pr_done < VS_NUM_PRESETS; pr_done++) gm.cta_end[pr_done] = (uint32_t)((order.size() - r_first) / 32);
+            for (; pr_done < n_groups; pr_done++) gm.cta_end[pr_done] = (uint32_t)((order.size() - r_first) / group_rows);
             /* pulse-table cache: the largest sum of distinct (padded) tables over the warps of the slab */
             gm.cache_doubles = 0;
             if (b.mode != VS_MODE_FILTER) {
@@ -1250,11 +1320,17 @@ int run_batch(vs_ctx *ctx, const Batch &b)
                 ra.grid = std::max(1u, std::min((ra.n_rows + rows_per_cta - 1u) / rows_per_cta, render_sms * 4u));
                 CU(vs_launch_flow_rows(ra, sl.compute));
                 sl.ticket_base += ra.n_rows + ra.grid * rows_per_cta;       /* wraps like the device counter does */
+            } else if (tracts) {
+                VsTractBlock tb;                             /* copied into the launch's parameter space */
+                memcpy(tb.cta_end, sl.plan_geom[k].cta_end, sizeof tb.cta_end);
+                memset(tb.ncoef, 0, sizeof tb.ncoef);
+                memcpy(tb.ncoef, ctx->in_ncoef.data(), ctx->in_ncoef.size() * sizeof(double));
+                CU(vs_launch_render(ra, &tb, b.mode, gen, any_noise, filt, sl.compute));
             } else
-                CU(vs_launch_render(ra, b.mode, gen, any_noise, filt, sl.compute));
+                CU(vs_launch_render(ra, nullptr, b.mode, gen, any_noise, filt, sl.compute));
             ctx->timing.launches++;
             ctx->timing.render_path = (gen == VS_GEN_FAST || flow_rows ? 1u : 0u) | (any_noise ? 2u : 0u) | ((uint32_t)(b.raw_out && filt == VS_FILT_INT ? VS_FILT_FMA : filt) << 2) |
-                                      (flow_rows ? 32u : 0u);
+                                      (flow_rows ? 32u : 0u) | (tracts ? 64u : 0u);
             if (g == 0) { cudaEvent_t e2 = timing_event(sl); CU(cudaEventRecord(e2, sl.compute)); }
 
             if (!out_dev) {
@@ -1454,7 +1530,7 @@ int vs_ctx_set_option(vs_ctx *ctx, int option, double value)
     case VS_OPT_CHUNK_SAMPLES: ctx->opt_chunk = value; return VS_OK;
     case VS_OPT_CARRY_TOL:
         if (!(value > 0.0 && value < 1.0)) return VS_EINVAL;
-        ctx->opt_tol = value; compute_warmups(ctx); return VS_OK;
+        ctx->opt_tol = value; compute_warmups(ctx); ctx->tract_warm.clear(); return VS_OK;
     case VS_OPT_EXACT_FILTER: ctx->opt_exact = value != 0.0; return VS_OK;
     case VS_OPT_SLAB_STREAMS: ctx->opt_slab = value > 0 ? (int)value : 0; return VS_OK;
     case VS_OPT_TARGET_WARPS: if (!(value > 0)) return VS_EINVAL; ctx->opt_warps = value; return VS_OK;
@@ -1594,14 +1670,22 @@ int vs_filter_warmup(vs_ctx *ctx, int preset_key, float gain)
 
 int vs_flowgen_batch(vs_ctx *ctx, const vs_flow_params *p, size_t n, int16_t *pcm_out, const uint64_t *offsets, vs_period_log *log)
 {
-    Batch b = {VS_MODE_FLOW, n, p, nullptr, nullptr, nullptr, nullptr, pcm_out, offsets, nullptr, log};
+    Batch b = {VS_MODE_FLOW, n, p, nullptr, nullptr, nullptr, nullptr, nullptr, pcm_out, offsets, nullptr, log};
     return run_batch(ctx, b);
 }
 
 int vs_vowel_filter_batch(vs_ctx *ctx, const int16_t *flow_in, const uint64_t *in_offsets, const uint64_t *nsamp,
                           const vs_filter_params *f, size_t n, int16_t *pcm_out, const uint64_t *out_offsets, double *raw_out)
 {
-    Batch b = {VS_MODE_FILTER, n, nullptr, f, flow_in, in_offsets, nsamp, pcm_out, out_offsets, raw_out, nullptr};
+    Batch b = {VS_MODE_FILTER, n, nullptr, f, nullptr, flow_in, in_offsets, nsamp, pcm_out, out_offsets, raw_out, nullptr};
+    return run_batch(ctx, b);
+}
+
+int vs_vowel_filter_batch_tract(vs_ctx *ctx, const int16_t *flow_in, const uint64_t *in_offsets, const uint64_t *nsamp,
+                                const vs_tract_params *t, size_t n, int16_t *pcm_out, const uint64_t *out_offsets, double *raw_out)
+{
+    if (!t) return fail(ctx, VS_EINVAL, "tract params are NULL");
+    Batch b = {VS_MODE_FILTER, n, nullptr, nullptr, t, flow_in, in_offsets, nsamp, pcm_out, out_offsets, raw_out, nullptr};
     return run_batch(ctx, b);
 }
 
@@ -1717,8 +1801,48 @@ int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offs
 int vs_synth_batch(vs_ctx *ctx, const vs_flow_params *p, const vs_filter_params *f, size_t n, int16_t *pcm_out,
                    const uint64_t *offsets, double *raw_out)
 {
-    Batch b = {VS_MODE_SYNTH, n, p, f, nullptr, nullptr, nullptr, pcm_out, offsets, raw_out, nullptr};
+    Batch b = {VS_MODE_SYNTH, n, p, f, nullptr, nullptr, nullptr, nullptr, pcm_out, offsets, raw_out, nullptr};
     return run_batch(ctx, b);
+}
+
+int vs_synth_batch_tract(vs_ctx *ctx, const vs_flow_params *p, const vs_tract_params *t, size_t n, int16_t *pcm_out,
+                         const uint64_t *offsets, double *raw_out)
+{
+    if (!t) return fail(ctx, VS_EINVAL, "tract params are NULL");
+    Batch b = {VS_MODE_SYNTH, n, p, nullptr, t, nullptr, nullptr, nullptr, pcm_out, offsets, raw_out, nullptr};
+    return run_batch(ctx, b);
+}
+
+int vs_tract_from_formants(const float *freq_hz, const float *bw_hz, int n_formants, int32_t fs, double den[23])
+{
+    if (!freq_hz || !bw_hz || !den || n_formants < 1 || 2 * n_formants > VS_ORDER) return VS_EINVAL;
+    if (fs <= 0) return VS_ERANGE;
+    const double pi = 3.14159265358979323846, rate = (double)fs;
+    for (int k = 0; k < n_formants; k++) {
+        const double F = freq_hz[k], B = bw_hz[k];
+        if (!(F > 0.0 && F < 0.5 * rate) || !(B > 0.0) || !std::isfinite(B)) return VS_ERANGE;
+    }
+    double d[VS_ORDER + 1] = {1.0};
+    for (int k = 0; k < n_formants; k++) {
+        const double r = std::exp(-pi * (double)bw_hz[k] / rate), th = 2.0 * pi * (double)freq_hz[k] / rate;
+        const double b1 = -2.0 * r * std::cos(th), b2 = r * r;
+        for (int j = 2 * k + 2; j >= 1; j--) {         /* d <- d * (1 + b1 z^-1 + b2 z^-2), in place from the top */
+            double v = d[j] + b1 * d[j - 1];
+            if (j >= 2) v += b2 * d[j - 2];
+            d[j] = v;
+        }
+    }
+    memcpy(den, d, sizeof d);
+    return VS_OK;
+}
+
+int vs_tract_from_preset(int preset_key, double den[23])
+{
+    const int k = preset_index(preset_key);
+    if (k < 0) return VS_EPRESET;
+    if (!den) return VS_EINVAL;
+    memcpy(den, vs_preset_den[k], (VS_ORDER + 1) * sizeof(double));
+    return VS_OK;
 }
 
 } /* extern "C" */

@@ -140,6 +140,15 @@ struct VsRenderArgs {
     uint32_t        ticket_base;    /* ... and its value when the launch starts                      */
 };
 
+/* the caller's vocal tracts (vs_synth_batch_tract, vs_vowel_filter_batch_tract): the render kernel's second,
+ * __grid_constant__ parameter block, one per launch.  Rows are grouped by tract and every group is padded to whole
+ * CTAs of VS_NT rows, so that a CTA's tract -- and the address of its coefficients -- is uniform. */
+#define VS_MAX_TRACTS_I 128   /* == VS_MAX_TRACTS (voicesynth.h) */
+struct VsTractBlock {
+    uint32_t cta_end[VS_MAX_TRACTS_I];          /* CTAs [cta_end[t-1], cta_end[t]) of the launch belong to tract t */
+    double   ncoef[VS_MAX_TRACTS_I][VS_ORDER];  /* ncoef[t][j-1] = -A_t[j], j = 1..22                              */
+};
+
 /* vowel -n (N1): one entry per stream */
 struct VsNoiseRow {
     uint64_t off;          /* samples, relative to the pcm pointer */

@@ -27,6 +27,8 @@
 #include "vs_device.cuh"
 #include "vs_presets.h"
 
+#include <type_traits>
+
 static_assert(VS_NUM_PRESETS == VS_NUM_PRESETS_I, "preset count");
 
 __constant__ double c_ncoef[VS_NUM_PRESETS][VS_RING];      /* c_ncoef[p][j] = -A_p[j], j = 1..22 (vowel_new.c:450-544) */
@@ -95,11 +97,16 @@ __device__ __forceinline__ void vs_pair_barrier(int pair)
     asm volatile("bar.sync %0, 64;" ::"r"(1 + pair) : "memory");
 }
 
-/* ---- F: one lane, one row: the order-22 recurrence (vowel_new.c:266-289) window after window, in place ------- */
+/* ---- F: one lane, one row: the order-22 recurrence (vowel_new.c:266-289) window after window, in place ------- *
+ * Coefficients: PRESET >= 0 reads c_ncoef[PRESET] at literal constant-bank addresses; PRESET < 0 reads tcoef[0..21]
+ * (= -A[1..22]) inside the kernel's parameter block (the tract kernels).  The operations and their order are the
+ * same either way. */
 template <int WIN, int NT, int FILT, bool RAW, int PRESET>
 __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane's row in tile 0 */, const int pair, const int nwin,
-                                               const double gaind, const double pred, double *rrow, const int blk0, const int lo, const int hi)
+                                               const double gaind, const double pred, double *rrow, const int blk0, const int lo, const int hi,
+                                               const double *tcoef)
 {
+#define VS_NC(j) (PRESET >= 0 ? c_ncoef[PRESET < 0 ? 0 : PRESET][j] : tcoef[(j) - 1])
     constexpr int TILE = 32 * WIN * 2;
     double y[VS_RING];
 #pragma unroll
@@ -131,18 +138,18 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
                         acc = (double)((xi + x_prev * npre_i) * gain_i);
                         x_prev = xi;
 #pragma unroll
-                        for (int j = VS_ORDER; j >= 1; j--) acc = __fma_rn(y[(k + VS_RING - j) % VS_RING], c_ncoef[PRESET][j], acc);
+                        for (int j = VS_ORDER; j >= 1; j--) acc = __fma_rn(y[(k + VS_RING - j) % VS_RING], VS_NC(j), acc);
                         v = acc;
                     } else if (FILT == VS_FILT_FMA) {
                         acc = __dmul_rn((double)xi, gaind);                                          /* vowel_new.c:266-269 */
 #pragma unroll
-                        for (int j = VS_ORDER; j >= 1; j--) acc = __fma_rn(y[(k + VS_RING - j) % VS_RING], c_ncoef[PRESET][j], acc);
+                        for (int j = VS_ORDER; j >= 1; j--) acc = __fma_rn(y[(k + VS_RING - j) % VS_RING], VS_NC(j), acc);
                         v = __fma_rn(-pred, y[(k + VS_RING - 1) % VS_RING], acc);                    /* :284 */
                     } else {
                         acc = __dmul_rn((double)xi, gaind);
 #pragma unroll
                         for (int j = 1; j <= VS_ORDER; j++)                                          /* :279-281, same order, unfused */
-                            acc = __dsub_rn(acc, __dmul_rn(-c_ncoef[PRESET][j], y[(k + VS_RING - j) % VS_RING]));
+                            acc = __dsub_rn(acc, __dmul_rn(-VS_NC(j), y[(k + VS_RING - j) % VS_RING]));
                         v = __dsub_rn(acc, __dmul_rn(pred, y[(k + VS_RING - 1) % VS_RING]));
                     }
                     y[k] = acc;                                                                      /* :287-289 (ring) */
@@ -168,6 +175,7 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
         vs_fence_async();                                   /* the TMA engine will read what this lane wrote */
         vs_pair_barrier(pair);                              /* window w filtered; window w+1 generated */
     }
+#undef VS_NC
 }
 
 #define VS_RENDER_THREADS(MODE) ((MODE) == VS_MODE_FLOW ? VS_NT : 2 * VS_NT)
@@ -175,8 +183,13 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
  * share an SM and the other warps run while a warp waits for its tile to be read out */
 #define VS_RENDER_TILES(MODE)   ((MODE) == VS_MODE_FLOW ? 1 : 3)
 
-template <int MODE, int GEN, bool NOISE, int FILT, bool RAW>
-__global__ void __launch_bounds__(VS_RENDER_THREADS(MODE), MODE == VS_MODE_FLOW ? 4 : 1) vs_render_kernel(const VsRenderArgs a)
+/* the second parameter block: the caller's vocal tracts (vs_*_batch_tract), nothing for the preset kernels */
+struct VsNoTracts {};
+template <bool TRACT> using VsTractParam = typename std::conditional<TRACT, VsTractBlock, VsNoTracts>::type;
+
+template <int MODE, int GEN, bool NOISE, int FILT, bool RAW, bool TRACT>
+__global__ void __launch_bounds__(VS_RENDER_THREADS(MODE), MODE == VS_MODE_FLOW ? 4 : 1)
+vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRACT> tr)
 {
     constexpr int WIN = vs_win(MODE), TSB = WIN * 2, TILE = 32 * TSB, NGRP = WIN / VS_GROUP;
     constexpr int NT = VS_RENDER_TILES(MODE);
@@ -202,13 +215,24 @@ __global__ void __launch_bounds__(VS_RENDER_THREADS(MODE), MODE == VS_MODE_FLOW 
      * next calls); a pair of warps takes blocks of 32 rows round robin until the batch is done.  Rows are sorted
      * longest first inside a preset, so every pair gets a similar mix. */
     const uint32_t n_blocks = a.n_rows / 32u;
-    for (uint32_t pb = blockIdx.x * 4u + (uint32_t)pair; pb < n_blocks; pb += gridDim.x * 4u) {
+    for (uint32_t pb = blockIdx.x * 4u + (uint32_t)pair, cb = blockIdx.x; pb < n_blocks; pb += gridDim.x * 4u, cb += gridDim.x) {
     /* vowel preset of this block of rows: a function of its index and kernel parameters (rows are grouped by preset
      * and padded to whole blocks) */
     int preset = 0;
-    if (HASFILT) {
+    if (HASFILT && !TRACT) {
 #pragma unroll
         for (int p = 0; p < VS_NUM_PRESETS - 1; p++) preset += pb >= a.cta_end[p] ? 1 : 0;
+    }
+    /* vocal tract of this CTA's rows (tract kernels): a binary search over the group ends, which are counted in CTAs
+     * (tract groups are padded to whole CTAs, so the 4 pairs of a CTA share a tract).  The tract is CTA-uniform, but
+     * the compiler does not prove it inside this loop, whose body branches on the warp role: it loads the 22
+     * coefficients into registers once per block of rows and the F loop runs three-register DFMAs (DESIGN.md 4.6). */
+    const double *tcoef = nullptr;
+    if constexpr (TRACT) {
+        int t = 0;
+#pragma unroll
+        for (int s = VS_MAX_TRACTS_I / 2; s > 0; s >>= 1) t += cb >= tr.cta_end[t + s - 1] ? s : 0;
+        tcoef = tr.ncoef[t];
     }
 
     /* ---- the lane's row (lane l of F and lane l of G serve the same row) -------------------------------- */
@@ -251,10 +275,11 @@ __global__ void __launch_bounds__(VS_RENDER_THREADS(MODE), MODE == VS_MODE_FLOW 
         const double gaind = active ? (double)st->gain : 0.0, pred = active ? (double)st->pre : 0.0;
         double *rrow = (RAW && active && a.raw_out) ? a.raw_out + st->out_off : nullptr;
         unsigned char *tiles = smem + tile_off + (uint32_t)lane * TSB;
-        switch (preset) {
-#define VS_F_CASE(P) case P: vs_filter_rows<WIN, NT, FILT, RAW, P>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi); break;
+        if constexpr (TRACT) vs_filter_rows<WIN, NT, FILT, RAW, -1>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, tcoef);
+        else switch (preset) {
+#define VS_F_CASE(P) case P: vs_filter_rows<WIN, NT, FILT, RAW, P>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, nullptr); break;
             VS_F_CASE(0) VS_F_CASE(1) VS_F_CASE(2) VS_F_CASE(3) VS_F_CASE(4) VS_F_CASE(5) VS_F_CASE(6) VS_F_CASE(7) VS_F_CASE(8)
-            default: vs_filter_rows<WIN, NT, FILT, RAW, 9>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi); break;
+            default: vs_filter_rows<WIN, NT, FILT, RAW, 9>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, nullptr); break;
 #undef VS_F_CASE
         }
         continue;
@@ -635,8 +660,8 @@ cudaError_t vs_render_init_device()
 int vs_render_window(int mode) { return vs_win(mode); }
 int vs_render_tiles(int mode) { return VS_RENDER_TILES(mode); }
 
-template <int MODE, int GEN, bool NOISE, int FILT, bool RAW>
-static cudaError_t vs_go(const VsRenderArgs &a, cudaStream_t s)
+template <int MODE, int GEN, bool NOISE, int FILT, bool RAW, bool TRACT = false>
+static cudaError_t vs_go(const VsRenderArgs &a, const VsTractBlock *tb, cudaStream_t s)
 {
     const unsigned grid = a.grid;
     const int dyn = 4 * (int)a.warp_bytes + (NOISE ? VS_RNG_DEG * VS_NT * 4 : 0);      /* warp_bytes: per pair of warps */
@@ -645,34 +670,42 @@ static cudaError_t vs_go(const VsRenderArgs &a, cudaStream_t s)
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 16 && granted[dev] < dyn) {
-        const cudaError_t e = cudaFuncSetAttribute(vs_render_kernel<MODE, GEN, NOISE, FILT, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
+        const cudaError_t e = cudaFuncSetAttribute(vs_render_kernel<MODE, GEN, NOISE, FILT, RAW, TRACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
         if (e != cudaSuccess) return e;
         granted[dev] = dyn;
     } else if (dev >= 16) {
-        cudaFuncSetAttribute(vs_render_kernel<MODE, GEN, NOISE, FILT, RAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
+        cudaFuncSetAttribute(vs_render_kernel<MODE, GEN, NOISE, FILT, RAW, TRACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
     }
-    vs_render_kernel<MODE, GEN, NOISE, FILT, RAW><<<grid, VS_RENDER_THREADS(MODE), dyn, s>>>(a);
+    if constexpr (TRACT) vs_render_kernel<MODE, GEN, NOISE, FILT, RAW, true><<<grid, VS_RENDER_THREADS(MODE), dyn, s>>>(a, *tb);
+    else vs_render_kernel<MODE, GEN, NOISE, FILT, RAW, false><<<grid, VS_RENDER_THREADS(MODE), dyn, s>>>(a, VsNoTracts());
     return cudaGetLastError();
 }
 
-template <int MODE, int GEN, bool NOISE>
-static cudaError_t vs_go_filt(const VsRenderArgs &a, int filt, cudaStream_t s)
+template <int MODE, int GEN, bool NOISE, bool TRACT>
+static cudaError_t vs_go_filt(const VsRenderArgs &a, const VsTractBlock *tb, int filt, cudaStream_t s)
 {
     const bool raw = a.raw_out != nullptr;
-    if (filt == VS_FILT_EXACT) return raw ? vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, true>(a, s) : vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, false>(a, s);
-    if (raw) return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, true>(a, s);
-    if (filt == VS_FILT_INT) return vs_go<MODE, GEN, NOISE, VS_FILT_INT, false>(a, s);
-    return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, false>(a, s);
+    if (filt == VS_FILT_EXACT) return raw ? vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, true, TRACT>(a, tb, s) : vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, false, TRACT>(a, tb, s);
+    if (raw) return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, true, TRACT>(a, tb, s);
+    if (filt == VS_FILT_INT) return vs_go<MODE, GEN, NOISE, VS_FILT_INT, false, TRACT>(a, tb, s);
+    return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, false, TRACT>(a, tb, s);
 }
 
-/* gen: VS_GEN_FAST / VS_GEN_SIMPLE; filt: VS_FILT_INT / _FMA / _EXACT (raw output forces _FMA or _EXACT) */
-cudaError_t vs_launch_render(const VsRenderArgs &a, int mode, int gen, bool noise, int filt, cudaStream_t s)
+template <bool TRACT>
+static cudaError_t vs_go_filter_modes(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s)
 {
-    if (mode == VS_MODE_FILTER) return vs_go_filt<VS_MODE_FILTER, VS_GEN_SIMPLE, false>(a, filt, s);
+    if (mode == VS_MODE_FILTER) return vs_go_filt<VS_MODE_FILTER, VS_GEN_SIMPLE, false, TRACT>(a, tb, filt, s);
+    if (gen == VS_GEN_FAST) return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, true, TRACT>(a, tb, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, false, TRACT>(a, tb, filt, s);
+    return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, true, TRACT>(a, tb, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, false, TRACT>(a, tb, filt, s);
+}
+
+/* gen: VS_GEN_FAST / VS_GEN_SIMPLE; filt: VS_FILT_INT / _FMA / _EXACT (raw output forces _FMA or _EXACT);
+ * tb: the caller's vocal tracts (synth and filter modes), nullptr for the presets */
+cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s)
+{
     if (mode == VS_MODE_FLOW) {
-        if (gen == VS_GEN_FAST) return noise ? vs_go<VS_MODE_FLOW, VS_GEN_FAST, true, VS_FILT_FMA, false>(a, s) : vs_go<VS_MODE_FLOW, VS_GEN_FAST, false, VS_FILT_FMA, false>(a, s);
-        return noise ? vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, true, VS_FILT_FMA, false>(a, s) : vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, false, VS_FILT_FMA, false>(a, s);
+        if (gen == VS_GEN_FAST) return noise ? vs_go<VS_MODE_FLOW, VS_GEN_FAST, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_FAST, false, VS_FILT_FMA, false>(a, nullptr, s);
+        return noise ? vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, false, VS_FILT_FMA, false>(a, nullptr, s);
     }
-    if (gen == VS_GEN_FAST) return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, true>(a, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, false>(a, filt, s);
-    return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, true>(a, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, false>(a, filt, s);
+    return tb ? vs_go_filter_modes<true>(a, tb, mode, gen, noise, filt, s) : vs_go_filter_modes<false>(a, nullptr, mode, gen, noise, filt, s);
 }
