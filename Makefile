@@ -7,9 +7,9 @@ NVFLAGS   := -O3 -std=c++17 $(ARCH) -lineinfo -fmad=false -cudart static \
 LIBDIR    := voice_synth_b200/lib
 LIB       := $(LIBDIR)/libvoicesynth_cuda.so
 CSRC      := voice_synth_b200/csrc
-SRCS      := $(CSRC)/vs_api.cu $(CSRC)/vs_plan.cu $(CSRC)/vs_render.cu $(CSRC)/vs_flow_rows.cu $(CSRC)/vs_analyze.cu
+SRCS      := $(CSRC)/vs_api.cu $(CSRC)/vs_batch_plan.cpp $(CSRC)/vs_plan.cu $(CSRC)/vs_render.cu $(CSRC)/vs_flow_rows.cu $(CSRC)/vs_analyze.cu
 OBJDIR    := build/obj
-OBJS      := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(SRCS))
+OBJS      := $(patsubst $(CSRC)/%,$(OBJDIR)/%.o,$(basename $(SRCS)))
 HDRS      := include/voicesynth.h $(CSRC)/vs_internal.h $(CSRC)/vs_presets.h $(CSRC)/vs_device.cuh
 
 all: lib host oracle
@@ -19,6 +19,11 @@ lib:
 $(OBJDIR)/%.o: $(CSRC)/%.cu $(HDRS)
 	mkdir -p $(OBJDIR)
 	$(NVCC) $(NVFLAGS) -c -o $@ $<
+# the batch planner is host code: the same host flags through nvcc (-O3, -ffp-contract=off)
+$(OBJDIR)/%.o: $(CSRC)/%.cpp $(HDRS)
+	mkdir -p $(OBJDIR)
+	$(NVCC) $(NVFLAGS) -c -o $@ $<
+$(OBJDIR)/vs_api.o $(OBJDIR)/vs_batch_plan.o: $(CSRC)/vs_batch_plan.h
 $(LIB): $(OBJS)
 	mkdir -p $(LIBDIR)
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(OBJS)

@@ -115,6 +115,7 @@ typedef struct vs_timing {
     uint64_t d2h_bytes;       /* device->host bytes the call copied (PCM, raw, period log)         */
     uint32_t render_path;     /* which render kernel ran (last launch): bit 0 = branch-free generator, bit 1 = glottal-noise
                                  variant, bits 2-3 = filter arithmetic (0 integer pre-emphasis, 1 FMA, 2 exact),
+                                 bit 5 = flow only on the warp-per-row kernel (lanes along the row),
                                  bit 6 = caller-defined tract coefficients (vs_*_batch_tract)                          */
     uint32_t reserved;
 } vs_timing;
@@ -124,7 +125,7 @@ typedef struct vs_timing {
 #define VS_OPT_CARRY_TOL       2  /* relative size the free response must decay to during warm-up (1e-12) */
 #define VS_OPT_EXACT_FILTER    3  /* 1: unfused mul+sub in the reference's order (bit-exact, 2x FP64 work, no chunking) */
 #define VS_OPT_SLAB_STREAMS    4  /* streams per launch/copy slab for host outputs; 0 = auto            */
-#define VS_OPT_TARGET_WARPS    5  /* auto-chunking aims at this many warps per SM sub-partition (2)      */
+#define VS_OPT_TARGET_WARPS    5  /* no effect; a value > 0 is accepted for compatibility                */
 #define VS_OPT_ASYNC_HOST      7  /* 1: calls with PINNED host buffers also return after enqueueing; the
                                      PCM of call k crosses PCIe while call k+1 renders (two device
                                      scratch buffers alternate).  vs_sync() before reading.  (0)          */

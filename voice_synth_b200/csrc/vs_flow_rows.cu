@@ -21,7 +21,6 @@
  * instruction F2I.F64 runs on the quarter-rate XU pipe, which would bind this kernel.  |A*table| < 2^31 holds for
  * every stream row_validate() accepts with T2 >= 2 (the host sends other batches to the lane-per-row kernel).
  * ============================================================================================== */
-#define VS_FLOWROWS_WARPS 8
 #define VS_SPAN 256            /* samples per warp step: 32 lanes x 4 pairs */
 
 __device__ __forceinline__ int vs_ceil_magic(double p)
@@ -65,7 +64,7 @@ __global__ void __launch_bounds__(VS_FLOWROWS_WARPS * 32, 4) vs_flow_rows_kernel
         }
         int16_t *orow = a.pcm_out + st->out_off;
         const uint2 *ptab = reinterpret_cast<const uint2 *>(a.table) + st->tab_off;           /* VsPeriodC */
-        /* the pulse table: n2 entries, two zeros, and the same again moved up by one entry (vs_api.cu, pulse_table_for) */
+        /* the pulse table: n2 entries, two zeros, and the same again moved up by one entry (vs_batch_plan.cpp, VsTables::pulse_table) */
         const double *tab = a.costab + st->pulse_off;
         const uint32_t n2 = 2u * (uint32_t)st->T2;
         const int DCs = st->DCs;
@@ -176,5 +175,4 @@ cudaError_t vs_launch_flow_rows(const VsRenderArgs &a, cudaStream_t s)
     vs_flow_rows_kernel<<<a.grid, VS_FLOWROWS_WARPS * 32, 0, s>>>(a);
     return cudaGetLastError();
 }
-int vs_flow_rows_warps(void) { return VS_FLOWROWS_WARPS; }
 

@@ -1,4 +1,4 @@
-/* vs_internal.h -- structures shared by the host side (vs_api.cu) and the kernels (vs_kernels.cu).
+/* vs_internal.h -- structures shared by the host side (vs_api.cu, vs_batch_plan.cpp) and the kernels.
  * Not part of the ABI. */
 #ifndef VS_INTERNAL_H
 #define VS_INTERNAL_H
@@ -29,6 +29,16 @@
 #define VS_WIN_SYNTH  168
 #define VS_WIN_FLOW   120
 #define VS_WIN_FILTER 120
+
+/* what a batch call computes, which generator the render kernel uses for the flow, and how it filters */
+enum { VS_MODE_FLOW = 0, VS_MODE_SYNTH = 1, VS_MODE_FILTER = 2 };
+enum { VS_GEN_FAST = 0, VS_GEN_SIMPLE = 1 };
+enum { VS_FILT_INT = 0, VS_FILT_FMA = 1, VS_FILT_EXACT = 2 };
+#define VS_WIN(MODE) ((MODE) == VS_MODE_SYNTH ? VS_WIN_SYNTH : (MODE) == VS_MODE_FLOW ? VS_WIN_FLOW : VS_WIN_FILTER)
+/* tiles per 32 rows of the render kernel.  Fused / filter-only: F's, G's and the one the TMA engine reads.  Flow
+ * only: one -- four CTAs share an SM and the other warps run while a warp waits for its tile to be read out */
+#define VS_RENDER_TILES(MODE) ((MODE) == VS_MODE_FLOW ? 1 : 3)
+#define VS_FLOWROWS_WARPS 8     /* warps per CTA of vs_flow_rows_kernel, one row each at a time */
 
 /* per-stream descriptor, prepared on the host, read once per thread */
 struct VsStream {
@@ -129,7 +139,7 @@ struct VsRenderArgs {
     int             general_pulse;  /* 1: some stream has -z Kvar > 0, its falling branch needs Knew of each period; 0: every
                                        pulse_off table already holds K*c - K + 1, a sample is ceil(A * table[i])              */
     int32_t        *status;         /* device error flag (shared with the plan kernel)              */
-    /* shared-memory geometry chosen by the host (vs_api.cu, render_geometry) */
+    /* shared-memory geometry chosen by the host (vs_batch_plan.cpp, vs_render_geometry) */
     uint32_t        warp_bytes;     /* per-warp region: 2 tiles | period ring | pulse-table cache    */
     uint32_t        ring_R;         /* period-ring entries per lane (power of two)                   */
     uint32_t        ring_fetch;     /* entries a lane may fetch per window                           */

@@ -33,11 +33,6 @@ static_assert(VS_NUM_PRESETS == VS_NUM_PRESETS_I, "preset count");
 
 __constant__ double c_ncoef[VS_NUM_PRESETS][VS_RING];      /* c_ncoef[p][j] = -A_p[j], j = 1..22 (vowel_new.c:450-544) */
 
-enum { VS_MODE_FLOW = 0, VS_MODE_SYNTH = 1, VS_MODE_FILTER = 2 };
-enum { VS_GEN_FAST = 0, VS_GEN_SIMPLE = 1 };
-enum { VS_FILT_INT = 0, VS_FILT_FMA = 1, VS_FILT_EXACT = 2 };
-
-__host__ __device__ constexpr int vs_win(int mode) { return mode == VS_MODE_SYNTH ? VS_WIN_SYNTH : (mode == VS_MODE_FLOW ? VS_WIN_FLOW : VS_WIN_FILTER); }
 #define VS_BIG_T 0x3fffffff
 #define VS_GROUP 8
 
@@ -179,9 +174,6 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
 }
 
 #define VS_RENDER_THREADS(MODE) ((MODE) == VS_MODE_FLOW ? VS_NT : 2 * VS_NT)
-/* tiles per 32 rows.  Fused / filter-only: F's, G's and the one the TMA engine reads.  Flow only: one -- four CTAs
- * share an SM and the other warps run while a warp waits for its tile to be read out */
-#define VS_RENDER_TILES(MODE)   ((MODE) == VS_MODE_FLOW ? 1 : 3)
 
 /* the second parameter block: the caller's vocal tracts (vs_*_batch_tract), nothing for the preset kernels */
 struct VsNoTracts {};
@@ -191,7 +183,7 @@ template <int MODE, int GEN, bool NOISE, int FILT, bool RAW, bool TRACT>
 __global__ void __launch_bounds__(VS_RENDER_THREADS(MODE), MODE == VS_MODE_FLOW ? 4 : 1)
 vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRACT> tr)
 {
-    constexpr int WIN = vs_win(MODE), TSB = WIN * 2, TILE = 32 * TSB, NGRP = WIN / VS_GROUP;
+    constexpr int WIN = VS_WIN(MODE), TSB = WIN * 2, TILE = 32 * TSB, NGRP = WIN / VS_GROUP;
     constexpr int NT = VS_RENDER_TILES(MODE);
     constexpr bool HASGEN = MODE != VS_MODE_FILTER, HASFILT = MODE != VS_MODE_FLOW;
     constexpr bool FAST = HASGEN && GEN == VS_GEN_FAST;
@@ -656,9 +648,6 @@ cudaError_t vs_render_init_device()
         for (int j = 0; j < VS_RING; j++) h[p][j] = j <= VS_ORDER ? -vs_preset_den[p][j] : 0.0;
     return cudaMemcpyToSymbol(c_ncoef, h, sizeof h);
 }
-
-int vs_render_window(int mode) { return vs_win(mode); }
-int vs_render_tiles(int mode) { return VS_RENDER_TILES(mode); }
 
 template <int MODE, int GEN, bool NOISE, int FILT, bool RAW, bool TRACT = false>
 static cudaError_t vs_go(const VsRenderArgs &a, const VsTractBlock *tb, cudaStream_t s)

@@ -13,7 +13,7 @@ def shard_range(n, rank, world):
 
 def shard_by_samples(nsamples, world):
     """cut points [world+1] over streams such that every rank gets ~the same number of samples
-    (the rule vs_api.cu applies to the device slots of one ctx)"""
+    (the rule vs_split_slots in vs_batch_plan.cpp applies to the device slots of one ctx)"""
     ns = np.asarray(nsamples, dtype=np.uint64)
     total = int(ns.sum())
     cuts = [0]
