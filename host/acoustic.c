@@ -2,9 +2,11 @@
  * (SURVEY.md 8f N4).  The reference's README (:14-16) describes `acoustic` analysis tools that are not in its tree;
  * this one makes the measurements vs_flow_analyze_batch() defines (include/voicesynth.h).
  *
- *   acoustic [-l lo] [-h hi] file.wav [file.wav ...]      thresholds of the onset trigger (default 0 0; with glottal
+ *   acoustic [-l lo] [-h hi] [-x] file.wav [file.wav ...]  thresholds of the onset trigger (default 0 0; with glottal
  *                                                          noise: above the noise, below the weakest pulse)
- * One line per file:  name  fs  samples  cycles  F0[Hz]  jitter[%]  shimmer[%]  mean_period  mean_peak */
+ * One line per file:  name  fs  samples  cycles  F0[Hz]  jitter[%]  shimmer[%]  mean_period  mean_peak
+ * -x (voice report, vs_flow_report_batch) appends ten columns:  jitter_abs[us]  RAP[%]  PPQ5[%]  DDP[%]  shimmer[dB]
+ *    APQ3[%]  APQ5[%]  APQ11[%]  DDA[%]  HNR[dB]   (nan where a measure needs more cycles, see include/voicesynth.h) */
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -14,13 +16,21 @@
 
 int main(int argc, char **argv)
 {
-    int lo = 0, hi = 0, a = 1;
-    while (a + 1 < argc && argv[a][0] == '-' && (argv[a][1] == 'l' || argv[a][1] == 'h') && argv[a][2] == 0) {
-        if (argv[a][1] == 'l') lo = atoi(argv[a + 1]); else hi = atoi(argv[a + 1]);
-        a += 2;
+    int lo = 0, hi = 0, a = 1, report = 0;
+    for (;;) {
+        if (a < argc && strcmp(argv[a], "-x") == 0) {
+            report = 1;
+            a += 1;
+        } else if (a + 1 < argc && argv[a][0] == '-' && (argv[a][1] == 'l' || argv[a][1] == 'h') && argv[a][2] == 0) {
+            if (argv[a][1] == 'l') lo = atoi(argv[a + 1]); else hi = atoi(argv[a + 1]);
+            a += 2;
+        } else {
+            break;
+        }
     }
     if (a >= argc || lo > hi || lo < -32768 || hi > 32767) {
-        printf("usage: acoustic [-l lo] [-h hi] file.wav [file.wav ...]   (lo <= hi: thresholds of the onset trigger)\n");
+        printf("usage: acoustic [-l lo] [-h hi] [-x] file.wav [file.wav ...]   (lo <= hi: thresholds of the onset trigger;"
+               " -x: voice report columns)\n");
         return 0;
     }
     const size_t n = (size_t)(argc - a);
@@ -49,14 +59,22 @@ int main(int argc, char **argv)
     int rc = vs_ctx_create(&ctx, &dev, 1, 0);
     if (rc) { fprintf(stderr, "acoustic: no CUDA device: %s\n", vs_strerror(rc)); return 1; }
     vs_flow_stats *st = (vs_flow_stats *)calloc(n, sizeof *st);
-    rc = vs_flow_analyze_batch(ctx, flow, offs, ns, fs, tl, th, n, st);
+    vs_flow_report *rp = report ? (vs_flow_report *)calloc(n, sizeof *rp) : NULL;
+    rc = report ? vs_flow_report_batch(ctx, flow, offs, ns, fs, tl, th, n, rp) : vs_flow_analyze_batch(ctx, flow, offs, ns, fs, tl, th, n, st);
     if (rc) { fprintf(stderr, "acoustic: %s (%s)\n", vs_strerror(rc), vs_last_error(ctx)); return 1; }
     for (size_t i = 0; i < n; i++) {
-        if (st[i].flags & VS_STATS_OVERFLOW)
+        if (report) st[i] = rp[i].base;
+        if (st[i].flags & VS_STATS_OVERFLOW) {
             printf("%s %d %llu: %u onsets -- the thresholds lie inside an oscillation, raise them\n", argv[a + i], fs[i], (unsigned long long)ns[i], st[i].onsets);
-        else
-            printf("%s %d %llu %u %.3f %.4f %.4f %.3f %.2f\n", argv[a + i], fs[i], (unsigned long long)ns[i], st[i].cycles,
-                   st[i].f0_hz, st[i].jitter_pct, st[i].shimmer_pct, st[i].mean_period, st[i].mean_peak);
+            continue;
+        }
+        printf("%s %d %llu %u %.3f %.4f %.4f %.3f %.2f", argv[a + i], fs[i], (unsigned long long)ns[i], st[i].cycles,
+               st[i].f0_hz, st[i].jitter_pct, st[i].shimmer_pct, st[i].mean_period, st[i].mean_peak);
+        if (report)
+            printf(" %.3f %.4f %.4f %.4f %.4f %.4f %.4f %.4f %.4f %.3f", rp[i].jitter_abs_us, rp[i].jitter_rap_pct, rp[i].jitter_ppq5_pct,
+                   rp[i].jitter_ddp_pct, rp[i].shimmer_db, rp[i].shimmer_apq3_pct, rp[i].shimmer_apq5_pct, rp[i].shimmer_apq11_pct,
+                   rp[i].shimmer_dda_pct, rp[i].hnr_db);
+        printf("\n");
     }
     vs_ctx_destroy(ctx);
     return 0;

@@ -201,6 +201,42 @@ typedef struct vs_flow_stats {
 int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp,
                           const int32_t *fs, const int16_t *lo, const int16_t *hi, size_t n, vs_flow_stats *stats);
 
+/* Voice report: vs_flow_stats plus the perturbation quotients of Praat's voice report and a cycle-synchronous
+ * harmonics-to-noise ratio.  Same arguments, checks and error codes as vs_flow_analyze_batch; `base` is byte for
+ * byte what that call returns for the same stream and thresholds.  With K = base.cycles complete cycles k = 0..K-1
+ * of the trigger above, their lengths T_k, peaks P_k and means mean T, mean P (Praat's formulas, without its
+ * period-exclusion rules):
+ *   jitter_abs_us   = 1e6 * (sum_{k>=1} |T_k - T_k-1| / (K-1)) / fs                              K >= 2
+ *   jitter_rap_pct  = 100 * (sum_{k=1..K-2} |3 T_k - (T_k-1 + T_k + T_k+1)| / 3 / (K-2)) / mean T   K >= 3
+ *   jitter_ppq5_pct = the same with the 5-point window: k = 2..K-3, / 5 / (K-4)                 K >= 5
+ *   jitter_ddp_pct  = 100 * (sum_{k=1..K-2} |T_k+1 - 2 T_k + T_k-1| / (K-2)) / mean T  (= 3 * RAP)  K >= 3
+ *   shimmer_apq3_pct, shimmer_apq5_pct, shimmer_dda_pct: RAP, PPQ5 and DDP applied to P_k over mean P;
+ *   shimmer_apq11_pct: the 11-point window, k = 5..K-6, / 11 / (K-10), K >= 11; all four need mean P > 0
+ *   shimmer_db      = sum_{k>=1} |20 log10(P_k / P_k-1)| / (K-1)                      K >= 2 and every P_k > 0
+ *   hnr_db, by cycle-synchronous averaging (Yumoto, Gould and Baer 1982): L = hnr_len = min T_k; the cycles are
+ *   aligned at their onsets o_k, S_j = sum_k x[o_k + j] and E = sum_k sum_{j<L} x[o_k + j]^2 for j < L;
+ *     hnr_db = 10 log10( sum_j S_j^2 / (K E - sum_j S_j^2) ),  +inf when the denominator is 0;   K >= 2
+ *   The average of the aligned cycles is the harmonic part, the rest is noise.  Amplitude perturbation counts as
+ *   noise: 3 % shimmer alone brings a noise-free voice down to about 10 dB.  This generator's jitter only changes
+ *   the closed phase, after the first L samples of a cycle, so a jitter-only noise-free voice gives +inf.  For
+ *   noise-only voices hnr_db is the SNR of the period log, sum x_pow (T3 - T4) / sum w_pow T, within 0.1 dB
+ *   (about 2.2 dB below the -n value, which relates the open phase's power to the noise).
+ * Sums are exact integers (S_j and E in int64, K E and sum S_j^2 in 128 bits) up to the final FP64 quotient,
+ * except the logarithms of shimmer_db; each field is rounded to float.  A field whose condition fails is NaN;
+ * hnr_len is L when hnr_db is defined (K >= 2), else 0.  With VS_STATS_OVERFLOW in base.flags every new field is
+ * NaN and hnr_len is 0. */
+typedef struct vs_flow_report {
+    vs_flow_stats base;        /* what vs_flow_analyze_batch returns                          */
+    float    jitter_abs_us;    /* local absolute jitter                                       */
+    float    jitter_rap_pct, jitter_ppq5_pct, jitter_ddp_pct;
+    float    shimmer_db, shimmer_apq3_pct, shimmer_apq5_pct, shimmer_apq11_pct, shimmer_dda_pct;
+    float    hnr_db;           /* cycle-synchronous average, above                            */
+    uint32_t hnr_len;          /* L: samples per cycle the HNR compares                       */
+    uint32_t reserved;
+} vs_flow_report;              /* 80 bytes */
+int vs_flow_report_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp,
+                         const int32_t *fs, const int16_t *lo, const int16_t *hi, size_t n, vs_flow_report *out);
+
 /* SURVEY 8f N1 -- `vowel -n`: white noise added to already filtered PCM, IN PLACE (vowel_new.c:302-324).
  * Per stream and per frame of 50*((int)(fs*0.001/2.0)*2) samples: float power of the frame, uniform
  * noise of width sqrt(12*power/snr) drawn with random() seeded by srandom(seed[i]) (vowel_new.c:234),

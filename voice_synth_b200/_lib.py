@@ -8,7 +8,7 @@ EXPORTS = ["vs_abi_version", "vs_device_count", "vs_strerror", "vs_last_error", 
            "vs_ctx_set_option", "vs_ctx_set_stream", "vs_sync", "vs_get_timing", "vs_measure_fp64_peak", "vs_host_alloc", "vs_host_free",
            "vs_flow_nsamples", "vs_flow_max_periods", "vs_flow_validate", "vs_filter_warmup",
            "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch",
-           "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset"]
+           "vs_flow_report_batch", "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset"]
 
 
 class FlowParamsC(C.Structure):
@@ -76,6 +76,8 @@ def load():
                                  C.c_void_p, C.c_void_p, C.c_void_p]
     L.vs_flow_analyze_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_size_t, C.c_void_p]
+    L.vs_flow_report_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_size_t, C.c_void_p]
     L.vs_synth_batch_tract.argtypes = [C.c_void_p, C.POINTER(FlowParamsC), C.POINTER(TractParamsC), C.c_size_t,
                                        C.c_void_p, C.c_void_p, C.c_void_p]
     L.vs_vowel_filter_batch_tract.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(TractParamsC),

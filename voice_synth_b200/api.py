@@ -24,6 +24,11 @@ assert PERIOD_DTYPE.itemsize == 56
 FLOW_STATS_DTYPE = np.dtype([("onsets", "<u4"), ("cycles", "<u4"), ("flags", "<u4"), ("f0_hz", "<f4"), ("jitter_pct", "<f4"),
                              ("shimmer_pct", "<f4"), ("mean_period", "<f4"), ("mean_peak", "<f4")])
 assert FLOW_STATS_DTYPE.itemsize == 32
+FLOW_REPORT_DTYPE = np.dtype([("base", FLOW_STATS_DTYPE), ("jitter_abs_us", "<f4"), ("jitter_rap_pct", "<f4"),
+                              ("jitter_ppq5_pct", "<f4"), ("jitter_ddp_pct", "<f4"), ("shimmer_db", "<f4"),
+                              ("shimmer_apq3_pct", "<f4"), ("shimmer_apq5_pct", "<f4"), ("shimmer_apq11_pct", "<f4"),
+                              ("shimmer_dda_pct", "<f4"), ("hnr_db", "<f4"), ("hnr_len", "<u4"), ("reserved", "<u4")])
+assert FLOW_REPORT_DTYPE.itemsize == 80
 
 _FLOW_FIELDS = [("dur", np.float32, 1.0), ("jitter", np.float32, 0.0), ("shimmer", np.float32, 0.0),
                 ("cq", np.float32, 0.55), ("K", np.float32, 0.65), ("Kvar", np.float32, 0.0), ("F0", np.float32, 120.0),
@@ -387,16 +392,23 @@ class Context:
     def flow_analyze_batch(self, flow, nsamp, offsets=None, fs=None, lo=None, hi=None):
         """cycle-to-cycle analysis of glottal flow (SURVEY 8f N4, include/voicesynth.h): F0, local jitter and shimmer
         per stream as a structured array (FLOW_STATS_DTYPE). flow: numpy array or device tensor."""
+        return self._analysis(self.L.vs_flow_analyze_batch, FLOW_STATS_DTYPE, flow, nsamp, offsets, fs, lo, hi)
+
+    def flow_report_batch(self, flow, nsamp, offsets=None, fs=None, lo=None, hi=None):
+        """voice report of glottal flow (include/voicesynth.h): flow_analyze_batch's statistics in `base`, Praat's jitter
+        and shimmer quotients and a cycle-averaged HNR, per stream as a structured array (FLOW_REPORT_DTYPE)."""
+        return self._analysis(self.L.vs_flow_report_batch, FLOW_REPORT_DTYPE, flow, nsamp, offsets, fs, lo, hi)
+
+    def _analysis(self, call, dtype, flow, nsamp, offsets, fs, lo, hi):
         ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
         n = len(ns)
         offs = None if offsets is None else np.ascontiguousarray(offsets, dtype=np.uint64)
         rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), (n,)))
         tl = None if lo is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lo, dtype=np.int16), (n,)))
         th = None if hi is None else np.ascontiguousarray(np.broadcast_to(np.asarray(hi, dtype=np.int16), (n,)))
-        stats = np.zeros(n, dtype=FLOW_STATS_DTYPE)
-        self._check(self.L.vs_flow_analyze_batch(self.h, _ptr(flow), _ptr(offs), ns.ctypes.data, _ptr(rate), _ptr(tl), _ptr(th),
-                                                 n, stats.ctypes.data))
-        return stats
+        res = np.zeros(n, dtype=dtype)
+        self._check(call(self.h, _ptr(flow), _ptr(offs), ns.ctypes.data, _ptr(rate), _ptr(tl), _ptr(th), n, res.ctypes.data))
+        return res
 
     def synth_batch(self, p, f, out=None, offsets=None, want_raw=False):
         """f: FilterParams (the presets) or TractParams (caller-defined tracts, vs_synth_batch_tract)."""

@@ -23,6 +23,8 @@ cudaError_t vs_launch_fp64_peak(double *scratch, int blocks, int iters, cudaStre
 cudaError_t vs_launch_vnoise(int16_t *pcm, const VsNoiseRow *rows, uint32_t n_rows, cudaStream_t s);
 cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
                               vs_flow_stats *out, cudaStream_t s);
+cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
+                             vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
 
 namespace {
 
@@ -985,10 +987,11 @@ int vs_vowel_noise_batch(vs_ctx *ctx, int16_t *pcm, const uint64_t *offsets, con
     return VS_OK;
 }
 
-int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
-                          const int16_t *lo, const int16_t *hi, size_t n, vs_flow_stats *stats)
+/* vs_flow_analyze_batch (report NULL: stats is the caller's) and vs_flow_report_batch (stats NULL: the statistics
+ * stay on the device, the report kernel copies them into report[i].base) */
+static int flow_analysis(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                         const int16_t *lo, const int16_t *hi, size_t n, vs_flow_stats *stats, vs_flow_report *report)
 {
-    if (!ctx || !flow || !nsamp || !stats) return VS_EINVAL;
     if (n == 0) return VS_OK;
     if (n > 0x7fffffffull) return fail(ctx, VS_EINVAL, "too many streams");
     int rc = vs_sync(ctx);                                    /* the flow may be the output of a call still in flight */
@@ -1018,10 +1021,12 @@ int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offs
     int dev = -1;
     const bool on_dev = classify(flow, &dev) == PK_DEVICE;
     if (on_dev && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
-    /* scratch: rows | per-stream onset counts | stats | onset lists */
+    /* scratch: rows | per-stream onset counts | stats | onset lists, and for the report: | peak lists | reports */
     const size_t rows_b = (n * sizeof(VsAnalyzeRow) + 255) & ~(size_t)255, cnt_b = (n * sizeof(uint32_t) + 255) & ~(size_t)255;
     const size_t st_b = (n * sizeof(vs_flow_stats) + 255) & ~(size_t)255;
-    if ((rc = dev_reserve(ctx, sl, sl.analyze, rows_b + cnt_b + st_b + slots * sizeof(uint32_t)))) return rc;
+    const size_t ons_b = (slots * sizeof(uint32_t) + 255) & ~(size_t)255;
+    const size_t rep_b = report ? ons_b + n * sizeof(vs_flow_report) : 0;
+    if ((rc = dev_reserve(ctx, sl, sl.analyze, rows_b + cnt_b + st_b + (report ? ons_b : slots * sizeof(uint32_t)) + rep_b))) return rc;
     unsigned char *base = (unsigned char *)sl.analyze.p;
     CU(cudaMemcpyAsync(base, rows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, sl.compute));
     const int16_t *d_flow = flow;
@@ -1030,11 +1035,33 @@ int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offs
         d_flow = (const int16_t *)sl.pcm[0].p - first;
         CU(cudaMemcpyAsync(sl.pcm[0].p, flow + first, (last - first) * sizeof(int16_t), cudaMemcpyHostToDevice, sl.compute));
     }
-    CU(vs_launch_analyze(d_flow, (const VsAnalyzeRow *)base, (uint32_t)n, (uint32_t *)(base + rows_b + cnt_b + st_b),
-                         (uint32_t *)(base + rows_b), (vs_flow_stats *)(base + rows_b + cnt_b), sl.compute));
-    CU(cudaMemcpyAsync(stats, base + rows_b + cnt_b, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, sl.compute));
-    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` and `stats` are the caller's / pageable memory */
+    if (!report) {
+        CU(vs_launch_analyze(d_flow, (const VsAnalyzeRow *)base, (uint32_t)n, (uint32_t *)(base + rows_b + cnt_b + st_b),
+                             (uint32_t *)(base + rows_b), (vs_flow_stats *)(base + rows_b + cnt_b), sl.compute));
+        CU(cudaMemcpyAsync(stats, base + rows_b + cnt_b, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, sl.compute));
+    } else {
+        unsigned char *peaks = base + rows_b + cnt_b + st_b + ons_b, *reps = peaks + ons_b;
+        CU(vs_launch_report(d_flow, (const VsAnalyzeRow *)base, (uint32_t)n, (uint32_t *)(base + rows_b + cnt_b + st_b),
+                            (uint32_t *)(base + rows_b), (vs_flow_stats *)(base + rows_b + cnt_b), (int32_t *)peaks,
+                            (vs_flow_report *)reps, sl.compute));
+        CU(cudaMemcpyAsync(report, reps, n * sizeof(vs_flow_report), cudaMemcpyDeviceToHost, sl.compute));
+    }
+    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` and the results are the caller's / pageable memory */
     return VS_OK;
+}
+
+int vs_flow_analyze_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                          const int16_t *lo, const int16_t *hi, size_t n, vs_flow_stats *stats)
+{
+    if (!ctx || !flow || !nsamp || !stats) return VS_EINVAL;
+    return flow_analysis(ctx, flow, offsets, nsamp, fs, lo, hi, n, stats, nullptr);
+}
+
+int vs_flow_report_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                         const int16_t *lo, const int16_t *hi, size_t n, vs_flow_report *out)
+{
+    if (!ctx || !flow || !nsamp || !out) return VS_EINVAL;
+    return flow_analysis(ctx, flow, offsets, nsamp, fs, lo, hi, n, nullptr, out);
 }
 
 int vs_synth_batch(vs_ctx *ctx, const vs_flow_params *p, const vs_filter_params *f, size_t n, int16_t *pcm_out,
