@@ -7,7 +7,8 @@ NVFLAGS   := -O3 -std=c++17 $(ARCH) -lineinfo -fmad=false -cudart static \
 LIBDIR    := voice_synth_b200/lib
 LIB       := $(LIBDIR)/libvoicesynth_cuda.so
 CSRC      := voice_synth_b200/csrc
-SRCS      := $(CSRC)/vs_api.cu $(CSRC)/vs_batch_plan.cpp $(CSRC)/vs_plan.cu $(CSRC)/vs_render.cu $(CSRC)/vs_flow_rows.cu $(CSRC)/vs_analyze.cu
+SRCS      := $(CSRC)/vs_api.cu $(CSRC)/vs_batch_plan.cpp $(CSRC)/vs_plan.cu $(CSRC)/vs_render.cu $(CSRC)/vs_flow_rows.cu $(CSRC)/vs_analyze.cu \
+             $(CSRC)/vs_formants.cu
 OBJDIR    := build/obj
 OBJS      := $(patsubst $(CSRC)/%,$(OBJDIR)/%.o,$(basename $(SRCS)))
 HDRS      := include/voicesynth.h $(CSRC)/vs_internal.h $(CSRC)/vs_presets.h $(CSRC)/vs_device.cuh

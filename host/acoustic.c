@@ -6,7 +6,12 @@
  *                                                          noise: above the noise, below the weakest pulse)
  * One line per file:  name  fs  samples  cycles  F0[Hz]  jitter[%]  shimmer[%]  mean_period  mean_peak
  * -x (voice report, vs_flow_report_batch) appends ten columns:  jitter_abs[us]  RAP[%]  PPQ5[%]  DDP[%]  shimmer[dB]
- *    APQ3[%]  APQ5[%]  APQ11[%]  DDA[%]  HNR[dB]   (nan where a measure needs more cycles, see include/voicesynth.h) */
+ *    APQ3[%]  APQ5[%]  APQ11[%]  DDA[%]  HNR[dB]   (nan where a measure needs more cycles, see include/voicesynth.h)
+ *
+ *   acoustic -F [-p order] file.wav [file.wav ...]         formant analysis of vowel PCM (vs_formant_batch, default
+ *                                                          options; -p sets the LPC order, 2..32, even)
+ * One line per file:  name  fs  samples  frames  analysed  F1..Fn[Hz]  B1..Bn[Hz]   (the means over the analysed frames,
+ *    n = min(5, order/2); nan where no frame has that many formants) */
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -16,11 +21,17 @@
 
 int main(int argc, char **argv)
 {
-    int lo = 0, hi = 0, a = 1, report = 0;
+    int lo = 0, hi = 0, a = 1, report = 0, formants = 0, order = 14;
     for (;;) {
         if (a < argc && strcmp(argv[a], "-x") == 0) {
             report = 1;
             a += 1;
+        } else if (a < argc && strcmp(argv[a], "-F") == 0) {
+            formants = 1;
+            a += 1;
+        } else if (a + 1 < argc && strcmp(argv[a], "-p") == 0) {
+            order = atoi(argv[a + 1]);
+            a += 2;
         } else if (a + 1 < argc && argv[a][0] == '-' && (argv[a][1] == 'l' || argv[a][1] == 'h') && argv[a][2] == 0) {
             if (argv[a][1] == 'l') lo = atoi(argv[a + 1]); else hi = atoi(argv[a + 1]);
             a += 2;
@@ -28,9 +39,10 @@ int main(int argc, char **argv)
             break;
         }
     }
-    if (a >= argc || lo > hi || lo < -32768 || hi > 32767) {
+    if (a >= argc || lo > hi || lo < -32768 || hi > 32767 || order < 2 || order > 32 || order % 2) {
         printf("usage: acoustic [-l lo] [-h hi] [-x] file.wav [file.wav ...]   (lo <= hi: thresholds of the onset trigger;"
-               " -x: voice report columns)\n");
+               " -x: voice report columns)\n"
+               "       acoustic -F [-p order] file.wav [file.wav ...]          (formants of vowel PCM; order even, 2..32)\n");
         return 0;
     }
     const size_t n = (size_t)(argc - a);
@@ -58,6 +70,20 @@ int main(int argc, char **argv)
     vs_ctx *ctx = NULL;
     int rc = vs_ctx_create(&ctx, &dev, 1, 0);
     if (rc) { fprintf(stderr, "acoustic: no CUDA device: %s\n", vs_strerror(rc)); return 1; }
+    if (formants) {
+        vs_formant_opts fo = {25.0f, 10.0f, 50.0f, 700.0f, (uint32_t)order, (uint32_t)(order / 2 < 5 ? order / 2 : 5)};
+        vs_formant_stats *fs_out = (vs_formant_stats *)calloc(n, sizeof *fs_out);
+        rc = vs_formant_batch(ctx, flow, offs, ns, fs, n, &fo, fs_out, NULL, NULL);
+        if (rc) { fprintf(stderr, "acoustic: %s (%s)\n", vs_strerror(rc), vs_last_error(ctx)); return 1; }
+        for (size_t i = 0; i < n; i++) {
+            printf("%s %d %llu %u %u", argv[a + i], fs[i], (unsigned long long)ns[i], fs_out[i].frames, fs_out[i].analysed);
+            for (uint32_t k = 0; k < fo.n_formants; k++) printf(" %.1f", fs_out[i].f_mean_hz[k]);
+            for (uint32_t k = 0; k < fo.n_formants; k++) printf(" %.1f", fs_out[i].bw_mean_hz[k]);
+            printf("\n");
+        }
+        vs_ctx_destroy(ctx);
+        return 0;
+    }
     vs_flow_stats *st = (vs_flow_stats *)calloc(n, sizeof *st);
     vs_flow_report *rp = report ? (vs_flow_report *)calloc(n, sizeof *rp) : NULL;
     rc = report ? vs_flow_report_batch(ctx, flow, offs, ns, fs, tl, th, n, rp) : vs_flow_analyze_batch(ctx, flow, offs, ns, fs, tl, th, n, st);

@@ -237,6 +237,68 @@ typedef struct vs_flow_report {
 int vs_flow_report_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offsets, const uint64_t *nsamp,
                          const int32_t *fs, const int16_t *lo, const int16_t *hi, size_t n, vs_flow_report *out);
 
+/* Formant analysis of PCM (vowels rendered by vs_synth_batch, vs_vowel_filter_batch and their tract forms): frame-wise
+ * LPC, its poles, and per-stream formant statistics.  The definitions are this library's own (the reference has no
+ * formant tool); tests/formant_ref.py restates them in numpy.  With fs the stream's rate (fs NULL: 22050 for every
+ * stream) and p = order:
+ *   frames     Nw = lround(win_ms fs / 1000), H = lround(hop_ms fs / 1000), in double; a stream of n samples has
+ *              n >= Nw ? (n - Nw) / H + 1 : 0 frames, frame f covers samples [f H, f H + Nw);
+ *   signal     y[m] = (x[fH+m] - mu x[fH+m-1]) w[m], m = 0..Nw-1, in FP64, mu = exp(-2 pi preemph_hz / fs) (0 when
+ *              preemph_hz is 0), w[m] = 0.54 - 0.46 cos(2 pi m / (Nw - 1)); x[-1] = 0 only at the stream's first
+ *              sample.  w and mu are computed on the host with libm in double;
+ *   LPC        r[k] = sum_m y[m] y[m+k], k = 0..p, FP64 in any order; r[0] == 0: the frame is VS_FRAME_SILENT.
+ *              Levinson-Durbin gives A(z) = 1 + a1 z^-1 + ... + ap z^-p; a reflection coefficient with |k_i| >= 1 or a
+ *              prediction error <= 0: VS_FRAME_SINGULAR (a numerical guard: for a frame that is not all zero the
+ *              autocorrelation matrix is positive definite, and no input is known to reach it);
+ *   poles      all p roots of z^p + a1 z^(p-1) + ... + ap in FP64 (Aberth-Ehrlich from 0.9 exp(i (2 pi j / p + 0.4)),
+ *              until every root's correction is at most 1e-13 of its modulus, at most 64 iterations, then one Newton
+ *              step; more iterations needed: VS_FRAME_NOCONV).  Each root with Im z > 0 gives
+ *              F = atan2(Im z, Re z) fs / (2 pi) and B = -ln|z| fs / pi; kept when 50 < F < fs/2 - 50 and, when
+ *              bmax_hz > 0, B < bmax_hz; sorted by ascending F, the first n_formants are the frame's formants;
+ *   frames[]   f_hz[k], bw_hz[k] for k < found (float), NaN past it; a flagged frame has found = 0;
+ *   stats      over the frames without a flag ("analysed"): count[k] = frames with found > k, the mean of F_k, its
+ *              sample SD (NaN for count[k] < 2) and the mean of B_k, in FP64 from the unrounded values, each rounded
+ *              to float; NaN where count[k] == 0.  frames = the stream's frames, unconverged = its VS_FRAME_NOCONV
+ *              frames.
+ * Errors (vs_formant_frames returns the same ones, in the same order): NULL ctx / pcm / nsamp / stats, an odd order or
+ * one outside 2..32, n_formants outside 1..VS_MAX_FORMANTS or above p/2 -> VS_EINVAL; a negative (or NaN) preemph_hz
+ * or bmax_hz, then per stream in index order: a row above 2^31-1 samples -> VS_EOVERLAP; fs <= 0, Nw < p+1,
+ * Nw > VS_FORMANT_MAX_WIN (the kernel stages a frame in shared memory), H < 1 or H > 2^31-1 -> VS_ERANGE.
+ * pcm may be host or device memory (as for vs_flow_analyze_batch); offsets NULL: dense rows of stride max nsamp.
+ * stats [n] and frames are host memory; stream i's frames go to frames + frame_offsets[i] (frame_offsets NULL: the
+ * prefix sum of the frame counts, densely packed); frames NULL: no per-frame output, the statistics are the same. */
+#define VS_MAX_FORMANTS     8
+#define VS_FORMANT_MAX_WIN  4096
+#define VS_FRAME_SILENT     1u
+#define VS_FRAME_SINGULAR   2u
+#define VS_FRAME_NOCONV     4u
+typedef struct vs_formant_opts {      /* NULL = all defaults; a non-NULL struct is taken literally    */
+    float    win_ms;                  /* Hamming window length (25)                                   */
+    float    hop_ms;                  /* frame step (10)                                              */
+    float    preemph_hz;              /* pre-emphasis corner, 0 = none (50)                           */
+    float    bmax_hz;                 /* drop poles with bandwidth >= bmax; 0 = no limit (700)        */
+    uint32_t order;                   /* LPC order p, even, 2..32 (14)                                */
+    uint32_t n_formants;              /* 1..VS_MAX_FORMANTS and <= p/2 (5)                            */
+} vs_formant_opts;
+
+typedef struct vs_formant_frame {     /* 72 bytes */
+    float    f_hz[VS_MAX_FORMANTS], bw_hz[VS_MAX_FORMANTS];   /* ascending F; NaN past `found`                */
+    uint32_t found;                   /* formants found in the frame                                  */
+    uint32_t flags;                   /* VS_FRAME_SILENT | VS_FRAME_SINGULAR | VS_FRAME_NOCONV        */
+} vs_formant_frame;
+
+typedef struct vs_formant_stats {     /* 144 bytes */
+    uint32_t frames, analysed, unconverged, reserved;
+    uint32_t count[VS_MAX_FORMANTS];  /* analysed frames with found > k                               */
+    float    f_mean_hz[VS_MAX_FORMANTS], f_sd_hz[VS_MAX_FORMANTS], bw_mean_hz[VS_MAX_FORMANTS];
+} vs_formant_stats;
+
+/* host only: validates exactly as vs_formant_batch does (first offender -> its error) and returns frames per stream */
+int vs_formant_frames(const vs_formant_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *frames_out);
+int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                     size_t n, const vs_formant_opts *o, vs_formant_stats *stats,
+                     vs_formant_frame *frames, const uint64_t *frame_offsets);
+
 /* SURVEY 8f N1 -- `vowel -n`: white noise added to already filtered PCM, IN PLACE (vowel_new.c:302-324).
  * Per stream and per frame of 50*((int)(fs*0.001/2.0)*2) samples: float power of the frame, uniform
  * noise of width sqrt(12*power/snr) drawn with random() seeded by srandom(seed[i]) (vowel_new.c:234),

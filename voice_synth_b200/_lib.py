@@ -8,7 +8,8 @@ EXPORTS = ["vs_abi_version", "vs_device_count", "vs_strerror", "vs_last_error", 
            "vs_ctx_set_option", "vs_ctx_set_stream", "vs_sync", "vs_get_timing", "vs_measure_fp64_peak", "vs_host_alloc", "vs_host_free",
            "vs_flow_nsamples", "vs_flow_max_periods", "vs_flow_validate", "vs_filter_warmup",
            "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch",
-           "vs_flow_report_batch", "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset"]
+           "vs_flow_report_batch", "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset",
+           "vs_formant_frames", "vs_formant_batch"]
 
 
 class FlowParamsC(C.Structure):
@@ -22,6 +23,11 @@ class FilterParamsC(C.Structure):
 
 class TractParamsC(C.Structure):
     _fields_ = [("den", C.c_void_p), ("n_tracts", C.c_uint32), ("tract", C.c_void_p), ("gain", C.c_void_p), ("pre", C.c_void_p)]
+
+
+class FormantOptsC(C.Structure):
+    _fields_ = [("win_ms", C.c_float), ("hop_ms", C.c_float), ("preemph_hz", C.c_float), ("bmax_hz", C.c_float),
+                ("order", C.c_uint32), ("n_formants", C.c_uint32)]
 
 
 class PeriodLogC(C.Structure):
@@ -84,5 +90,8 @@ def load():
                                               C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]
     L.vs_tract_from_formants.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int32, C.c_void_p]
     L.vs_tract_from_preset.argtypes = [C.c_int, C.c_void_p]
+    L.vs_formant_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    L.vs_formant_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L

@@ -11,7 +11,7 @@ import re
 import numpy as np
 
 from . import _lib
-from ._lib import FilterParamsC, FlowParamsC, PeriodLogC, TimingC, TractParamsC
+from ._lib import FilterParamsC, FlowParamsC, FormantOptsC, PeriodLogC, TimingC, TractParamsC
 
 VS_F_JITTER, VS_F_SHIMMER, VS_F_NOISE = 1, 2, 4
 VS_OK, VS_EINVAL, VS_ERANGE, VS_EPRESET, VS_ENOMEM, VS_ECUDA, VS_ENODEV, VS_EOVERLAP = 0, -1, -2, -3, -4, -5, -6, -7
@@ -29,6 +29,16 @@ FLOW_REPORT_DTYPE = np.dtype([("base", FLOW_STATS_DTYPE), ("jitter_abs_us", "<f4
                               ("shimmer_apq3_pct", "<f4"), ("shimmer_apq5_pct", "<f4"), ("shimmer_apq11_pct", "<f4"),
                               ("shimmer_dda_pct", "<f4"), ("hnr_db", "<f4"), ("hnr_len", "<u4"), ("reserved", "<u4")])
 assert FLOW_REPORT_DTYPE.itemsize == 80
+MAX_FORMANTS = 8
+FRAME_SILENT, FRAME_SINGULAR, FRAME_NOCONV = 1, 2, 4
+FORMANT_FRAME_DTYPE = np.dtype([("f_hz", "<f4", (MAX_FORMANTS,)), ("bw_hz", "<f4", (MAX_FORMANTS,)), ("found", "<u4"),
+                                ("flags", "<u4")])
+assert FORMANT_FRAME_DTYPE.itemsize == 72
+FORMANT_STATS_DTYPE = np.dtype([("frames", "<u4"), ("analysed", "<u4"), ("unconverged", "<u4"), ("reserved", "<u4"),
+                                ("count", "<u4", (MAX_FORMANTS,)), ("f_mean_hz", "<f4", (MAX_FORMANTS,)),
+                                ("f_sd_hz", "<f4", (MAX_FORMANTS,)), ("bw_mean_hz", "<f4", (MAX_FORMANTS,))])
+assert FORMANT_STATS_DTYPE.itemsize == 144
+FORMANT_DEFAULTS = dict(win_ms=25.0, hop_ms=10.0, preemph_hz=50.0, bmax_hz=700.0, order=14, n_formants=5)
 
 _FLOW_FIELDS = [("dur", np.float32, 1.0), ("jitter", np.float32, 0.0), ("shimmer", np.float32, 0.0),
                 ("cq", np.float32, 0.55), ("K", np.float32, 0.65), ("Kvar", np.float32, 0.0), ("F0", np.float32, 120.0),
@@ -273,6 +283,28 @@ def flow_nsamples(p):
     return out
 
 
+def formant_opts(opts=None):
+    """vs_formant_opts from a dict of the fields to change (the rest keep FORMANT_DEFAULTS); None stays None (NULL)"""
+    if opts is None or isinstance(opts, FormantOptsC):
+        return opts
+    unknown = set(opts) - set(FORMANT_DEFAULTS)
+    if unknown:
+        raise ValueError(f"unknown formant options {sorted(unknown)}")
+    return FormantOptsC(**{**FORMANT_DEFAULTS, **opts})
+
+
+def formant_frames(nsamp, fs=None, opts=None):
+    """frames per stream of vs_formant_batch (host only, validates like the batch call; raises VsError)"""
+    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+    rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), ns.shape))
+    o = formant_opts(opts)
+    out = np.zeros(len(ns), dtype=np.uint64)
+    rc = _lib.load().vs_formant_frames(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
+    if rc:
+        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
+    return out
+
+
 def _ptr(x):
     """numpy array -> host pointer; int -> raw (device) pointer; object with data_ptr() -> torch tensor."""
     if x is None:
@@ -409,6 +441,26 @@ class Context:
         res = np.zeros(n, dtype=dtype)
         self._check(call(self.h, _ptr(flow), _ptr(offs), ns.ctypes.data, _ptr(rate), _ptr(tl), _ptr(th), n, res.ctypes.data))
         return res
+
+    def formant_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_frames=False):
+        """formant analysis (vs_formant_batch): per-stream statistics (FORMANT_STATS_DTYPE) and, with want_frames, the
+        list of each stream's frame records (FORMANT_FRAME_DTYPE).  pcm: numpy array or device tensor; opts: None (the
+        defaults) or a dict of the vs_formant_opts fields to change."""
+        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+        n = len(ns)
+        offs = None if offsets is None else np.ascontiguousarray(offsets, dtype=np.uint64)
+        rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), (n,)))
+        o = formant_opts(opts)
+        st = np.zeros(n, dtype=FORMANT_STATS_DTYPE)
+        fr, fo = None, None
+        if want_frames:
+            fo = np.concatenate([[0], np.cumsum(formant_frames(ns, fs, opts))]).astype(np.uint64)
+            fr = np.zeros(int(fo[-1]), dtype=FORMANT_FRAME_DTYPE)
+        self._check(self.L.vs_formant_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
+                                            None if o is None else C.byref(o), st.ctypes.data, _ptr(fr), None))
+        if want_frames:
+            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
+        return st
 
     def synth_batch(self, p, f, out=None, offsets=None, want_raw=False):
         """f: FilterParams (the presets) or TractParams (caller-defined tracts, vs_synth_batch_tract)."""

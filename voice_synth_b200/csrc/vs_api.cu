@@ -25,6 +25,7 @@ cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uin
                               vs_flow_stats *out, cudaStream_t s);
 cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
                              vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
+cudaError_t vs_launch_formants(const VsFormantArgs &a, vs_formant_stats *stats, vs_formant_frame *frames, cudaStream_t s);
 
 namespace {
 
@@ -1062,6 +1063,143 @@ int vs_flow_report_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offse
 {
     if (!ctx || !flow || !nsamp || !out) return VS_EINVAL;
     return flow_analysis(ctx, flow, offsets, nsamp, fs, lo, hi, n, nullptr, out);
+}
+
+/* the option and per-stream checks of vs_formant_frames and vs_formant_batch, in the header's order; fills o (the
+ * defaults for in == NULL) and, per stream, Nw, H and the frame count */
+static int formant_geometry(const vs_formant_opts *in, const uint64_t *nsamp, const int32_t *fs, size_t n, vs_formant_opts &o,
+                            uint32_t *Nw, uint32_t *H, uint64_t *frames, std::string *err)
+{
+    o = in ? *in : vs_formant_opts{25.0f, 10.0f, 50.0f, 700.0f, 14u, 5u};
+    if (o.order < 2 || o.order > VS_FMT_MAX_ORDER || (o.order & 1u)) return vs_error(err, VS_EINVAL, "order %u: even, 2..%d", o.order, VS_FMT_MAX_ORDER);
+    if (o.n_formants < 1 || o.n_formants > VS_MAX_FORMANTS || o.n_formants > o.order / 2)
+        return vs_error(err, VS_EINVAL, "n_formants %u: 1..%d and at most order / 2", o.n_formants, VS_MAX_FORMANTS);
+    if (!(o.preemph_hz >= 0.0f) || !(o.bmax_hz >= 0.0f)) return vs_error(err, VS_ERANGE, "preemph_hz and bmax_hz must be >= 0");
+    for (size_t i = 0; i < n; i++) {
+        if (nsamp[i] > 0x7fffffffull) return vs_error(err, VS_EOVERLAP, "stream %zu: too many samples", i);
+        const int32_t rate = fs ? fs[i] : 22050;
+        if (rate <= 0) return vs_error(err, VS_ERANGE, "stream %zu: sampling rate", i);
+        const double wl = (double)o.win_ms * rate / 1000.0, hl = (double)o.hop_ms * rate / 1000.0;
+        const long nw = wl > -1e9 && wl < 1e9 ? lround(wl) : -1;
+        if (nw < (long)o.order + 1 || nw > VS_FORMANT_MAX_WIN)
+            return vs_error(err, VS_ERANGE, "stream %zu: window of %ld samples, needs %u..%d", i, nw, o.order + 1, VS_FORMANT_MAX_WIN);
+        if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
+        const uint64_t h = (uint64_t)lround(hl);
+        if (Nw) Nw[i] = (uint32_t)nw;
+        if (H) H[i] = (uint32_t)h;
+        frames[i] = nsamp[i] >= (uint64_t)nw ? (nsamp[i] - (uint64_t)nw) / h + 1 : 0;
+    }
+    return VS_OK;
+}
+
+int vs_formant_frames(const vs_formant_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *frames_out)
+{
+    if (!nsamp || !frames_out) return VS_EINVAL;
+    vs_formant_opts oo;
+    return formant_geometry(o, nsamp, fs, n, oo, nullptr, nullptr, frames_out, nullptr);
+}
+
+int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                     size_t n, const vs_formant_opts *o, vs_formant_stats *stats, vs_formant_frame *frames,
+                     const uint64_t *frame_offsets)
+{
+    if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
+    vs_formant_opts op;
+    std::vector<uint32_t> Nw(n), H(n);
+    std::vector<uint64_t> nfr(n);
+    int rc = formant_geometry(o, nsamp, fs, n, op, Nw.data(), H.data(), nfr.data(), &ctx->err);
+    if (rc) return rc;
+    if (n == 0) return VS_OK;
+    if (n > 0x7fffffffull) return fail(ctx, VS_EINVAL, "too many streams");
+    if ((rc = vs_sync(ctx))) return rc;                       /* the PCM may be the output of a call still in flight */
+    DeviceGuard restore_device;
+    Slot &sl = ctx->slots[0];
+    CU(cudaSetDevice(sl.dev));
+
+    /* rows, the frame prefix and one window table per distinct window length; host libm in double */
+    const double pi = 3.14159265358979323846;
+    std::vector<VsFormantRow> rows(n);
+    std::vector<uint64_t> frame0(n + 1, 0);
+    std::vector<double> win;
+    std::vector<std::pair<uint32_t, uint32_t>> win_at;        /* (Nw, offset) */
+    uint64_t max_n = 0, first = ~0ull, last = 0;
+    uint32_t max_nw = 0;
+    for (size_t i = 0; i < n; i++) max_n = std::max(max_n, nsamp[i]);
+    for (size_t i = 0; i < n; i++) {
+        const double rate = fs ? (double)fs[i] : 22050.0;
+        VsFormantRow &r = rows[i];
+        r.off = offsets ? offsets[i] : (uint64_t)i * max_n;
+        r.n = (uint32_t)nsamp[i];
+        r.Nw = Nw[i]; r.H = H[i];
+        r.fs = rate;
+        r.mu = op.preemph_hz > 0.0f ? std::exp(-2.0 * pi * (double)op.preemph_hz / rate) : 0.0;
+        auto it = std::find_if(win_at.begin(), win_at.end(), [&](const std::pair<uint32_t, uint32_t> &e) { return e.first == r.Nw; });
+        if (it == win_at.end()) {
+            win_at.push_back({r.Nw, (uint32_t)win.size()});
+            for (uint32_t m = 0; m < r.Nw; m++) win.push_back(0.54 - 0.46 * std::cos(2.0 * pi * (double)m / (double)(r.Nw - 1)));
+            it = win_at.end() - 1;
+        }
+        r.win_off = it->second;
+        max_nw = std::max(max_nw, r.Nw);
+        frame0[i + 1] = frame0[i] + nfr[i];
+        first = std::min(first, r.off);
+        last = std::max(last, r.off + r.n);
+    }
+    const uint64_t F = frame0[n];
+    VsFormantArgs a = {};
+    a.n_rows = (uint32_t)n; a.order = op.order; a.nf = op.n_formants; a.max_nw = max_nw; a.n_frames = F; a.bmax = op.bmax_hz;
+    for (uint32_t j = 0; j < op.order; j++) {
+        const double t = 2.0 * pi * (double)j / (double)op.order + 0.4;
+        a.seed_re[j] = 0.9 * std::cos(t);
+        a.seed_im[j] = 0.9 * std::sin(t);
+    }
+
+    int dev = -1;
+    const bool on_dev = classify(pcm, &dev) == PK_DEVICE;
+    if (on_dev && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
+    /* scratch: rows | frame prefix | windows | per-frame found/flags | per-frame F, B | stats | frame records */
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t rows_b = al(n * sizeof(VsFormantRow)), pre_b = al((n + 1) * sizeof(uint64_t)), win_b = al(win.size() * sizeof(double));
+    const size_t ff_b = al(F * sizeof(uint32_t)), fb_b = al(F * 2 * op.n_formants * sizeof(double)), st_b = al(n * sizeof(vs_formant_stats));
+    const size_t fr_b = frames ? F * sizeof(vs_formant_frame) : 0;
+    if ((rc = dev_reserve(ctx, sl, sl.analyze, rows_b + pre_b + win_b + ff_b + fb_b + st_b + fr_b))) return rc;
+    unsigned char *base = (unsigned char *)sl.analyze.p;
+    a.rows = (const VsFormantRow *)base;
+    a.frame0 = (const uint64_t *)(base + rows_b);
+    a.win = (const double *)(base + rows_b + pre_b);
+    a.ff = (uint32_t *)(base + rows_b + pre_b + win_b);
+    a.fb = (double *)(base + rows_b + pre_b + win_b + ff_b);
+    vs_formant_stats *d_stats = (vs_formant_stats *)(base + rows_b + pre_b + win_b + ff_b + fb_b);
+    vs_formant_frame *d_frames = frames ? (vs_formant_frame *)((unsigned char *)d_stats + st_b) : nullptr;
+    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsFormantRow), cudaMemcpyHostToDevice, sl.compute));
+    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, sl.compute));
+    if (!win.empty()) CU(cudaMemcpyAsync((void *)a.win, win.data(), win.size() * sizeof(double), cudaMemcpyHostToDevice, sl.compute));
+    a.pcm = pcm;
+    if (!on_dev && last > first) {
+        if ((rc = dev_reserve(ctx, sl, sl.pcm[0], (last - first) * sizeof(int16_t) + 256))) return rc;
+        a.pcm = (const int16_t *)sl.pcm[0].p - first;
+        CU(cudaMemcpyAsync(sl.pcm[0].p, pcm + first, (last - first) * sizeof(int16_t), cudaMemcpyHostToDevice, sl.compute));
+    }
+    CU(vs_launch_formants(a, d_stats, d_frames, sl.compute));
+    CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_formant_stats), cudaMemcpyDeviceToHost, sl.compute));
+    if (frames && F) {
+        if (!frame_offsets) {
+            CU(cudaMemcpyAsync(frames, d_frames, F * sizeof(vs_formant_frame), cudaMemcpyDeviceToHost, sl.compute));
+        } else {
+            /* streams whose records sit next to each other on both sides travel as one copy */
+            size_t i = 0;
+            while (i < n) {
+                if (!nfr[i]) { i++; continue; }
+                size_t j = i + 1;
+                while (j < n && frame_offsets[j] == frame_offsets[j - 1] + nfr[j - 1]) j++;
+                CU(cudaMemcpyAsync(frames + frame_offsets[i], d_frames + frame0[i], (frame0[j] - frame0[i]) * sizeof(vs_formant_frame),
+                                   cudaMemcpyDeviceToHost, sl.compute));
+                i = j;
+            }
+        }
+    }
+    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` and the results are pageable host memory */
+    return VS_OK;
 }
 
 int vs_synth_batch(vs_ctx *ctx, const vs_flow_params *p, const vs_filter_params *f, size_t n, int16_t *pcm_out,

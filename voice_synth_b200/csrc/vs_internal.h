@@ -178,4 +178,31 @@ struct VsAnalyzeRow {
     int16_t  lo, hi;       /* trigger thresholds */
 };
 
+/* formant analysis (vs_formant_batch): one entry per stream */
+struct VsFormantRow {
+    uint64_t off;          /* samples, relative to the pcm pointer                  */
+    uint32_t n;            /* samples                                               */
+    uint32_t Nw, H;        /* window length and frame step                          */
+    uint32_t win_off;      /* first entry of the stream's window in the table       */
+    double   mu;           /* pre-emphasis factor                                   */
+    double   fs;
+};
+
+/* the launch arguments of the two formant kernels */
+#define VS_FMT_MAX_ORDER 32
+struct VsFormantArgs {
+    const int16_t      *pcm;
+    const VsFormantRow *rows;
+    const uint64_t     *frame0;     /* [n_rows + 1]: global index of each stream's first frame (prefix sum)   */
+    const double       *win;        /* window tables, one per distinct Nw                                   */
+    double             *fb;         /* [frame][2 * nf]: F_0..F_nf-1, B_0..B_nf-1 of each frame, unrounded      */
+    uint32_t           *ff;         /* [frame]: found | flags << 16                                         */
+    uint32_t            n_rows;
+    uint32_t            order, nf;
+    uint32_t            max_nw;     /* longest window of the call: the shared-memory stride of a warp        */
+    uint64_t            n_frames;
+    double              bmax;
+    double              seed_re[VS_FMT_MAX_ORDER], seed_im[VS_FMT_MAX_ORDER];   /* root-finder start points */
+};
+
 #endif
