@@ -106,8 +106,11 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
     double y[VS_RING];
 #pragma unroll
     for (int j = 0; j < VS_RING; j++) y[j] = 0.0;
-    const int gain_i = (int)gaind, npre_i = -(int)pred;
-    int x_prev = 0, mbase = blk0, ti = 0;
+    const int gain_i = (int)gaind;
+    /* FILT_INT: the bytes {-pre, 1} of a two-way 16x8 dot product (pre is 0 or 1) */
+    const int pre_b = (int)(((uint32_t)-(int)pred & 0xffu) | 0x100u);
+    uint32_t w_prev = 0;                                    /* the last input word read: its high half is x[n-1] */
+    int mbase = blk0, ti = 0;
 
     vs_pair_barrier(pair);                                  /* window 0 generated */
     for (int w = 0; w < nwin; w++) {
@@ -129,9 +132,11 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
                     double acc, v;
                     if (FILT == VS_FILT_INT) {
                         /* gain and pre-emphasis on the integer input; the recurrence then yields the
-                         * pre-emphasised waveform directly (the filter is LTI) */
-                        acc = (double)((xi + x_prev * npre_i) * gain_i);
-                        x_prev = xi;
+                         * pre-emphasised waveform directly (the filter is LTI).  x[n] - pre*x[n-1] is one
+                         * dp2a on a word whose halves are (x[n-1], x[n]): an input word itself for odd u, the
+                         * high half of the previous word and the low half of this one for even u. */
+                        const uint32_t xx = (u & 1) ? xw[u >> 1] : __byte_perm(u == 0 ? w_prev : xw[(u >> 1) - 1], xw[u >> 1], 0x5432);
+                        acc = (double)(__dp2a_lo((int)xx, pre_b, 0) * gain_i);
 #pragma unroll
                         for (int j = VS_ORDER; j >= 1; j--) acc = __fma_rn(y[(k + VS_RING - j) % VS_RING], VS_NC(j), acc);
                         v = acc;
@@ -164,6 +169,7 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
                     ow[u >> 1] = FILT == VS_FILT_EXACT ? pk : __vmaxs2(pk, 0x80018001u);             /* -32768 -> -32767 */
                 }
                 *piece = make_uint4(ow[0], ow[1], ow[2], ow[3]);
+                w_prev = xw[3];
                 mbase += VS_GROUP;
             }
         }
@@ -394,8 +400,13 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
      * belong to the stream); the amplitude is picked by the sign of ic+u-Tc.  With the table zero beyond the open
      * phase and A <= 32767, flowgen_shimmer.c:319-335 is  x = max(ceil(A * table[i]), (short)DC):  values below DC
      * become DC (the rising branch's test :320; on the falling branch the first such value ends it, :329, and the
-     * factor only decreases from there), the closed phase is ceil(0) = 0 <= DC. */
-    auto gen_fast = [&](int (&x)[VS_GROUP], const bool first) {
+     * factor only decreases from there), the closed phase is ceil(0) = 0 <= DC.
+     * Output: the group's 8 samples as 4 words of int16 pairs.  Without noise the maximum is taken two samples at a
+     * time after a saturating pack: ceil(A * table[i]) <= 32767 (A <= 32767, table <= 1), and a value below -32768
+     * saturates to -32768 <= (short)DC, so max16(sat16(v), DC) == max(v, DC). */
+    const uint32_t dcs2 = (uint32_t)(uint16_t)DCs * 0x10001u;
+    auto gen_fast = [&](uint32_t (&ow)[VS_GROUP / 2], const bool first) {
+        int x[VS_GROUP];
         const int icT = ic - Tc;
         const double Adn = (double)An;
         uint32_t bc = smem_base + tb + (uint32_t)ic * 8u, bn = smem_base + tb + (uint32_t)(icT * 8);   /* table entry of sample 0 in the current / next period */
@@ -417,6 +428,7 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
             const double fac = vs_lds_f64((nx ? bn : bc) + (uint32_t)(u * 8));
             const double A = nx ? Adn : Adc;
             const int v = __double2int_ru(__dmul_rn(A, fac));
+            if (!NOISE && !first) { x[u] = v; continue; }   /* the maximum with DC comes after the pack */
             int xv = max(v, first ? (nx ? DCs : 0) : DCs);
             if (NOISE) {
                 /* glibc random(): r[n] = r[n-31] + r[n-3]; the slot of r[n-31] takes r[n].  Branch free: every lane
@@ -436,6 +448,16 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
                 xv = ns ? vs_add_clip(xv, w) : xv;
             }
             x[u] = xv;
+        }
+#pragma unroll
+        for (int u = 0; u < VS_GROUP; u += 2) {
+            if (!NOISE && !first) {
+                uint32_t pk;
+                asm("cvt.pack.sat.s16.s32 %0, %1, %2;" : "=r"(pk) : "r"(x[u + 1]), "r"(x[u]));
+                ow[u >> 1] = __vmaxs2(pk, dcs2);
+            } else {
+                ow[u >> 1] = __byte_perm((uint32_t)x[u], (uint32_t)x[u + 1], 0x5410);
+            }
         }
         /* the group's last sample may have been the period's last: promote `next`, read the entry after it */
         const bool pr = icT + VS_GROUP >= 0;
@@ -560,22 +582,19 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
             return;
         }
         unsigned char *trow = tbase + (uint32_t)lane * TSB;
-        auto put = [&](const int g, const int (&x)[VS_GROUP]) {
-            uint32_t ow[VS_GROUP / 2];
-#pragma unroll
-            for (int u = 0; u < VS_GROUP; u += 2) ow[u >> 1] = __byte_perm((uint32_t)x[u], (uint32_t)x[u + 1], 0x5410);
+        auto put = [&](const int g, const uint32_t (&ow)[VS_GROUP / 2]) {
             *reinterpret_cast<uint4 *>(trow + g * VS_GROUP * 2) = make_uint4(ow[0], ow[1], ow[2], ow[3]);
         };
+        uint32_t ow[VS_GROUP / 2];
         if (FAST && wfast) {                                /* (the choice of generator is made once per window, not per group) */
             ring_refill();
-            int x[VS_GROUP];
-            if (w == 0) gen_fast(x, true);
-            else gen_fast(x, false);
-            put(0, x);
+            if (w == 0) gen_fast(ow, true);
+            else gen_fast(ow, false);
+            put(0, ow);
 #pragma unroll 1
             for (int g = 1; g < NGRP; g++) {
-                gen_fast(x, false);
-                put(g, x);
+                gen_fast(ow, false);
+                put(g, ow);
             }
         } else {
 #pragma unroll 1
@@ -583,7 +602,9 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
                 int x[VS_GROUP];
 #pragma unroll
                 for (int u = 0; u < VS_GROUP; u++) x[u] = gen_simple();
-                put(g, x);
+#pragma unroll
+                for (int u = 0; u < VS_GROUP; u += 2) ow[u >> 1] = __byte_perm((uint32_t)x[u], (uint32_t)x[u + 1], 0x5410);
+                put(g, ow);
             }
         }
     };
