@@ -296,13 +296,18 @@ def formant_opts(opts=None):
 def formant_frames(nsamp, fs=None, opts=None):
     """frames per stream of vs_formant_batch (host only, validates like the batch call; raises VsError)"""
     ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-    rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), ns.shape))
+    rate = _per_stream(fs, np.int32, len(ns))
     o = formant_opts(opts)
     out = np.zeros(len(ns), dtype=np.uint64)
     rc = _lib.load().vs_formant_frames(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
     if rc:
         raise VsError(rc, _lib.load().vs_strerror(rc).decode())
     return out
+
+
+def _per_stream(x, dtype, n):
+    """a per-stream argument as n contiguous values of dtype (a scalar stands for every stream); None stays None (NULL)"""
+    return None if x is None else np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=dtype), (n,)))
 
 
 def _ptr(x):
@@ -414,9 +419,7 @@ class Context:
         n = len(ns)
         db = np.broadcast_to(np.asarray(snr_db, dtype=np.float32), (n,))
         snr = np.array([np.float32(math.pow(10.0, float(d / np.float32(10)))) if d > 0 else np.float32(0) for d in db], dtype=np.float32)
-        sd = np.ascontiguousarray(np.broadcast_to(np.asarray(seeds, dtype=np.uint32), (n,)))
-        rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), (n,)))
-        offs = None if offsets is None else np.ascontiguousarray(offsets, dtype=np.uint64)
+        offs, rate, sd = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32), (seeds, np.uint32)))
         self._check(self.L.vs_vowel_noise_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, snr.ctypes.data,
                                                 _ptr(rate), sd.ctypes.data, n))
         return pcm
@@ -434,10 +437,7 @@ class Context:
     def _analysis(self, call, dtype, flow, nsamp, offsets, fs, lo, hi):
         ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
         n = len(ns)
-        offs = None if offsets is None else np.ascontiguousarray(offsets, dtype=np.uint64)
-        rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), (n,)))
-        tl = None if lo is None else np.ascontiguousarray(np.broadcast_to(np.asarray(lo, dtype=np.int16), (n,)))
-        th = None if hi is None else np.ascontiguousarray(np.broadcast_to(np.asarray(hi, dtype=np.int16), (n,)))
+        offs, rate, tl, th = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32), (lo, np.int16), (hi, np.int16)))
         res = np.zeros(n, dtype=dtype)
         self._check(call(self.h, _ptr(flow), _ptr(offs), ns.ctypes.data, _ptr(rate), _ptr(tl), _ptr(th), n, res.ctypes.data))
         return res
@@ -448,8 +448,7 @@ class Context:
         defaults) or a dict of the vs_formant_opts fields to change."""
         ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
         n = len(ns)
-        offs = None if offsets is None else np.ascontiguousarray(offsets, dtype=np.uint64)
-        rate = None if fs is None else np.ascontiguousarray(np.broadcast_to(np.asarray(fs, dtype=np.int32), (n,)))
+        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
         o = formant_opts(opts)
         st = np.zeros(n, dtype=FORMANT_STATS_DTYPE)
         fr, fo = None, None

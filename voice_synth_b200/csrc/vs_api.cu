@@ -698,6 +698,91 @@ int run_batch(vs_ctx *ctx, const VsBatch &b)
     return VS_OK;
 }
 
+/* ---- calls on PCM the caller owns: output noise, flow analysis and report, formants ---------------------------------- */
+/* the checks of these calls, in index order so that the first offender decides: the stream count, then per stream its
+ * length, its sampling rate (fs NULL: 22050 Hz) and the call's own checks, stream(i, rate) */
+template <class Stream>
+int check_streams(std::string *err, const uint64_t *nsamp, const int32_t *fs, size_t n, Stream stream)
+{
+    if (n > 0x7fffffffull) return vs_error(err, VS_EINVAL, "too many streams");
+    for (size_t i = 0; i < n; i++) {
+        if (nsamp[i] > 0x7fffffffull) return vs_error(err, VS_EOVERLAP, "stream %zu: too many samples", i);
+        const int32_t rate = fs ? fs[i] : 22050;
+        if (rate <= 0) return vs_error(err, VS_ERANGE, "stream %zu: sampling rate", i);
+        if (const int rc = stream(i, rate)) return rc;
+    }
+    return VS_OK;
+}
+
+/* sets rows[i].off, where stream i starts in the caller's PCM (offsets NULL: dense rows at a stride of the longest
+ * one), and returns the samples [first, last) the rows cover */
+struct Span { uint64_t first, last; };
+template <class Row>
+Span place_rows(const uint64_t *offsets, const uint64_t *nsamp, std::vector<Row> &rows)
+{
+    uint64_t stride = 0;
+    for (size_t i = 0; i < rows.size(); i++) stride = std::max(stride, nsamp[i]);
+    Span s = {~0ull, 0};
+    for (size_t i = 0; i < rows.size(); i++) {
+        rows[i].off = offsets ? offsets[i] : (uint64_t)i * stride;
+        s.first = std::min(s.first, rows[i].off);
+        s.last = std::max(s.last, rows[i].off + nsamp[i]);
+    }
+    return s;
+}
+
+/* a call's device scratch: pieces at 256-byte aligned offsets, in the order they are taken */
+struct Scratch {
+    size_t bytes = 0;
+    size_t take(size_t b) { const size_t at = bytes; bytes = (bytes + b + 255) & ~(size_t)255; return at; }
+};
+
+/* the device side of a call whose arguments have passed: earlier work must have landed (the PCM may be the output of
+ * a call still in flight, and the noise call writes it in place); slot 0 runs it (one device is plenty: 0.75 ms for
+ * the noise of 4096 x 1 s); the scratch and the staged PCM.  The caller holds a DeviceGuard. */
+template <class T> struct PcmDev {
+    cudaStream_t st;
+    T *pcm;                      /* the PCM as the kernels address it: row offsets are relative to this */
+    bool staged;                 /* the caller's PCM is host memory, staged into pcm[0] */
+    unsigned char *scratch;
+};
+template <class T>
+int pcm_call_begin(vs_ctx *ctx, T *pcm, const Span &span, size_t scratch_bytes, PcmDev<T> &d)
+{
+    int rc, dev = -1;
+    if ((rc = vs_sync(ctx))) return rc;
+    Slot &sl = ctx->slots[0];
+    CU(cudaSetDevice(sl.dev));
+    d = {sl.compute, pcm, classify(pcm, &dev) != PK_DEVICE, nullptr};
+    if (!d.staged && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
+    if ((rc = dev_reserve(ctx, sl, sl.analyze, scratch_bytes))) return rc;
+    d.scratch = (unsigned char *)sl.analyze.p;
+    if (d.staged) {
+        const size_t bytes = (span.last - span.first) * sizeof(int16_t);
+        if ((rc = dev_reserve(ctx, sl, sl.pcm[0], bytes + 256))) return rc;
+        d.pcm = (T *)sl.pcm[0].p - span.first;
+        CU(cudaMemcpyAsync(sl.pcm[0].p, pcm + span.first, bytes, cudaMemcpyHostToDevice, d.st));
+    }
+    return VS_OK;
+}
+
+/* device-to-host copy of n rows, row(i) = {offset in src, offset in dst, elements}; a row that continues the previous
+ * non-empty one on both sides travels with it as one copy */
+struct RowCopy { uint64_t s, d, n; };
+template <class T, class Row>
+int copy_rows_home(vs_ctx *ctx, T *dst, const T *src, size_t n, Row row, cudaStream_t st)
+{
+    RowCopy run = {0, 0, 0};
+    for (size_t i = 0; i <= n; i++) {
+        const RowCopy r = i < n ? row(i) : RowCopy{0, 0, 0};
+        if (i < n && !r.n) continue;
+        if (r.n && run.n && r.s == run.s + run.n && r.d == run.d + run.n) { run.n += r.n; continue; }
+        if (run.n) CU(cudaMemcpyAsync(dst + run.d, src + run.s, run.n * sizeof(T), cudaMemcpyDeviceToHost, st));
+        run = r;
+    }
+    return VS_OK;
+}
+
 } // namespace
 
 /* ================================================================================================
@@ -936,55 +1021,26 @@ int vs_vowel_noise_batch(vs_ctx *ctx, int16_t *pcm, const uint64_t *offsets, con
 {
     if (!ctx || !pcm || !nsamp || !snr) return VS_EINVAL;
     if (n == 0) return VS_OK;
-    if (n > 0x7fffffffull) return fail(ctx, VS_EINVAL, "too many streams");
-    int rc = vs_sync(ctx);                                    /* in-place: earlier work on this PCM must have landed */
-    if (rc) return rc;
-    DeviceGuard restore_device;
-    Slot &sl = ctx->slots[0];                                 /* one warp per stream and 0.75 ms for 4096 x 1 s: one device is plenty */
-    CU(cudaSetDevice(sl.dev));
-    std::vector<VsNoiseRow> rows(n);
-    uint64_t max_n = 0, lo = ~0ull, hi = 0;
-    for (size_t i = 0; i < n; i++) max_n = std::max(max_n, nsamp[i]);
-    for (size_t i = 0; i < n; i++) {
-        if (nsamp[i] > 0x7fffffffull) return fail(ctx, VS_EOVERLAP, "stream %zu: too many samples", i);
-        const int32_t rate = fs ? fs[i] : 22050;
-        if (rate <= 0) return fail(ctx, VS_ERANGE, "stream %zu: sampling rate", i);
+    std::vector<VsNoiseRow> rows;
+    int rc = check_streams(&ctx->err, nsamp, fs, n, [&](size_t i, int32_t rate) {
         const int ms1 = (int)((uint32_t)rate * 0.001 / 2.0) * 2;       /* vowel_new.c:361 */
         const long frame = 50L * ms1;                                  /* :363 */
         if (snr[i] > 0.0f && (frame <= 0 || frame > 32767)) return fail(ctx, VS_ERANGE, "stream %zu: frame length %ld", i, frame);
-        rows[i].off = offsets ? offsets[i] : (uint64_t)i * max_n;
-        rows[i].n = (uint32_t)nsamp[i];
-        rows[i].frame = (uint32_t)frame;
-        rows[i].snr = snr[i];
-        rows[i].seed = seed ? seed[i] : 1u;
-        lo = std::min(lo, rows[i].off);
-        hi = std::max(hi, rows[i].off + rows[i].n);
-    }
-    int dev = -1;
-    const bool on_dev = classify(pcm, &dev) == PK_DEVICE;
-    if (on_dev && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
-    if ((rc = dev_reserve(ctx, sl, sl.log, n * sizeof(VsNoiseRow)))) return rc;          /* the log scratch doubles as row storage */
-    CU(cudaMemcpyAsync(sl.log.p, rows.data(), n * sizeof(VsNoiseRow), cudaMemcpyHostToDevice, sl.compute));
-    int16_t *d_pcm = pcm;
-    if (!on_dev) {
-        if ((rc = dev_reserve(ctx, sl, sl.pcm[0], (hi - lo) * sizeof(int16_t) + 64))) return rc;
-        d_pcm = (int16_t *)sl.pcm[0].p - lo;
-        CU(cudaMemcpyAsync(sl.pcm[0].p, pcm + lo, (hi - lo) * sizeof(int16_t), cudaMemcpyHostToDevice, sl.compute));
-    }
-    CU(vs_launch_vnoise(d_pcm, (const VsNoiseRow *)sl.log.p, (uint32_t)n, sl.compute));
-    if (!on_dev) {
-        /* only the rows come back (gaps between them are not ours); rows that touch travel as one copy */
-        uint64_t run_lo = 0, run_hi = 0;
-        for (size_t i = 0; i <= n; i++) {
-            const bool take = i < n && rows[i].n && rows[i].snr > 0.0f;
-            if (take && run_hi > run_lo && rows[i].off == run_hi) { run_hi += rows[i].n; continue; }
-            if (run_hi > run_lo)
-                CU(cudaMemcpyAsync(pcm + run_lo, d_pcm + run_lo, (run_hi - run_lo) * sizeof(int16_t), cudaMemcpyDeviceToHost, sl.compute));
-            run_lo = take ? rows[i].off : 0;
-            run_hi = take ? rows[i].off + rows[i].n : 0;
-        }
-    }
-    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` is pageable host memory */
+        if (i == 0) rows.resize(n);                                    /* n has passed the stream-count check */
+        rows[i] = {0, (uint32_t)nsamp[i], (uint32_t)frame, snr[i], seed ? seed[i] : 1u};
+        return VS_OK;
+    });
+    if (rc) return rc;
+    const Span span = place_rows(offsets, nsamp, rows);
+    DeviceGuard restore_device;
+    PcmDev<int16_t> d;
+    if ((rc = pcm_call_begin(ctx, pcm, span, n * sizeof(VsNoiseRow), d))) return rc;
+    CU(cudaMemcpyAsync(d.scratch, rows.data(), n * sizeof(VsNoiseRow), cudaMemcpyHostToDevice, d.st));
+    CU(vs_launch_vnoise(d.pcm, (const VsNoiseRow *)d.scratch, (uint32_t)n, d.st));
+    /* host memory: only the noised rows come back, the bytes between and around them are the caller's */
+    auto noised = [&](size_t i) { return RowCopy{rows[i].off, rows[i].off, rows[i].snr > 0.0f ? rows[i].n : 0u}; };
+    if (d.staged && (rc = copy_rows_home(ctx, pcm, d.pcm, n, noised, d.st))) return rc;
+    CU(cudaStreamSynchronize(d.st));                          /* `rows` is pageable host memory */
     return VS_OK;
 }
 
@@ -994,60 +1050,40 @@ static int flow_analysis(vs_ctx *ctx, const int16_t *flow, const uint64_t *offse
                          const int16_t *lo, const int16_t *hi, size_t n, vs_flow_stats *stats, vs_flow_report *report)
 {
     if (n == 0) return VS_OK;
-    if (n > 0x7fffffffull) return fail(ctx, VS_EINVAL, "too many streams");
-    int rc = vs_sync(ctx);                                    /* the flow may be the output of a call still in flight */
-    if (rc) return rc;
-    DeviceGuard restore_device;
-    Slot &sl = ctx->slots[0];
-    CU(cudaSetDevice(sl.dev));
-    std::vector<VsAnalyzeRow> rows(n);
-    uint64_t max_n = 0, first = ~0ull, last = 0, slots = 0;
-    for (size_t i = 0; i < n; i++) max_n = std::max(max_n, nsamp[i]);
-    for (size_t i = 0; i < n; i++) {
-        if (nsamp[i] > 0x7fffffffull) return fail(ctx, VS_EOVERLAP, "stream %zu: too many samples", i);
-        const int32_t rate = fs ? fs[i] : 22050;
-        if (rate <= 0) return fail(ctx, VS_ERANGE, "stream %zu: sampling rate", i);
+    std::vector<VsAnalyzeRow> rows;
+    uint64_t slots = 0;
+    int rc = check_streams(&ctx->err, nsamp, fs, n, [&](size_t i, int32_t rate) {
         const int16_t tl = lo ? lo[i] : (int16_t)0, th = hi ? hi[i] : (int16_t)0;
         if (tl > th) return fail(ctx, VS_ERANGE, "stream %zu: thresholds lo > hi", i);
-        VsAnalyzeRow &r = rows[i];
-        r.off = offsets ? offsets[i] : (uint64_t)i * max_n;
-        r.n = (uint32_t)nsamp[i];
-        r.cap = r.n / 16u + 4u;
-        r.ons_off = slots;
-        r.fs = rate; r.lo = tl; r.hi = th;
-        slots += r.cap;
-        first = std::min(first, r.off);
-        last = std::max(last, r.off + r.n);
-    }
-    int dev = -1;
-    const bool on_dev = classify(flow, &dev) == PK_DEVICE;
-    if (on_dev && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
+        const uint32_t len = (uint32_t)nsamp[i], cap = len / 16u + 4u;
+        if (i == 0) rows.resize(n);                                    /* n has passed the stream-count check */
+        rows[i] = {0, slots, len, cap, rate, tl, th};
+        slots += cap;
+        return VS_OK;
+    });
+    if (rc) return rc;
+    const Span span = place_rows(offsets, nsamp, rows);
     /* scratch: rows | per-stream onset counts | stats | onset lists, and for the report: | peak lists | reports */
-    const size_t rows_b = (n * sizeof(VsAnalyzeRow) + 255) & ~(size_t)255, cnt_b = (n * sizeof(uint32_t) + 255) & ~(size_t)255;
-    const size_t st_b = (n * sizeof(vs_flow_stats) + 255) & ~(size_t)255;
-    const size_t ons_b = (slots * sizeof(uint32_t) + 255) & ~(size_t)255;
-    const size_t rep_b = report ? ons_b + n * sizeof(vs_flow_report) : 0;
-    if ((rc = dev_reserve(ctx, sl, sl.analyze, rows_b + cnt_b + st_b + (report ? ons_b : slots * sizeof(uint32_t)) + rep_b))) return rc;
-    unsigned char *base = (unsigned char *)sl.analyze.p;
-    CU(cudaMemcpyAsync(base, rows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, sl.compute));
-    const int16_t *d_flow = flow;
-    if (!on_dev) {
-        if ((rc = dev_reserve(ctx, sl, sl.pcm[0], (last - first) * sizeof(int16_t) + 256))) return rc;
-        d_flow = (const int16_t *)sl.pcm[0].p - first;
-        CU(cudaMemcpyAsync(sl.pcm[0].p, flow + first, (last - first) * sizeof(int16_t), cudaMemcpyHostToDevice, sl.compute));
-    }
+    Scratch sc;
+    const size_t o_rows = sc.take(n * sizeof(VsAnalyzeRow)), o_cnt = sc.take(n * sizeof(uint32_t));
+    const size_t o_st = sc.take(n * sizeof(vs_flow_stats)), o_ons = sc.take(slots * sizeof(uint32_t));
+    const size_t o_peaks = report ? sc.take(slots * sizeof(uint32_t)) : 0, o_rep = report ? sc.take(n * sizeof(vs_flow_report)) : 0;
+    DeviceGuard restore_device;
+    PcmDev<const int16_t> d;
+    if ((rc = pcm_call_begin(ctx, flow, span, sc.bytes, d))) return rc;
+    const VsAnalyzeRow *d_rows = (const VsAnalyzeRow *)(d.scratch + o_rows);
+    uint32_t *d_cnt = (uint32_t *)(d.scratch + o_cnt), *d_ons = (uint32_t *)(d.scratch + o_ons);
+    vs_flow_stats *d_st = (vs_flow_stats *)(d.scratch + o_st);
+    CU(cudaMemcpyAsync(d.scratch + o_rows, rows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, d.st));
     if (!report) {
-        CU(vs_launch_analyze(d_flow, (const VsAnalyzeRow *)base, (uint32_t)n, (uint32_t *)(base + rows_b + cnt_b + st_b),
-                             (uint32_t *)(base + rows_b), (vs_flow_stats *)(base + rows_b + cnt_b), sl.compute));
-        CU(cudaMemcpyAsync(stats, base + rows_b + cnt_b, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, sl.compute));
+        CU(vs_launch_analyze(d.pcm, d_rows, (uint32_t)n, d_ons, d_cnt, d_st, d.st));
+        CU(cudaMemcpyAsync(stats, d_st, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, d.st));
     } else {
-        unsigned char *peaks = base + rows_b + cnt_b + st_b + ons_b, *reps = peaks + ons_b;
-        CU(vs_launch_report(d_flow, (const VsAnalyzeRow *)base, (uint32_t)n, (uint32_t *)(base + rows_b + cnt_b + st_b),
-                            (uint32_t *)(base + rows_b), (vs_flow_stats *)(base + rows_b + cnt_b), (int32_t *)peaks,
-                            (vs_flow_report *)reps, sl.compute));
-        CU(cudaMemcpyAsync(report, reps, n * sizeof(vs_flow_report), cudaMemcpyDeviceToHost, sl.compute));
+        vs_flow_report *d_rep = (vs_flow_report *)(d.scratch + o_rep);
+        CU(vs_launch_report(d.pcm, d_rows, (uint32_t)n, d_ons, d_cnt, d_st, (int32_t *)(d.scratch + o_peaks), d_rep, d.st));
+        CU(cudaMemcpyAsync(report, d_rep, n * sizeof(vs_flow_report), cudaMemcpyDeviceToHost, d.st));
     }
-    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` and the results are the caller's / pageable memory */
+    CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are the caller's / pageable memory */
     return VS_OK;
 }
 
@@ -1066,37 +1102,33 @@ int vs_flow_report_batch(vs_ctx *ctx, const int16_t *flow, const uint64_t *offse
 }
 
 /* the option and per-stream checks of vs_formant_frames and vs_formant_batch, in the header's order; fills o (the
- * defaults for in == NULL) and, per stream, Nw, H and the frame count */
+ * defaults for in == NULL), each stream's frame count and, unless rows is NULL, its row but for off, win_off and mu */
 static int formant_geometry(const vs_formant_opts *in, const uint64_t *nsamp, const int32_t *fs, size_t n, vs_formant_opts &o,
-                            uint32_t *Nw, uint32_t *H, uint64_t *frames, std::string *err)
+                            VsFormantRow *rows, uint64_t *frames, std::string *err)
 {
     o = in ? *in : vs_formant_opts{25.0f, 10.0f, 50.0f, 700.0f, 14u, 5u};
     if (o.order < 2 || o.order > VS_FMT_MAX_ORDER || (o.order & 1u)) return vs_error(err, VS_EINVAL, "order %u: even, 2..%d", o.order, VS_FMT_MAX_ORDER);
     if (o.n_formants < 1 || o.n_formants > VS_MAX_FORMANTS || o.n_formants > o.order / 2)
         return vs_error(err, VS_EINVAL, "n_formants %u: 1..%d and at most order / 2", o.n_formants, VS_MAX_FORMANTS);
     if (!(o.preemph_hz >= 0.0f) || !(o.bmax_hz >= 0.0f)) return vs_error(err, VS_ERANGE, "preemph_hz and bmax_hz must be >= 0");
-    for (size_t i = 0; i < n; i++) {
-        if (nsamp[i] > 0x7fffffffull) return vs_error(err, VS_EOVERLAP, "stream %zu: too many samples", i);
-        const int32_t rate = fs ? fs[i] : 22050;
-        if (rate <= 0) return vs_error(err, VS_ERANGE, "stream %zu: sampling rate", i);
+    return check_streams(err, nsamp, fs, n, [&](size_t i, int32_t rate) {
         const double wl = (double)o.win_ms * rate / 1000.0, hl = (double)o.hop_ms * rate / 1000.0;
         const long nw = wl > -1e9 && wl < 1e9 ? lround(wl) : -1;
         if (nw < (long)o.order + 1 || nw > VS_FORMANT_MAX_WIN)
             return vs_error(err, VS_ERANGE, "stream %zu: window of %ld samples, needs %u..%d", i, nw, o.order + 1, VS_FORMANT_MAX_WIN);
         if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
         const uint64_t h = (uint64_t)lround(hl);
-        if (Nw) Nw[i] = (uint32_t)nw;
-        if (H) H[i] = (uint32_t)h;
+        if (rows) rows[i] = {0, (uint32_t)nsamp[i], (uint32_t)nw, (uint32_t)h, 0, 0.0, (double)rate};
         frames[i] = nsamp[i] >= (uint64_t)nw ? (nsamp[i] - (uint64_t)nw) / h + 1 : 0;
-    }
-    return VS_OK;
+        return VS_OK;
+    });
 }
 
 int vs_formant_frames(const vs_formant_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *frames_out)
 {
     if (!nsamp || !frames_out) return VS_EINVAL;
     vs_formant_opts oo;
-    return formant_geometry(o, nsamp, fs, n, oo, nullptr, nullptr, frames_out, nullptr);
+    return formant_geometry(o, nsamp, fs, n, oo, nullptr, frames_out, nullptr);
 }
 
 int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
@@ -1105,34 +1137,21 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
 {
     if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
     vs_formant_opts op;
-    std::vector<uint32_t> Nw(n), H(n);
+    std::vector<VsFormantRow> rows(n);
     std::vector<uint64_t> nfr(n);
-    int rc = formant_geometry(o, nsamp, fs, n, op, Nw.data(), H.data(), nfr.data(), &ctx->err);
+    int rc = formant_geometry(o, nsamp, fs, n, op, rows.data(), nfr.data(), &ctx->err);
     if (rc) return rc;
     if (n == 0) return VS_OK;
-    if (n > 0x7fffffffull) return fail(ctx, VS_EINVAL, "too many streams");
-    if ((rc = vs_sync(ctx))) return rc;                       /* the PCM may be the output of a call still in flight */
-    DeviceGuard restore_device;
-    Slot &sl = ctx->slots[0];
-    CU(cudaSetDevice(sl.dev));
 
-    /* rows, the frame prefix and one window table per distinct window length; host libm in double */
+    /* pre-emphasis, the frame prefix and one window table per distinct window length; host libm in double */
     const double pi = 3.14159265358979323846;
-    std::vector<VsFormantRow> rows(n);
     std::vector<uint64_t> frame0(n + 1, 0);
     std::vector<double> win;
     std::vector<std::pair<uint32_t, uint32_t>> win_at;        /* (Nw, offset) */
-    uint64_t max_n = 0, first = ~0ull, last = 0;
     uint32_t max_nw = 0;
-    for (size_t i = 0; i < n; i++) max_n = std::max(max_n, nsamp[i]);
     for (size_t i = 0; i < n; i++) {
-        const double rate = fs ? (double)fs[i] : 22050.0;
         VsFormantRow &r = rows[i];
-        r.off = offsets ? offsets[i] : (uint64_t)i * max_n;
-        r.n = (uint32_t)nsamp[i];
-        r.Nw = Nw[i]; r.H = H[i];
-        r.fs = rate;
-        r.mu = op.preemph_hz > 0.0f ? std::exp(-2.0 * pi * (double)op.preemph_hz / rate) : 0.0;
+        r.mu = op.preemph_hz > 0.0f ? std::exp(-2.0 * pi * (double)op.preemph_hz / r.fs) : 0.0;
         auto it = std::find_if(win_at.begin(), win_at.end(), [&](const std::pair<uint32_t, uint32_t> &e) { return e.first == r.Nw; });
         if (it == win_at.end()) {
             win_at.push_back({r.Nw, (uint32_t)win.size()});
@@ -1142,9 +1161,8 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
         r.win_off = it->second;
         max_nw = std::max(max_nw, r.Nw);
         frame0[i + 1] = frame0[i] + nfr[i];
-        first = std::min(first, r.off);
-        last = std::max(last, r.off + r.n);
     }
+    const Span span = place_rows(offsets, nsamp, rows);
     const uint64_t F = frame0[n];
     VsFormantArgs a = {};
     a.n_rows = (uint32_t)n; a.order = op.order; a.nf = op.n_formants; a.max_nw = max_nw; a.n_frames = F; a.bmax = op.bmax_hz;
@@ -1154,51 +1172,32 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
         a.seed_im[j] = 0.9 * std::sin(t);
     }
 
-    int dev = -1;
-    const bool on_dev = classify(pcm, &dev) == PK_DEVICE;
-    if (on_dev && dev != sl.dev) return fail(ctx, VS_EINVAL, "device buffer lives on device %d, ctx on %d", dev, sl.dev);
     /* scratch: rows | frame prefix | windows | per-frame found/flags | per-frame F, B | stats | frame records */
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t rows_b = al(n * sizeof(VsFormantRow)), pre_b = al((n + 1) * sizeof(uint64_t)), win_b = al(win.size() * sizeof(double));
-    const size_t ff_b = al(F * sizeof(uint32_t)), fb_b = al(F * 2 * op.n_formants * sizeof(double)), st_b = al(n * sizeof(vs_formant_stats));
-    const size_t fr_b = frames ? F * sizeof(vs_formant_frame) : 0;
-    if ((rc = dev_reserve(ctx, sl, sl.analyze, rows_b + pre_b + win_b + ff_b + fb_b + st_b + fr_b))) return rc;
-    unsigned char *base = (unsigned char *)sl.analyze.p;
-    a.rows = (const VsFormantRow *)base;
-    a.frame0 = (const uint64_t *)(base + rows_b);
-    a.win = (const double *)(base + rows_b + pre_b);
-    a.ff = (uint32_t *)(base + rows_b + pre_b + win_b);
-    a.fb = (double *)(base + rows_b + pre_b + win_b + ff_b);
-    vs_formant_stats *d_stats = (vs_formant_stats *)(base + rows_b + pre_b + win_b + ff_b + fb_b);
-    vs_formant_frame *d_frames = frames ? (vs_formant_frame *)((unsigned char *)d_stats + st_b) : nullptr;
-    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsFormantRow), cudaMemcpyHostToDevice, sl.compute));
-    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, sl.compute));
-    if (!win.empty()) CU(cudaMemcpyAsync((void *)a.win, win.data(), win.size() * sizeof(double), cudaMemcpyHostToDevice, sl.compute));
-    a.pcm = pcm;
-    if (!on_dev && last > first) {
-        if ((rc = dev_reserve(ctx, sl, sl.pcm[0], (last - first) * sizeof(int16_t) + 256))) return rc;
-        a.pcm = (const int16_t *)sl.pcm[0].p - first;
-        CU(cudaMemcpyAsync(sl.pcm[0].p, pcm + first, (last - first) * sizeof(int16_t), cudaMemcpyHostToDevice, sl.compute));
-    }
-    CU(vs_launch_formants(a, d_stats, d_frames, sl.compute));
-    CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_formant_stats), cudaMemcpyDeviceToHost, sl.compute));
-    if (frames && F) {
-        if (!frame_offsets) {
-            CU(cudaMemcpyAsync(frames, d_frames, F * sizeof(vs_formant_frame), cudaMemcpyDeviceToHost, sl.compute));
-        } else {
-            /* streams whose records sit next to each other on both sides travel as one copy */
-            size_t i = 0;
-            while (i < n) {
-                if (!nfr[i]) { i++; continue; }
-                size_t j = i + 1;
-                while (j < n && frame_offsets[j] == frame_offsets[j - 1] + nfr[j - 1]) j++;
-                CU(cudaMemcpyAsync(frames + frame_offsets[i], d_frames + frame0[i], (frame0[j] - frame0[i]) * sizeof(vs_formant_frame),
-                                   cudaMemcpyDeviceToHost, sl.compute));
-                i = j;
-            }
-        }
-    }
-    CU(cudaStreamSynchronize(sl.compute));                    /* `rows` and the results are pageable host memory */
+    Scratch sc;
+    const size_t o_rows = sc.take(n * sizeof(VsFormantRow)), o_pre = sc.take((n + 1) * sizeof(uint64_t));
+    const size_t o_win = sc.take(win.size() * sizeof(double)), o_ff = sc.take(F * sizeof(uint32_t));
+    const size_t o_fb = sc.take(F * 2 * op.n_formants * sizeof(double)), o_st = sc.take(n * sizeof(vs_formant_stats));
+    const size_t o_fr = sc.take(frames ? F * sizeof(vs_formant_frame) : 0);
+    DeviceGuard restore_device;
+    PcmDev<const int16_t> d;
+    if ((rc = pcm_call_begin(ctx, pcm, span, sc.bytes, d))) return rc;
+    a.pcm = d.pcm;
+    a.rows = (const VsFormantRow *)(d.scratch + o_rows);
+    a.frame0 = (const uint64_t *)(d.scratch + o_pre);
+    a.win = (const double *)(d.scratch + o_win);
+    a.ff = (uint32_t *)(d.scratch + o_ff);
+    a.fb = (double *)(d.scratch + o_fb);
+    vs_formant_stats *d_stats = (vs_formant_stats *)(d.scratch + o_st);
+    vs_formant_frame *d_frames = frames ? (vs_formant_frame *)(d.scratch + o_fr) : nullptr;
+    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsFormantRow), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.win, win.data(), win.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
+    CU(vs_launch_formants(a, d_stats, d_frames, d.st));
+    CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_formant_stats), cudaMemcpyDeviceToHost, d.st));
+    /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
+    auto records = [&](size_t i) { return RowCopy{frame0[i], frame_offsets ? frame_offsets[i] : frame0[i], nfr[i]}; };
+    if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;
+    CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are pageable host memory */
     return VS_OK;
 }
 
