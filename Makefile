@@ -24,7 +24,7 @@ $(OBJDIR)/%.o: $(CSRC)/%.cu $(HDRS)
 $(OBJDIR)/%.o: $(CSRC)/%.cpp $(HDRS)
 	mkdir -p $(OBJDIR)
 	$(NVCC) $(NVFLAGS) -c -o $@ $<
-$(OBJDIR)/vs_api.o $(OBJDIR)/vs_batch_plan.o: $(CSRC)/vs_batch_plan.h
+$(OBJDIR)/vs_api.o $(OBJDIR)/vs_batch_plan.o $(OBJDIR)/vs_plan.o $(OBJDIR)/vs_render.o: $(CSRC)/vs_batch_plan.h
 $(LIB): $(OBJS)
 	mkdir -p $(LIBDIR)
 	$(NVCC) $(NVFLAGS) -shared -o $@ $(OBJS)

@@ -42,7 +42,8 @@ def _formant_tracts(L, nt):
 
 
 SHAPES = ["cfg2", "cfg3_shard", "cfg5_slice", "flow_cfg2", "flow_cfg3_shard", "filter_only", "tracts_10", "tracts_128",
-          "no_chunks", "fixed_chunks", "flow_fixed_chunks", "exact", "slab_97", "ragged", "period_log"]
+          "no_chunks", "fixed_chunks", "flow_fixed_chunks", "exact", "slab_97", "ragged", "period_log",
+          "simple_gen", "flow_simple_gen", "raw", "gain_10_5", "flow_exact", "kvar"]
 
 
 def shapes(L):
@@ -56,13 +57,18 @@ def shapes(L):
     ns_filter = rng.integers(500, 90000, 3000).astype(np.uint64)
     f_filter = api.FilterParams(3000)
     f_filter.preset[...] = [ord(workloads.PRESETS[(i * 7) % 10]) for i in range(3000)]
+    f_gain = f2.select(np.arange(f2.n))
+    f_gain.gain[0] = 10.5
+    p_kvar = p2.select(np.arange(p2.n))
+    p_kvar.Kvar[::7] = 0.3
     sub = np.arange(1024)
     p_sub, f_sub = p2.select(sub), f2.select(sub)
     ns_sub = _nsamples(L, p_sub)
     ragged = np.concatenate([[0], np.cumsum(ns_sub[:-1] + rng.integers(0, 300, 1023).astype(np.uint64))]).astype(np.uint64) + 3
     t10 = api.TractParams(4096, _preset_tracts(L), tract=np.arange(4096) % 10)
     t128 = api.TractParams(4096, _formant_tracts(L, 128), tract=(np.arange(4096) * 37) % 128)
-    d = dict(mode=SYNTH, f=None, nsamp=None, offsets=None, log=False, chunk=0, exact=0, slab=0, out_dev=True)
+    d = dict(mode=SYNTH, f=None, nsamp=None, offsets=None, log=False, chunk=0, exact=0, slab=0, simple_gen=0, raw=False,
+             out_dev=True)
     return {
         "cfg2": dict(d, p=p2, f=f2),
         "cfg3_shard": dict(d, p=p3, f=f3),
@@ -79,11 +85,63 @@ def shapes(L):
         "slab_97": dict(d, p=p2, f=f2, slab=97, out_dev=False),
         "ragged": dict(d, p=p_sub, f=f_sub, offsets=ragged),
         "period_log": dict(d, mode=FLOW, p=p3.select(np.arange(512)), log=True),
+        "simple_gen": dict(d, p=p2, f=f2, simple_gen=1),
+        "flow_simple_gen": dict(d, mode=FLOW, p=p2, simple_gen=1),
+        "raw": dict(d, p=p2, f=f2, raw=True),
+        "gain_10_5": dict(d, p=p2, f=f_gain),
+        "flow_exact": dict(d, mode=FLOW, p=p2, exact=1),
+        "kvar": dict(d, p=p_kvar, f=f2),
     }
 
 
 # total chunks and warm-up samples that vs_get_timing reports for these calls on a B200 (148 SMs), device output
 PINNED = {"cfg2": (17614, 32765084), "cfg3_shard": (30310, 53758613), "cfg5_slice": (15967, 24523171)}
+
+
+# The kernels of each shape: the record vs_shape makes (table format, warp-per-row flow, tracts, filter groups and their
+# padding, the thread-form plan kernel and its streams per CTA, filter arithmetic, raw output, glottal noise, -z), then
+# the generator and the vs_timing::render_path of every slab.  (Flow-only calls report the filter bits although they
+# run no filter.)
+TAB_FULL, TAB_C8, TAB_N16 = 0, 1, 2
+LEAN, PULSE, LOG = 0, 1, 2
+F_INT, F_FMA, F_EXACT = 0, 1, 2
+FAST, SIMPLE = 0, 1
+KERNELS = {
+    "cfg2":               (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "cfg3_shard":         (TAB_N16, 0, 0, 10, 32, PULSE, 512, F_INT, 0, 1, 0, FAST, 3),
+    "cfg5_slice":         (TAB_N16, 0, 0, 10, 32, PULSE, 512, F_INT, 0, 1, 0, FAST, 3),
+    "flow_cfg2":          (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 33),
+    "flow_cfg3_shard":    (TAB_N16, 0, 0, 10, 32, PULSE, 512, F_INT, 0, 1, 0, FAST, 3),
+    "filter_only":        (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "tracts_10":          (TAB_C8, 0, 1, 128, 128, LEAN, 1024, F_INT, 0, 0, 0, FAST, 65),
+    "tracts_128":         (TAB_C8, 0, 1, 128, 128, LEAN, 1024, F_INT, 0, 0, 0, FAST, 65),
+    "no_chunks":          (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "fixed_chunks":       (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "flow_fixed_chunks":  (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 33),
+    "exact":              (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_EXACT, 0, 0, 0, FAST, 9),
+    "slab_97":            (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "ragged":             (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "period_log":         (TAB_FULL, 0, 0, 10, 32, LOG, 512, F_INT, 0, 1, 0, SIMPLE, 2),
+    "simple_gen":         (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "flow_simple_gen":    (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "raw":                (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_FMA, 1, 0, 0, FAST, 5),
+    "gain_10_5":          (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_FMA, 0, 0, 0, FAST, 5),
+    "flow_exact":         (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_EXACT, 0, 0, 0, FAST, 41),
+    "kvar":               (TAB_FULL, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 1, SIMPLE, 0),
+}
+
+# VS_OPT_PLAN_WARPS, streams, glottal noise, period log, busy, burst -> the plan kernel's warp form
+PLAN_WARPS = [
+    (-1, 1024, 0, 0, 1, 2, 1), (-1, 1025, 0, 0, 1, 2, 0),        # a call in flight
+    (-1, 6144, 0, 0, 0, 0, 1), (-1, 6145, 0, 0, 0, 0, 0),        # an idle device
+    (-1, 12288, 1, 0, 0, 0, 1), (-1, 12289, 1, 0, 0, 0, 0),      # an idle device, glottal noise
+    (-1, 1024, 1, 0, 1, 2, 1), (-1, 1025, 1, 0, 1, 2, 0),        # a call in flight, glottal noise
+    (-1, 6144, 0, 0, 1, 1, 1), (-1, 6145, 0, 0, 1, 1, 0),        # the second call of a burst: the idle limit ...
+    (-1, 1024, 1, 0, 1, 1, 1), (-1, 1025, 1, 0, 1, 1, 0),        # ... but not with glottal noise
+    (0, 16, 0, 0, 0, 0, 0), (0, 16, 1, 0, 1, 1, 0),              # option 0: the thread form
+    (1, 50000, 0, 0, 1, 5, 1), (1, 50000, 1, 0, 0, 0, 1),        # option 1: the warp form
+    (-1, 16, 0, 1, 0, 0, 0), (1, 16, 1, 1, 1, 1, 0),             # a period log: the thread form whatever else
+]
 
 
 @pytest.fixture(scope="module")
@@ -95,8 +153,10 @@ def shim(tmp_path_factory):
     L = C.CDLL(str(out))
     L.shim_plan.restype = C.c_int
     L.shim_plan.argtypes = [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                            C.c_double, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_void_p]
+                            C.c_double, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_void_p]
     L.shim_fetch.restype = None
+    L.shim_plan_warps.restype = C.c_int
+    L.shim_plan_warps.argtypes = [C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_uint]
     L.vs_flow_max_periods.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
     return L
 
@@ -129,17 +189,19 @@ def plan(L, s):
     nsamp = None if s["nsamp"] is None else np.ascontiguousarray(s["nsamp"], dtype=np.uint64)
     offs = None if s["offsets"] is None else np.ascontiguousarray(s["offsets"], dtype=np.uint64)
     ptr = lambda a: None if a is None else a.ctypes.data  # noqa: E731
-    info = np.zeros(8, dtype=np.uint64)
-    rc = L.shim_plan(mode, n, fp, ff, ft, ptr(nsamp), ptr(offs), ptr(rec), float(s["chunk"]), s["exact"], s["slab"], SM_COUNT,
-                     int(s["out_dev"]), OUT_BASE if s["out_dev"] else 0, info.ctypes.data)
+    info = np.zeros(16, dtype=np.uint64)
+    rc = L.shim_plan(mode, n, fp, ff, ft, ptr(nsamp), ptr(offs), ptr(rec), float(s["chunk"]), s["exact"], s["slab"],
+                     s["simple_gen"], int(s["raw"]), SM_COUNT, int(s["out_dev"]), OUT_BASE if s["out_dev"] else 0, info.ctypes.data)
     assert rc == 0, rc
-    nc, nr, nsl, warm_total, flow_rows, group_rows, n_groups, n_warm = (int(v) for v in info)
+    nc, nr, nsl, warm_total, flow_rows, group_rows, n_groups, n_warm = (int(v) for v in info[:8])
     r = dict(warm_total=warm_total, flow_rows=bool(flow_rows), group_rows=group_rows, n_groups=n_groups,
+             record=tuple(int(v) for v in info[8:]),
              streams=np.zeros((n, 7), dtype=np.uint64), chunks=np.zeros((nc, 4), dtype=np.uint32),
              order=np.zeros(nr, dtype=np.uint32), slabs=np.zeros((nsl + 1, 4), dtype=np.uint64),
              cta_end=np.zeros((nsl, n_groups), dtype=np.uint32), cache=np.zeros(nsl, dtype=np.uint32),
-             warm=np.zeros(n_warm, dtype=np.int32))
-    L.shim_fetch(*(r[k].ctypes.data_as(C.c_void_p) for k in ("streams", "chunks", "order", "slabs", "cta_end", "cache", "warm")))
+             warm=np.zeros(n_warm, dtype=np.int32), gen=np.zeros(nsl, dtype=np.int32), render_path=np.zeros(nsl, dtype=np.uint32))
+    L.shim_fetch(*(r[k].ctypes.data_as(C.c_void_p)
+                   for k in ("streams", "chunks", "order", "slabs", "cta_end", "cache", "warm", "gen", "render_path")))
     return r
 
 
@@ -215,6 +277,20 @@ def test_batch_plan_invariants(shim, all_shapes, name):
                 assert r["cache"][k] >= sum(tabs.values())
     if name in PINNED:
         assert (len(ck), r["warm_total"]) == PINNED[name]
+
+
+@pytest.mark.parametrize("name", SHAPES)
+def test_batch_plan_kernels(shim, all_shapes, name):
+    r = plan(shim, all_shapes[name])
+    compact, tracts, plan_form, plan_nt, filt, raw, noise, general_pulse = r["record"]
+    record = (compact, int(r["flow_rows"]), tracts, r["n_groups"], r["group_rows"], plan_form, plan_nt, filt, raw, noise, general_pulse)
+    assert record == KERNELS[name][:11]
+    assert set(r["gen"].tolist()) == {KERNELS[name][11]} and set(r["render_path"].tolist()) == {KERNELS[name][12]}
+
+
+def test_plan_warps(shim):
+    for *args, warps in PLAN_WARPS:
+        assert shim.shim_plan_warps(*args) == warps, args
 
 
 def test_batch_plan_shapes_listed(all_shapes):

@@ -13,8 +13,8 @@
 
 #include "vs_batch_plan.h"
 
-cudaError_t vs_launch_plan(const VsPlanArgs &a, bool want_log, bool need_pulse, bool warp_per_stream, cudaStream_t s);
-cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s);
+cudaError_t vs_launch_plan(const VsPlanArgs &a, const VsShape &sh, bool warps, cudaStream_t s);
+cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, const VsShape &sh, int gen, cudaStream_t s);
 static_assert(VS_MAX_TRACTS == VS_MAX_TRACTS_I, "tract count");
 static_assert(VS_MAX_TRACTS <= 256, "a stream's tract index is a uint8_t");
 cudaError_t vs_render_init_device();
@@ -301,7 +301,7 @@ int slot_reserve(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, c
     if (c.b.mode != VS_MODE_FILTER) {
         const std::vector<double> &cos_host = ctx->tables.cos_host;
         if ((rc = ring_dev(sl.table, (sl.plan.tab_total + 8) * VS_TAB_ENTRY_BYTES(c.sh.compact)))) return rc;
-        if (ctx->in.facts.any_noise && (rc = ring_dev(sl.snap, nc * 32 * sizeof(uint32_t)))) return rc;
+        if (c.sh.noise && (rc = ring_dev(sl.snap, nc * 32 * sizeof(uint32_t)))) return rc;
         if ((rc = dev_reserve(ctx, sl, sl.costab, (cos_host.size() + VS_COS_SLACK) * sizeof(double)))) return rc;
         if (sl.costab_uploaded != cos_host.size()) {
             /* tables only ever grow; a synchronous copy keeps the host vector free to grow again */
@@ -328,7 +328,6 @@ int slot_reserve(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, c
 /* the plan kernel of every slab, on the plan stream (flow and synth modes) */
 int launch_plans(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t s0, const std::vector<VsRange> &slabs, cudaStream_t pstream)
 {
-    const bool any_noise = ctx->in.facts.any_noise;
     for (const VsRange &slab : slabs) {
         VsPlanArgs pa;
         memset(&pa, 0, sizeof pa);
@@ -337,37 +336,24 @@ int launch_plans(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t s0, c
         pa.chunks = (VsChunk *)sl.chunks[cp].p;
         pa.table = sl.table[cp].p;
         pa.compact = c.sh.compact;
-        pa.rng_snap = any_noise ? (uint32_t *)sl.snap[cp].p : nullptr;
+        pa.rng_snap = c.sh.noise ? (uint32_t *)sl.snap[cp].p : nullptr;
         pa.n_periods = (uint32_t *)sl.nper[cp].p + (slab.first - s0);
         pa.costab = (const double *)sl.costab.p;
         pa.log = c.want_log ? sl.log.p : nullptr;
         pa.status = (int32_t *)sl.status[cp].p;
-        pa.need_pulse = c.want_log;
-        /* One warp per stream while the batch is too small to fill the GPU with one thread per stream
-         * (measured crossover on B200: ~8 k streams, ~14 k with glottal noise, where a thread walks
-         * hundreds of serial pulse samples and draws per period).  The warp form issues ~7x the
-         * instructions, though: when the previous call is still rendering it would take issue slots
-         * from the FP64-bound render warps, while the thread form hides on its own SMs -- so with a
-         * call in flight only really small batches take it. */
-        bool plan_warps;
-        if (ctx->opt_plan_warps >= 0) plan_warps = ctx->opt_plan_warps != 0;
-        else {
+        bool busy = false;
+        if (ctx->opt_plan_warps < 0) {
             /* "in flight" = the previous call has not finished, or it was enqueued less than 2 ms ago (a
              * loop of calls whose host side momentarily fell behind the GPU is still a pipeline) */
-            bool busy = cudaEventQuery(sl.call_done[(cp + VS_DEPTH - 1u) % VS_DEPTH]) == cudaErrorNotReady;
+            busy = cudaEventQuery(sl.call_done[(cp + VS_DEPTH - 1u) % VS_DEPTH]) == cudaErrorNotReady;
             (void)cudaGetLastError();
             const auto now = std::chrono::steady_clock::now();
             if (std::chrono::duration<double, std::milli>(now - sl.last_enqueue).count() < 2.0) busy = true;
             sl.last_enqueue = now;
-            /* the second call of a burst that began on an idle device: its plan must be ready when the first
-             * call's render ends, one render time from now -- the thread form (0.39 ms on the bench batch, and it
-             * has to wait for free SMs behind the first call's warp-form plan) would be late by a quarter of a
-             * step, and every call behind it too until the pipeline has settled */
             sl.burst = busy ? sl.burst + 1u : 0u;
-            const bool early = busy && sl.burst == 1u && !any_noise;     /* (with glottal noise the warp form is too heavy to share the SMs with a render: cfg3 157 -> 150 Gsamples/s) */
-            plan_warps = pa.n_streams <= (busy && !early ? VS_PLAN_WARP_MAX : any_noise ? VS_PLAN_WARP_MAX_NOISE : VS_PLAN_WARP_MAX_IDLE);
         }
-        CU(vs_launch_plan(pa, c.want_log, any_noise || c.want_log, plan_warps, pstream));
+        const bool warps = vs_plan_warps(ctx->opt_plan_warps, pa.n_streams, c.sh.noise, c.want_log, busy, sl.burst);
+        CU(vs_launch_plan(pa, c.sh, warps, pstream));
         ctx->timing.launches++;
     }
     return VS_OK;
@@ -379,7 +365,6 @@ int render_slab(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, si
 {
     const VsBatch &b = c.b;
     const std::vector<VsStream> &hs = ctx->in.hs;
-    const VsFacts &fc = ctx->in.facts;
     const int d = (int)((sl.scratch_parity + k) & 1);
     int16_t *d_pcm = c.out_dev ? b.pcm_out : (int16_t *)sl.pcm[d].p;
     double *d_raw = b.raw_out ? (c.out_dev ? b.raw_out : (double *)sl.raw[d].p) : nullptr;
@@ -400,24 +385,19 @@ int render_slab(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, si
     const VsPlan &pl = sl.plan;
     VsRenderArgs ra;
     memset(&ra, 0, sizeof ra);
+    const int gen = vs_render_geometry(ctx->opt, c.sh, ctx->in.facts, sl.sm_count, ns, pl, k, ra);
     ra.streams = (const VsStream *)sl.streams[cp].p;
     ra.chunks = (const VsChunk *)sl.chunks[cp].p;
     ra.order = (const uint32_t *)sl.order[cp].p + pl.slab_r0[k];
-    ra.n_rows = (uint32_t)(pl.slab_r0[k + 1] - pl.slab_r0[k]);
-    memcpy(ra.cta_end, pl.geom[k].cta_end, sizeof ra.cta_end);
     ra.table = sl.table[cp].p;
-    ra.compact = c.sh.compact;
     ra.n_periods = (const uint32_t *)sl.nper[cp].p;
-    ra.rng_snap = fc.any_noise ? (const uint32_t *)sl.snap[cp].p : nullptr;
+    ra.rng_snap = c.sh.noise ? (const uint32_t *)sl.snap[cp].p : nullptr;
     ra.costab = (const double *)sl.costab.p;
     ra.flow_in = d_in;
     ra.pcm_out = d_pcm;
     ra.raw_out = d_raw;
-    ra.general_pulse = fc.any_kvar ? 1 : 0;
     ra.debug = (uint32_t)ctx->opt_debug;
     ra.status = (int32_t *)sl.status[cp].p;
-    const int gen = vs_render_geometry(ctx->opt, c.sh, fc, sl.sm_count, ns, pl.geom[k].cache_doubles, ra);
-    const int filt = ctx->opt.exact ? VS_FILT_EXACT : ((fc.int_filter && !b.raw_out) ? VS_FILT_INT : VS_FILT_FMA);
     if (c.sh.flow_rows) {
         if (!sl.ticket.p) {
             const int rc = dev_reserve(ctx, sl, sl.ticket, 256);
@@ -434,13 +414,11 @@ int render_slab(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, si
         memcpy(tb.cta_end, pl.geom[k].cta_end, sizeof tb.cta_end);
         memset(tb.ncoef, 0, sizeof tb.ncoef);
         memcpy(tb.ncoef, ctx->in.ncoef.data(), ctx->in.ncoef.size() * sizeof(double));
-        CU(vs_launch_render(ra, &tb, b.mode, gen, fc.any_noise, filt, sl.compute));
+        CU(vs_launch_render(ra, &tb, c.sh, gen, sl.compute));
     } else
-        CU(vs_launch_render(ra, nullptr, b.mode, gen, fc.any_noise, filt, sl.compute));
+        CU(vs_launch_render(ra, nullptr, c.sh, gen, sl.compute));
     ctx->timing.launches++;
-    ctx->timing.render_path = (gen == VS_GEN_FAST || c.sh.flow_rows ? 1u : 0u) | (fc.any_noise ? 2u : 0u) |
-                              ((uint32_t)(b.raw_out && filt == VS_FILT_INT ? VS_FILT_FMA : filt) << 2) |
-                              (c.sh.flow_rows ? 32u : 0u) | (c.sh.tracts ? 64u : 0u);
+    ctx->timing.render_path = vs_render_path(c.sh, gen);
     if (timed) { cudaEvent_t e2 = timing_event(sl); CU(cudaEventRecord(e2, sl.compute)); }
     if (c.out_dev) return VS_OK;
 
@@ -672,7 +650,8 @@ int run_batch(vs_ctx *ctx, const VsBatch &b)
     ctx->timing_pending = true;
 
     /* ---- 4. per slot: plan, descriptors up, then slabs of plan -> render -> copy -------------- */
-    const Call call = {b, want_log, same_inputs, out_dev, vs_shape(b.mode, b.ft != nullptr, want_log, ctx->in.facts, o),
+    const Call call = {b, want_log, same_inputs, out_dev,
+                       vs_shape(b.mode, b.ft != nullptr, want_log, ctx->in.facts, o),
                        out_dev ? (uint64_t)(reinterpret_cast<uintptr_t>(b.pcm_out) >> 1) : 0u, prof};
     for (size_t g = 0; g < nslots; g++) {
         if (cut[g + 1] <= cut[g]) continue;

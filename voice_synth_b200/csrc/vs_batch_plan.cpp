@@ -254,6 +254,7 @@ int vs_build_descriptors(const VsBatch &b, bool want_log, VsTables &tab, VsDescr
     std::vector<VsStream> &hs = d.hs;
     hs.assign(n, VsStream());
     VsFacts fc;
+    fc.raw = b.raw_out != nullptr;
     /* filter groups: the ten presets, or the caller's tracts (validated, warm-ups from the context's cache) */
     d.warm.assign(tab.warm, tab.warm + VS_NUM_PRESETS);
     d.ncoef.clear();
@@ -357,6 +358,9 @@ int vs_build_descriptors(const VsBatch &b, bool want_log, VsTables &tab, VsDescr
     return VS_OK;
 }
 
+/* what both branch-free generators (VS_GEN_FAST, vs_flow_rows_kernel) need: amplitudes within a short, periods >= 24 */
+static bool branch_free(const VsFacts &fc, const VsPlanOptions &o) { return fc.amp_fits && !o.simple_gen && fc.t_min >= 24; }
+
 VsShape vs_shape(int mode, bool tracts, bool want_log, const VsFacts &fc, const VsPlanOptions &o)
 {
     VsShape sh;
@@ -365,10 +369,16 @@ VsShape vs_shape(int mode, bool tracts, bool want_log, const VsFacts &fc, const 
     /* period table format: 8-byte entries (amplitude, length) where they suffice, 16-byte ones for plain glottal noise */
     sh.compact = (fc.any_kvar || want_log) ? VS_TAB_FULL : !fc.any_noise ? VS_TAB_C8 : fc.noise_simple ? VS_TAB_N16 : VS_TAB_FULL;
     /* flow without glottal noise: lanes along the row (vs_flow_rows_kernel).  T2 >= 2: row_validate() bounds A*K then */
-    sh.flow_rows = mode == VS_MODE_FLOW && sh.compact == VS_TAB_C8 && fc.amp_fits && !o.simple_gen && fc.t_min >= 24 && fc.t2_min >= 2;
+    sh.flow_rows = mode == VS_MODE_FLOW && sh.compact == VS_TAB_C8 && branch_free(fc, o) && fc.t2_min >= 2;
     sh.ph_mask = sh.flow_rows ? 63u : 7u;
-    /* streams per CTA of the thread-form plan kernel: without glottal noise and period log its lean form (vs_plan.cu) */
-    sh.plan_nt = (fc.any_noise || want_log) ? VS_PLAN_NT : VS_PLAN_NT_LEAN;
+    /* the plan kernel evaluates the open phase only for glottal noise and the period log; without either its lean form */
+    sh.plan = want_log ? VS_PLAN_LOG : fc.any_noise ? VS_PLAN_PULSE : VS_PLAN_LEAN;
+    sh.plan_nt = sh.plan == VS_PLAN_LEAN ? VS_PLAN_NT_LEAN : VS_PLAN_NT;
+    /* no integer-filter kernel writes raw output.  (Flow-only calls run no filter; render_path reports this value anyway) */
+    sh.filt = o.exact ? VS_FILT_EXACT : fc.int_filter && !fc.raw ? VS_FILT_INT : VS_FILT_FMA;
+    sh.raw = fc.raw;
+    sh.noise = fc.any_noise;
+    sh.general_pulse = fc.any_kvar;
     sh.n_groups = tracts ? VS_MAX_TRACTS_I : VS_NUM_PRESETS;
     sh.group_rows = tracts ? VS_NT : 32;   /* groups are padded to whole CTAs (tracts) or blocks of 32 rows (presets) */
     return sh;
@@ -657,9 +667,13 @@ void vs_plan_assign(const VsPlan &p, std::vector<VsStream> &hs, size_t s0, size_
     }
 }
 
-int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts &fc, int sm_count, size_t ns,
-                       uint32_t cache_doubles, VsRenderArgs &ra)
+int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts &fc, int sm_count, size_t ns, const VsPlan &p,
+                       size_t k, VsRenderArgs &ra)
 {
+    ra.n_rows = (uint32_t)(p.slab_r0[k + 1] - p.slab_r0[k]);
+    memcpy(ra.cta_end, p.geom[k].cta_end, sizeof ra.cta_end);
+    ra.compact = sh.compact;
+    ra.general_pulse = sh.general_pulse ? 1 : 0;
     /* shared-memory geometry.  The fast generator keeps, per lane, a ring of upcoming period entries (filled
      * one window ahead) and, per warp, the pulse tables of its rows; when the pitch periods of the batch are
      * too short or the tables too many for that, the general generator takes over. */
@@ -667,7 +681,7 @@ int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts 
     const uint32_t tile_bytes = (uint32_t)VS_RENDER_TILES(sh.mode) * 32u * (uint32_t)win * 2u;
     int gen = VS_GEN_SIMPLE;
     ra.warp_bytes = tile_bytes;
-    if (sh.mode != VS_MODE_FILTER && sh.compact != VS_TAB_FULL && fc.amp_fits && !o.simple_gen && fc.t_min >= 24 && fc.t_max <= 8192) {
+    if (sh.mode != VS_MODE_FILTER && sh.compact != VS_TAB_FULL && branch_free(fc, o) && fc.t_max <= 8192) {
         /* pitch periods a lane can enter in one window (+1: the generator may already have promoted the period
          * that starts with the next window); the ring holds two windows' worth */
         const uint32_t per_win = (uint32_t)((win + fc.t_min - 1) / fc.t_min) + 1u;
@@ -678,7 +692,7 @@ int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts 
          * (a warp that needs more renders its rows with the general generator) */
         const uint32_t budget = (sh.mode == VS_MODE_FLOW ? 100u : 200u) * 1024u / 4u;
         const uint32_t fixed = tile_bytes + R * 32u * VS_TAB_ENTRY_BYTES(sh.compact);
-        uint32_t cache = std::max(16u, (cache_doubles + 1u) & ~1u);
+        uint32_t cache = std::max(16u, (p.geom[k].cache_doubles + 1u) & ~1u);
         if (fixed + 4096u <= budget) cache = std::min(cache, ((budget - fixed) / 8u) & ~1u);
         const uint32_t wbytes = fixed + cache * 8u;
         if (R <= 64 && wbytes <= budget) {
@@ -692,13 +706,35 @@ int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts 
     const int plan_ctas = (int)((ns + (size_t)sh.plan_nt - 1) / (size_t)sh.plan_nt);
     const uint32_t sms = (uint32_t)std::max(1, sm_count - vs_plan_reserve(plan_ctas));
     uint32_t per_sm = 1;
-    if (sh.mode == VS_MODE_FLOW) per_sm = std::max(1u, std::min(4u, (220u * 1024u) / (4u * ra.warp_bytes + (fc.any_noise ? 16u * 1024u : 0u) + 1024u)));
+    if (sh.mode == VS_MODE_FLOW) per_sm = std::max(1u, std::min(4u, (220u * 1024u) / (4u * ra.warp_bytes + (sh.noise ? 16u * 1024u : 0u) + 1024u)));
     ra.grid = std::min(blocks, sms * per_sm);
     if (sh.flow_rows) {
         const uint32_t rows_per_cta = VS_FLOWROWS_WARPS;
         ra.grid = std::max(1u, std::min((ra.n_rows + rows_per_cta - 1u) / rows_per_cta, sms * 4u));
     }
     return gen;
+}
+
+uint32_t vs_render_path(const VsShape &sh, int gen)
+{
+    return (gen == VS_GEN_FAST || sh.flow_rows ? 1u : 0u) | (sh.noise ? 2u : 0u) | ((uint32_t)sh.filt << 2) | (sh.flow_rows ? 32u : 0u) |
+           (sh.tracts ? 64u : 0u);
+}
+
+/* One warp per stream while the batch is too small to fill the GPU with one thread per stream (measured crossover on
+ * B200: ~8 k streams, ~14 k with glottal noise).  The warp form issues ~7x the instructions, though: next to a render
+ * still running it would take issue slots from the FP64-bound render warps, while the thread form hides on its own SMs
+ * -- so with a call in flight only really small batches take it. */
+bool vs_plan_warps(int opt_plan_warps, size_t n_streams, bool any_noise, bool want_log, bool busy, unsigned burst)
+{
+    if (want_log) return false;                     /* the warp form writes no period log */
+    if (opt_plan_warps >= 0) return opt_plan_warps != 0;
+    /* the second call of a burst that began on an idle device: its plan must be ready when the first call's render ends;
+     * the thread form (0.39 ms on the bench batch, behind the first call's warp-form plan) would be late by a quarter of a
+     * step, and every call behind it too.  (With glottal noise the warp form is too heavy to share the SMs with a render:
+     * cfg3 157 -> 150 Gsamples/s) */
+    const bool early = busy && burst == 1u && !any_noise;
+    return n_streams <= (busy && !early ? VS_PLAN_WARP_MAX : any_noise ? VS_PLAN_WARP_MAX_NOISE : VS_PLAN_WARP_MAX_IDLE);
 }
 
 /* ---- the C ABI's helpers that do no GPU work ------------------------------------------------------------------- */

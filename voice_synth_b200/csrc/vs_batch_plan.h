@@ -66,6 +66,7 @@ struct VsFacts {
     bool int_filter = true;         /* every stream: integral gain, pre-emphasis 0 or 1 -> both commute to the integer input */
     bool amp_fits = true;           /* no amplitude can pass 32767 (fast generator) */
     bool noise_simple = true;       /* every noisy stream has DC <= 1 (then T4 == 0) and T2 >= 16: 16-byte period entries do */
+    bool raw = false;               /* the call asks for raw (double) output besides the PCM */
     int t_min = 0x7fffffff, t_max = 0, t2_min = 0x7fffffff;   /* bounds on the pitch periods; shortest half open phase */
 };
 struct VsDescriptors {
@@ -77,16 +78,23 @@ struct VsDescriptors {
 /* VS_OK, or an error code and its message in err; the tables may have grown either way */
 int vs_build_descriptors(const VsBatch &b, bool want_log, VsTables &tab, VsDescriptors &d, std::string &err);
 
-struct VsShape {                    /* the kernel forms of a batch */
+struct VsShape {                    /* the kernel forms of a batch: the kernels its launches run, but for the generator */
     int mode;
     bool tracts, flow_rows;         /* flow_rows: flow on vs_flow_rows_kernel, a warp per row */
     int compact;                    /* period table format, VS_TAB_* */
     uint64_t ph_mask;               /* a row's phase is its output address (in samples) & ph_mask */
-    int plan_nt;                    /* streams per CTA of the thread-form plan kernel */
+    int plan, plan_nt;              /* thread-form plan kernel, VS_PLAN_*, and its streams per CTA */
+    int filt;                       /* filter arithmetic, VS_FILT_* (never VS_FILT_INT with raw output) */
+    bool raw;                       /* raw (double) output besides the PCM */
+    bool noise, general_pulse;      /* some stream has glottal noise; some stream has -z (Kvar > 0), see VsRenderArgs */
     int n_groups;                   /* filter groups: presets or tracts ... */
     size_t group_rows;              /* ... each padded to this many rows */
 };
 VsShape vs_shape(int mode, bool tracts, bool want_log, const VsFacts &fc, const VsPlanOptions &o);
+
+/* the thread-form plan kernel (false) or the warp form (true) for a slab of n_streams.  busy: the previous call is
+ * still on the device; burst: calls since one found it idle.  opt_plan_warps: VS_OPT_PLAN_WARPS, -1 auto */
+bool vs_plan_warps(int opt_plan_warps, size_t n_streams, bool any_noise, bool want_log, bool busy, unsigned burst);
 
 /* stage 3: streams [cut[g], cut[g+1]) go to device slot g; a slot's streams go in slabs, launched and copied together */
 typedef std::pair<size_t, size_t> VsRange;
@@ -112,10 +120,12 @@ void vs_plan_chunks(const VsPlanOptions &o, const VsShape &sh, int sm_count, con
 void vs_plan_rows(const VsShape &sh, const std::vector<VsStream> &hs, size_t s0, VsPlan &p);   /* 4b, row order */
 void vs_plan_assign(const VsPlan &p, std::vector<VsStream> &hs, size_t s0, size_t s1);         /* chunk0, n_chunks, tab_off */
 
-/* the generator (VS_GEN_*), shared-memory geometry and grid of a slab's render launch, into ra (n_rows set); ns: the
- * slot's streams */
-int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts &fc, int sm_count, size_t ns,
-                       uint32_t cache_doubles, VsRenderArgs &ra);
+/* the generator (VS_GEN_*) of slab k's render launch; into ra what the plan decides of that launch: rows and group ends,
+ * table format, pulse form, shared-memory geometry and grid.  ns: the slot's streams */
+int vs_render_geometry(const VsPlanOptions &o, const VsShape &sh, const VsFacts &fc, int sm_count, size_t ns, const VsPlan &p,
+                       size_t k, VsRenderArgs &ra);
+/* vs_timing::render_path of a launch with generator gen */
+uint32_t vs_render_path(const VsShape &sh, int gen);
 
 #pragma GCC visibility pop
 #endif

@@ -15,7 +15,7 @@
 #define VS_PLAN_NT_LEAN 1024   /* ... of its form without the open phase (no glottal noise, no period log): 64 registers */
 #define VS_PLAN_SMEM (96 * 1024)
 #define VS_PLAN_SMS  32         /* most SMs the chunk planner leaves to the plan kernels of the next two calls */
-/* batches up to this many streams get one WARP per stream in the plan kernel (vs_api.cu, plan launch) */
+/* batches up to this many streams get one WARP per stream in the plan kernel (vs_batch_plan.cpp, vs_plan_warps) */
 #define VS_PLAN_WARP_MAX       1024    /* while the previous call is still on the GPU */
 #define VS_PLAN_WARP_MAX_IDLE  6144    /* GPU idle: the plan kernel is the call's critical path */
 #define VS_PLAN_WARP_MAX_NOISE 12288   /* some streams carry glottal noise */
@@ -34,6 +34,7 @@
 enum { VS_MODE_FLOW = 0, VS_MODE_SYNTH = 1, VS_MODE_FILTER = 2 };
 enum { VS_GEN_FAST = 0, VS_GEN_SIMPLE = 1 };
 enum { VS_FILT_INT = 0, VS_FILT_FMA = 1, VS_FILT_EXACT = 2 };
+enum { VS_PLAN_LEAN = 0, VS_PLAN_PULSE = 1, VS_PLAN_LOG = 2 };   /* thread-form plan kernel: no pulse, pulse, pulse + log */
 #define VS_WIN(MODE) ((MODE) == VS_MODE_SYNTH ? VS_WIN_SYNTH : (MODE) == VS_MODE_FLOW ? VS_WIN_FLOW : VS_WIN_FILTER)
 /* tiles per 32 rows of the render kernel.  Fused / filter-only: F's, G's and the one the TMA engine reads.  Flow
  * only: one -- four CTAs share an SM and the other warps run while a warp waits for its tile to be read out */
@@ -117,7 +118,6 @@ struct VsPlanArgs {
     const double   *costab;
     void           *log;            /* vs_period_rec* or NULL                                     */
     int32_t        *status;         /* device error flag                                          */
-    int             need_pulse;     /* evaluate the pulse for every stream (log requested)        */
 };
 
 struct VsRenderArgs {

@@ -14,6 +14,7 @@
  * written with explicit round-to-nearest intrinsics in the reference's evaluation order, so those
  * results are bit-exact.
  */
+#include "vs_batch_plan.h"
 #include "vs_device.cuh"
 
 /* ================================================================================================
@@ -651,25 +652,26 @@ cudaError_t vs_launch_fp64_peak(double *scratch, int blocks, int iters, cudaStre
 /* ------------------------------------------------------------------------------------------------
  * launch wrappers (called from vs_api.cu)
  * ---------------------------------------------------------------------------------------------- */
-cudaError_t vs_launch_plan(const VsPlanArgs &a, bool want_log, bool need_pulse, bool warp_per_stream, cudaStream_t s)
+/* warps: the warp form (vs_plan_warps); otherwise the record's thread form, sh.plan_nt streams per CTA */
+cudaError_t vs_launch_plan(const VsPlanArgs &a, const VsShape &sh, bool warps, cudaStream_t s)
 {
-    if (warp_per_stream && !want_log) {
+    if (warps) {
         vs_plan_warp_kernel<<<(a.n_streams + VS_PLANW_NT / 32 - 1) / (VS_PLANW_NT / 32), VS_PLANW_NT, 0, s>>>(a);
         return cudaGetLastError();
     }
-    const unsigned grid = (a.n_streams + VS_PLAN_NT - 1) / VS_PLAN_NT;
+    const unsigned grid = (a.n_streams + sh.plan_nt - 1) / sh.plan_nt;
     static_assert(VS_PLAN_SMEM >= VS_RNG_DEG * VS_PLAN_NT * 4, "plan kernel shared memory");
-    if (want_log) {
+    if (sh.plan == VS_PLAN_LOG) {
         cudaFuncSetAttribute(vs_plan_kernel<true, true, VS_PLAN_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, VS_PLAN_SMEM);
         vs_plan_kernel<true, true, VS_PLAN_NT><<<grid, VS_PLAN_NT, VS_PLAN_SMEM, s>>>(a);
-    } else if (need_pulse) {
+    } else if (sh.plan == VS_PLAN_PULSE) {
         cudaFuncSetAttribute(vs_plan_kernel<false, true, VS_PLAN_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, VS_PLAN_SMEM);
         vs_plan_kernel<false, true, VS_PLAN_NT><<<grid, VS_PLAN_NT, VS_PLAN_SMEM, s>>>(a);
     } else {
         constexpr int smem = VS_RNG_DEG * VS_PLAN_NT_LEAN * 4;
         static_assert(smem >= VS_PLAN_SMEM, "the lean plan CTA must not share an SM with a render CTA either");
         cudaFuncSetAttribute(vs_plan_kernel<false, false, VS_PLAN_NT_LEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        vs_plan_kernel<false, false, VS_PLAN_NT_LEAN><<<(a.n_streams + VS_PLAN_NT_LEAN - 1) / VS_PLAN_NT_LEAN, VS_PLAN_NT_LEAN, smem, s>>>(a);
+        vs_plan_kernel<false, false, VS_PLAN_NT_LEAN><<<grid, VS_PLAN_NT_LEAN, smem, s>>>(a);
     }
     return cudaGetLastError();
 }

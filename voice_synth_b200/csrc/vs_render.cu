@@ -24,8 +24,8 @@
  * Exact mode (VS_OPT_EXACT_FILTER) keeps the reference's unfused multiply/subtract order and its floor-based
  * round2int() bit for bit.
  */
+#include "vs_batch_plan.h"
 #include "vs_device.cuh"
-#include "vs_presets.h"
 
 #include <type_traits>
 
@@ -691,31 +691,30 @@ static cudaError_t vs_go(const VsRenderArgs &a, const VsTractBlock *tb, cudaStre
     return cudaGetLastError();
 }
 
+/* the record's filter arithmetic and raw output (no integer-filter kernel writes raw output) */
 template <int MODE, int GEN, bool NOISE, bool TRACT>
-static cudaError_t vs_go_filt(const VsRenderArgs &a, const VsTractBlock *tb, int filt, cudaStream_t s)
+static cudaError_t vs_go_filt(const VsRenderArgs &a, const VsTractBlock *tb, const VsShape &sh, cudaStream_t s)
 {
-    const bool raw = a.raw_out != nullptr;
-    if (filt == VS_FILT_EXACT) return raw ? vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, true, TRACT>(a, tb, s) : vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, false, TRACT>(a, tb, s);
-    if (raw) return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, true, TRACT>(a, tb, s);
-    if (filt == VS_FILT_INT) return vs_go<MODE, GEN, NOISE, VS_FILT_INT, false, TRACT>(a, tb, s);
-    return vs_go<MODE, GEN, NOISE, VS_FILT_FMA, false, TRACT>(a, tb, s);
+    if (sh.filt == VS_FILT_INT) return vs_go<MODE, GEN, NOISE, VS_FILT_INT, false, TRACT>(a, tb, s);
+    if (sh.filt == VS_FILT_EXACT) return sh.raw ? vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, true, TRACT>(a, tb, s) : vs_go<MODE, GEN, NOISE, VS_FILT_EXACT, false, TRACT>(a, tb, s);
+    return sh.raw ? vs_go<MODE, GEN, NOISE, VS_FILT_FMA, true, TRACT>(a, tb, s) : vs_go<MODE, GEN, NOISE, VS_FILT_FMA, false, TRACT>(a, tb, s);
 }
 
-template <bool TRACT>
-static cudaError_t vs_go_filter_modes(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s)
+/* The render kernel the record and the slab's generator (VS_GEN_*) select.  Flow only runs no filter; filter only
+ * generates nothing.  tb: the caller's vocal tracts when sh.tracts */
+cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, const VsShape &sh, int gen, cudaStream_t s)
 {
-    if (mode == VS_MODE_FILTER) return vs_go_filt<VS_MODE_FILTER, VS_GEN_SIMPLE, false, TRACT>(a, tb, filt, s);
-    if (gen == VS_GEN_FAST) return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, true, TRACT>(a, tb, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, false, TRACT>(a, tb, filt, s);
-    return noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, true, TRACT>(a, tb, filt, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, false, TRACT>(a, tb, filt, s);
-}
-
-/* gen: VS_GEN_FAST / VS_GEN_SIMPLE; filt: VS_FILT_INT / _FMA / _EXACT (raw output forces _FMA or _EXACT);
- * tb: the caller's vocal tracts (synth and filter modes), nullptr for the presets */
-cudaError_t vs_launch_render(const VsRenderArgs &a, const VsTractBlock *tb, int mode, int gen, bool noise, int filt, cudaStream_t s)
-{
-    if (mode == VS_MODE_FLOW) {
-        if (gen == VS_GEN_FAST) return noise ? vs_go<VS_MODE_FLOW, VS_GEN_FAST, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_FAST, false, VS_FILT_FMA, false>(a, nullptr, s);
-        return noise ? vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, false, VS_FILT_FMA, false>(a, nullptr, s);
+    const bool fast = gen == VS_GEN_FAST;
+    if (sh.mode == VS_MODE_FLOW) {
+        if (fast) return sh.noise ? vs_go<VS_MODE_FLOW, VS_GEN_FAST, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_FAST, false, VS_FILT_FMA, false>(a, nullptr, s);
+        return sh.noise ? vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, true, VS_FILT_FMA, false>(a, nullptr, s) : vs_go<VS_MODE_FLOW, VS_GEN_SIMPLE, false, VS_FILT_FMA, false>(a, nullptr, s);
     }
-    return tb ? vs_go_filter_modes<true>(a, tb, mode, gen, noise, filt, s) : vs_go_filter_modes<false>(a, nullptr, mode, gen, noise, filt, s);
+    if (sh.mode == VS_MODE_FILTER)
+        return sh.tracts ? vs_go_filt<VS_MODE_FILTER, VS_GEN_SIMPLE, false, true>(a, tb, sh, s) : vs_go_filt<VS_MODE_FILTER, VS_GEN_SIMPLE, false, false>(a, tb, sh, s);
+    if (sh.tracts) {
+        if (fast) return sh.noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, true, true>(a, tb, sh, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, false, true>(a, tb, sh, s);
+        return sh.noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, true, true>(a, tb, sh, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, false, true>(a, tb, sh, s);
+    }
+    if (fast) return sh.noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, true, false>(a, tb, sh, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_FAST, false, false>(a, tb, sh, s);
+    return sh.noise ? vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, true, false>(a, tb, sh, s) : vs_go_filt<VS_MODE_SYNTH, VS_GEN_SIMPLE, false, false>(a, tb, sh, s);
 }
