@@ -11,7 +11,12 @@
  *   acoustic -F [-p order] file.wav [file.wav ...]         formant analysis of vowel PCM (vs_formant_batch, default
  *                                                          options; -p sets the LPC order, 2..32, even)
  * One line per file:  name  fs  samples  frames  analysed  F1..Fn[Hz]  B1..Bn[Hz]   (the means over the analysed frames,
- *    n = min(5, order/2); nan where no frame has that many formants) */
+ *    n = min(5, order/2); nan where no frame has that many formants)
+ *
+ *   acoustic -P file.wav [file.wav ...]                    pitch and harmonicity of vowel PCM (vs_pitch_batch, default
+ *                                                          options: 75-600 Hz, 3 periods per window, 10 ms hop)
+ * One line per file:  name  fs  samples  frames  voiced  F0_mean[Hz]  F0_sd[Hz]  HNR_mean[dB]   (nan where no frame is
+ *    voiced, resp. periodic) */
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -21,13 +26,16 @@
 
 int main(int argc, char **argv)
 {
-    int lo = 0, hi = 0, a = 1, report = 0, formants = 0, order = 14;
+    int lo = 0, hi = 0, a = 1, report = 0, formants = 0, pitch = 0, order = 14;
     for (;;) {
         if (a < argc && strcmp(argv[a], "-x") == 0) {
             report = 1;
             a += 1;
         } else if (a < argc && strcmp(argv[a], "-F") == 0) {
             formants = 1;
+            a += 1;
+        } else if (a < argc && strcmp(argv[a], "-P") == 0) {
+            pitch = 1;
             a += 1;
         } else if (a + 1 < argc && strcmp(argv[a], "-p") == 0) {
             order = atoi(argv[a + 1]);
@@ -42,7 +50,8 @@ int main(int argc, char **argv)
     if (a >= argc || lo > hi || lo < -32768 || hi > 32767 || order < 2 || order > 32 || order % 2) {
         printf("usage: acoustic [-l lo] [-h hi] [-x] file.wav [file.wav ...]   (lo <= hi: thresholds of the onset trigger;"
                " -x: voice report columns)\n"
-               "       acoustic -F [-p order] file.wav [file.wav ...]          (formants of vowel PCM; order even, 2..32)\n");
+               "       acoustic -F [-p order] file.wav [file.wav ...]          (formants of vowel PCM; order even, 2..32)\n"
+               "       acoustic -P file.wav [file.wav ...]                     (pitch and harmonicity of vowel PCM)\n");
         return 0;
     }
     const size_t n = (size_t)(argc - a);
@@ -81,6 +90,16 @@ int main(int argc, char **argv)
             for (uint32_t k = 0; k < fo.n_formants; k++) printf(" %.1f", fs_out[i].bw_mean_hz[k]);
             printf("\n");
         }
+        vs_ctx_destroy(ctx);
+        return 0;
+    }
+    if (pitch) {
+        vs_pitch_stats *ps = (vs_pitch_stats *)calloc(n, sizeof *ps);
+        rc = vs_pitch_batch(ctx, flow, offs, ns, fs, n, NULL, ps, NULL, NULL);
+        if (rc) { fprintf(stderr, "acoustic: %s (%s)\n", vs_strerror(rc), vs_last_error(ctx)); return 1; }
+        for (size_t i = 0; i < n; i++)
+            printf("%s %d %llu %u %u %.3f %.3f %.2f\n", argv[a + i], fs[i], (unsigned long long)ns[i], ps[i].frames, ps[i].voiced,
+                   ps[i].f0_mean_hz, ps[i].f0_sd_hz, ps[i].hnr_mean_db);
         vs_ctx_destroy(ctx);
         return 0;
     }

@@ -299,6 +299,70 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
                      size_t n, const vs_formant_opts *o, vs_formant_stats *stats,
                      vs_formant_frame *frames, const uint64_t *frame_offsets);
 
+/* Pitch and harmonicity of PCM (the F0 and noise axes of rendered vowels): Boersma's (1993) autocorrelation corrected
+ * for the window, frame by frame, without Praat's path finder; the options and their defaults are those of Praat's
+ * "To Pitch (ac)" (periods = 4.5 gives the window of "To Harmonicity (ac)").  The definitions are the library's own;
+ * tests/pitch_ref.py restates them in numpy.  With fs the stream's rate (fs NULL: 22050 for every stream):
+ *   geometry   Nw = lround(periods fs / f_min), H = lround(hop_ms fs / 1000), tau_lo = max(2, ceil(fs / f_max)),
+ *              tau_hi = floor(fs / f_min), all in double; a stream of n samples has n >= Nw ? (n - Nw) / H + 1 : 0
+ *              frames, frame f covers samples [f H, f H + Nw);
+ *   signal     mu_f = the frame's mean (an exact integer sum over Nw), a[m] = x[fH+m] - mu_f, the local peak
+ *              P_f = max |a[m]|; w[m] = 0.5 - 0.5 cos(2 pi (m + 1/2) / Nw), y[m] = a[m] w[m], in FP64.  w and r_w are
+ *              computed on the host with libm in double, r_w in index order;
+ *   lags       r_a(tau) = sum_{m < Nw - tau} y[m] y[m+tau] in FP64 in any order, for tau = 0 and tau_lo-1 .. tau_hi+1;
+ *              r_w(tau) the same sum over w; r(tau) = (r_a(tau) / r_a(0)) (r_w(0) / r_w(tau)).  r_a(0) == 0 (a constant
+ *              frame): VS_PITCH_SILENT;
+ *   candidate  a tau in [tau_lo, tau_hi] with r(tau) > r(tau-1), r(tau) >= r(tau+1) and r(tau) > 0.  With a, b, c =
+ *              r(tau-1), r(tau), r(tau+1): d = 0.5 (a - c) / (a - 2b + c), tau* = tau + d, r* = b - 0.25 (a - c) d, and
+ *              r* > 1 (the parabola overshoots) becomes 1 / r*.  Strength S = r* - octave_cost log2(f_min tau* / fs);
+ *              the largest S wins, a tie goes to the smaller tau.  No candidate: VS_PITCH_NOPEAK;
+ *   per stream G = max_f P_f.  A frame without a flag is VS_PITCH_QUIET when P_f < silence_threshold G; a frame with
+ *              none of these three flags is "periodic", and VS_PITCH_VOICED as well when r* >= voicing_threshold.
+ *              F0 = fs / tau* (voiced frames), hnr_db = 10 log10(r* / (1 - r*)) (periodic frames; +inf for r* = 1);
+ *   frames[]   f0_hz (NaN unless voiced), strength = r* (NaN for SILENT and NOPEAK), hnr_db (NaN unless periodic), flags;
+ *   stats      the stream's frames, periodic and voiced frames; over the voiced frames the mean, sample SD, min and max
+ *              of F0; over the periodic frames the mean and sample SD of hnr_db and the mean r*.  FP64 from the unrounded
+ *              values in two passes (the means, then the squared deviations), each rounded to float; NaN where a
+ *              statistic has no frame (an SD: fewer than two); an hnr_db of +inf makes the mean +inf and the SD NaN.
+ * Errors (vs_pitch_frames returns the same ones, in the same order): NULL ctx / pcm / nsamp / stats -> VS_EINVAL; an
+ * option that is not finite, f_min_hz <= 0, f_max_hz <= f_min_hz, periods < 2, a threshold outside [0, 1] or
+ * octave_cost < 0 -> VS_ERANGE; then per stream in index order: a row above 2^31-1 samples -> VS_EOVERLAP; fs <= 0,
+ * tau_lo >= tau_hi, tau_hi + 1 >= Nw, Nw > VS_PITCH_MAX_WIN (the kernel stages a frame in shared memory), H < 1 or
+ * H > 2^31-1 -> VS_ERANGE.  Input, offsets, staging, stats and frame placement (frame_offsets) are as for
+ * vs_formant_batch; frames NULL: no per-frame output, the statistics are the same. */
+#define VS_PITCH_MAX_WIN    4096
+#define VS_PITCH_SILENT     1u
+#define VS_PITCH_NOPEAK     2u
+#define VS_PITCH_QUIET      4u
+#define VS_PITCH_VOICED     8u
+typedef struct vs_pitch_opts {        /* NULL = all defaults; a non-NULL struct is taken literally    */
+    float    f_min_hz;                /* pitch floor: the longest lag and, with periods, the window (75) */
+    float    f_max_hz;                /* pitch ceiling: the shortest lag (600)                        */
+    float    periods;                 /* window length in periods of f_min, >= 2 (3)                  */
+    float    hop_ms;                  /* frame step (10)                                              */
+    float    voicing_threshold;       /* r* at which a periodic frame is voiced, 0..1 (0.45)          */
+    float    silence_threshold;       /* local peak below this share of the stream's peak: QUIET (0.03) */
+    float    octave_cost;             /* favours the shorter of two similar lags, >= 0 (0.01)         */
+} vs_pitch_opts;
+
+typedef struct vs_pitch_frame {       /* 16 bytes */
+    float    f0_hz, strength, hnr_db;
+    uint32_t flags;                   /* VS_PITCH_*                                                   */
+} vs_pitch_frame;
+
+typedef struct vs_pitch_stats {       /* 48 bytes */
+    uint32_t frames, periodic, voiced;
+    float    f0_mean_hz, f0_sd_hz, f0_min_hz, f0_max_hz;   /* voiced frames                             */
+    float    hnr_mean_db, hnr_sd_db, strength_mean;         /* periodic frames                           */
+    uint32_t reserved[2];
+} vs_pitch_stats;
+
+/* host only: validates exactly as vs_pitch_batch does (first offender -> its error) and returns frames per stream */
+int vs_pitch_frames(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *frames_out);
+int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                   size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames,
+                   const uint64_t *frame_offsets);
+
 /* SURVEY 8f N1 -- `vowel -n`: white noise added to already filtered PCM, IN PLACE (vowel_new.c:302-324).
  * Per stream and per frame of 50*((int)(fs*0.001/2.0)*2) samples: float power of the frame, uniform
  * noise of width sqrt(12*power/snr) drawn with random() seeded by srandom(seed[i]) (vowel_new.c:234),

@@ -9,7 +9,7 @@ EXPORTS = ["vs_abi_version", "vs_device_count", "vs_strerror", "vs_last_error", 
            "vs_flow_nsamples", "vs_flow_max_periods", "vs_flow_validate", "vs_filter_warmup",
            "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch",
            "vs_flow_report_batch", "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset",
-           "vs_formant_frames", "vs_formant_batch"]
+           "vs_formant_frames", "vs_formant_batch", "vs_pitch_frames", "vs_pitch_batch"]
 
 
 class FlowParamsC(C.Structure):
@@ -28,6 +28,11 @@ class TractParamsC(C.Structure):
 class FormantOptsC(C.Structure):
     _fields_ = [("win_ms", C.c_float), ("hop_ms", C.c_float), ("preemph_hz", C.c_float), ("bmax_hz", C.c_float),
                 ("order", C.c_uint32), ("n_formants", C.c_uint32)]
+
+
+class PitchOptsC(C.Structure):
+    _fields_ = [(k, C.c_float) for k in ("f_min_hz", "f_max_hz", "periods", "hop_ms", "voicing_threshold", "silence_threshold",
+                                         "octave_cost")]
 
 
 class PeriodLogC(C.Structure):
@@ -93,5 +98,8 @@ def load():
     L.vs_formant_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     L.vs_formant_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p]
+    L.vs_pitch_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    L.vs_pitch_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L

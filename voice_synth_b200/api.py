@@ -11,7 +11,7 @@ import re
 import numpy as np
 
 from . import _lib
-from ._lib import FilterParamsC, FlowParamsC, FormantOptsC, PeriodLogC, TimingC, TractParamsC
+from ._lib import FilterParamsC, FlowParamsC, FormantOptsC, PeriodLogC, PitchOptsC, TimingC, TractParamsC
 
 VS_F_JITTER, VS_F_SHIMMER, VS_F_NOISE = 1, 2, 4
 VS_OK, VS_EINVAL, VS_ERANGE, VS_EPRESET, VS_ENOMEM, VS_ECUDA, VS_ENODEV, VS_EOVERLAP = 0, -1, -2, -3, -4, -5, -6, -7
@@ -39,6 +39,15 @@ FORMANT_STATS_DTYPE = np.dtype([("frames", "<u4"), ("analysed", "<u4"), ("unconv
                                 ("f_sd_hz", "<f4", (MAX_FORMANTS,)), ("bw_mean_hz", "<f4", (MAX_FORMANTS,))])
 assert FORMANT_STATS_DTYPE.itemsize == 144
 FORMANT_DEFAULTS = dict(win_ms=25.0, hop_ms=10.0, preemph_hz=50.0, bmax_hz=700.0, order=14, n_formants=5)
+PITCH_SILENT, PITCH_NOPEAK, PITCH_QUIET, PITCH_VOICED = 1, 2, 4, 8
+PITCH_FRAME_DTYPE = np.dtype([("f0_hz", "<f4"), ("strength", "<f4"), ("hnr_db", "<f4"), ("flags", "<u4")])
+assert PITCH_FRAME_DTYPE.itemsize == 16
+PITCH_STATS_DTYPE = np.dtype([("frames", "<u4"), ("periodic", "<u4"), ("voiced", "<u4"), ("f0_mean_hz", "<f4"),
+                              ("f0_sd_hz", "<f4"), ("f0_min_hz", "<f4"), ("f0_max_hz", "<f4"), ("hnr_mean_db", "<f4"),
+                              ("hnr_sd_db", "<f4"), ("strength_mean", "<f4"), ("reserved", "<u4", (2,))])
+assert PITCH_STATS_DTYPE.itemsize == 48
+PITCH_DEFAULTS = dict(f_min_hz=75.0, f_max_hz=600.0, periods=3.0, hop_ms=10.0, voicing_threshold=0.45, silence_threshold=0.03,
+                      octave_cost=0.01)
 
 _FLOW_FIELDS = [("dur", np.float32, 1.0), ("jitter", np.float32, 0.0), ("shimmer", np.float32, 0.0),
                 ("cq", np.float32, 0.55), ("K", np.float32, 0.65), ("Kvar", np.float32, 0.0), ("F0", np.float32, 120.0),
@@ -305,6 +314,28 @@ def formant_frames(nsamp, fs=None, opts=None):
     return out
 
 
+def pitch_opts(opts=None):
+    """vs_pitch_opts from a dict of the fields to change (the rest keep PITCH_DEFAULTS); None stays None (NULL)"""
+    if opts is None or isinstance(opts, PitchOptsC):
+        return opts
+    unknown = set(opts) - set(PITCH_DEFAULTS)
+    if unknown:
+        raise ValueError(f"unknown pitch options {sorted(unknown)}")
+    return PitchOptsC(**{**PITCH_DEFAULTS, **opts})
+
+
+def pitch_frames(nsamp, fs=None, opts=None):
+    """frames per stream of vs_pitch_batch (host only, validates like the batch call; raises VsError)"""
+    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+    rate = _per_stream(fs, np.int32, len(ns))
+    o = pitch_opts(opts)
+    out = np.zeros(len(ns), dtype=np.uint64)
+    rc = _lib.load().vs_pitch_frames(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
+    if rc:
+        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
+    return out
+
+
 def _per_stream(x, dtype, n):
     """a per-stream argument as n contiguous values of dtype (a scalar stands for every stream); None stays None (NULL)"""
     return None if x is None else np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=dtype), (n,)))
@@ -457,6 +488,25 @@ class Context:
             fr = np.zeros(int(fo[-1]), dtype=FORMANT_FRAME_DTYPE)
         self._check(self.L.vs_formant_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
                                             None if o is None else C.byref(o), st.ctypes.data, _ptr(fr), None))
+        if want_frames:
+            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
+        return st
+
+    def pitch_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_frames=False):
+        """pitch and harmonicity (vs_pitch_batch): per-stream statistics (PITCH_STATS_DTYPE) and, with want_frames, the
+        list of each stream's frame records (PITCH_FRAME_DTYPE).  pcm: numpy array or device tensor; opts: None (the
+        defaults) or a dict of the vs_pitch_opts fields to change."""
+        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+        n = len(ns)
+        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
+        o = pitch_opts(opts)
+        st = np.zeros(n, dtype=PITCH_STATS_DTYPE)
+        fr, fo = None, None
+        if want_frames:
+            fo = np.concatenate([[0], np.cumsum(pitch_frames(ns, fs, opts))]).astype(np.uint64)
+            fr = np.zeros(int(fo[-1]), dtype=PITCH_FRAME_DTYPE)
+        self._check(self.L.vs_pitch_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
+                                          None if o is None else C.byref(o), st.ctypes.data, _ptr(fr), None))
         if want_frames:
             return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
         return st

@@ -8,6 +8,8 @@
 #include <cstdlib>
 #include <cstring>
 #include <chrono>
+#include <cmath>
+#include <map>
 #include <string>
 #include <vector>
 
@@ -26,6 +28,7 @@ cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uin
 cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
                              vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
 cudaError_t vs_launch_formants(const VsFormantArgs &a, vs_formant_stats *stats, vs_formant_frame *frames, cudaStream_t s);
+cudaError_t vs_launch_pitch(const VsPitchArgs &a, vs_pitch_stats *stats, vs_pitch_frame *frames, cudaStream_t s);
 
 namespace {
 
@@ -1173,6 +1176,110 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
     CU(cudaMemcpyAsync((void *)a.win, win.data(), win.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
     CU(vs_launch_formants(a, d_stats, d_frames, d.st));
     CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_formant_stats), cudaMemcpyDeviceToHost, d.st));
+    /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
+    auto records = [&](size_t i) { return RowCopy{frame0[i], frame_offsets ? frame_offsets[i] : frame0[i], nfr[i]}; };
+    if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;
+    CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are pageable host memory */
+    return VS_OK;
+}
+
+/* the option and per-stream checks of vs_pitch_frames and vs_pitch_batch, in the header's order; fills o (the defaults
+ * for in == NULL), each stream's frame count and, unless rows is NULL, its row but for off and tab */
+static int pitch_geometry(const vs_pitch_opts *in, const uint64_t *nsamp, const int32_t *fs, size_t n, vs_pitch_opts &o,
+                          VsPitchRow *rows, uint64_t *frames, std::string *err)
+{
+    o = in ? *in : vs_pitch_opts{75.0f, 600.0f, 3.0f, 10.0f, 0.45f, 0.03f, 0.01f};
+    for (const float v : {o.f_min_hz, o.f_max_hz, o.periods, o.hop_ms, o.voicing_threshold, o.silence_threshold, o.octave_cost})
+        if (!std::isfinite(v)) return vs_error(err, VS_ERANGE, "pitch options must be finite");
+    if (!(o.f_min_hz > 0.0f) || !(o.f_max_hz > o.f_min_hz)) return vs_error(err, VS_ERANGE, "need 0 < f_min_hz < f_max_hz");
+    if (!(o.periods >= 2.0f)) return vs_error(err, VS_ERANGE, "periods %g: at least 2", o.periods);
+    if (!(o.voicing_threshold >= 0.0f && o.voicing_threshold <= 1.0f && o.silence_threshold >= 0.0f && o.silence_threshold <= 1.0f))
+        return vs_error(err, VS_ERANGE, "thresholds must lie in [0, 1]");
+    if (!(o.octave_cost >= 0.0f)) return vs_error(err, VS_ERANGE, "octave_cost must be >= 0");
+    return check_streams(err, nsamp, fs, n, [&](size_t i, int32_t rate) {
+        const double nw = std::round((double)o.periods * rate / (double)o.f_min_hz), hl = (double)o.hop_ms * rate / 1000.0;
+        const double tlo = std::max(2.0, std::ceil(rate / (double)o.f_max_hz)), thi = std::floor(rate / (double)o.f_min_hz);
+        if (!(tlo < thi)) return vs_error(err, VS_ERANGE, "stream %zu: lags %.0f..%.0f: fewer than two", i, tlo, thi);
+        if (!(thi + 1.0 < nw) || nw > VS_PITCH_MAX_WIN)
+            return vs_error(err, VS_ERANGE, "stream %zu: window of %.0f samples, needs %.0f..%d", i, nw, thi + 2.0, VS_PITCH_MAX_WIN);
+        if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
+        const uint64_t h = (uint64_t)std::lround(hl), w = (uint64_t)nw;
+        if (rows) rows[i] = {0, (uint32_t)w, (uint32_t)h, (uint32_t)tlo, (uint32_t)thi, 0, 0, (double)rate};
+        frames[i] = nsamp[i] >= w ? (nsamp[i] - w) / h + 1 : 0;
+        return VS_OK;
+    });
+}
+
+int vs_pitch_frames(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *frames_out)
+{
+    if (!nsamp || !frames_out) return VS_EINVAL;
+    vs_pitch_opts oo;
+    return pitch_geometry(o, nsamp, fs, n, oo, nullptr, frames_out, nullptr);
+}
+
+int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                   size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames, const uint64_t *frame_offsets)
+{
+    if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
+    vs_pitch_opts op;
+    std::vector<VsPitchRow> rows(n);
+    std::vector<uint64_t> nfr(n);
+    int rc = pitch_geometry(o, nsamp, fs, n, op, rows.data(), nfr.data(), &ctx->err);
+    if (rc) return rc;
+    if (n == 0) return VS_OK;
+
+    /* the frame prefix and one table per distinct (Nw, tau_lo, tau_hi), host libm in double: the window w[0..Nw), then
+     * r_w(0) / r_w(tau) for tau = tau_lo-1 .. tau_hi+1, each r_w summed in index order */
+    const double pi = 3.14159265358979323846;
+    std::vector<uint64_t> frame0(n + 1, 0);
+    std::vector<double> tab;
+    std::map<std::array<uint32_t, 3>, uint32_t> tab_at;
+    uint32_t warp_doubles = 0;
+    for (size_t i = 0; i < n; i++) {
+        VsPitchRow &r = rows[i];
+        const auto ins = tab_at.insert({{r.Nw, r.tau_lo, r.tau_hi}, (uint32_t)tab.size()});
+        if (ins.second) {
+            const size_t w0 = tab.size();
+            for (uint32_t m = 0; m < r.Nw; m++) tab.push_back(0.5 - 0.5 * std::cos(2.0 * pi * ((double)m + 0.5) / (double)r.Nw));
+            auto rw = [&](uint32_t tau) {
+                double s = 0.0;
+                for (uint32_t m = 0; m + tau < r.Nw; m++) s += tab[w0 + m] * tab[w0 + m + tau];
+                return s;
+            };
+            const double rw0 = rw(0);
+            for (uint32_t tau = r.tau_lo - 1; tau <= r.tau_hi + 1; tau++) tab.push_back(rw0 / rw(tau));
+        }
+        r.tab = ins.first->second;
+        warp_doubles = std::max(warp_doubles, (r.Nw + 32 + (r.tau_hi - r.tau_lo + 3) + 1) & ~1u);
+        frame0[i + 1] = frame0[i] + nfr[i];
+    }
+    const Span span = place_rows(offsets, nsamp, rows);
+    const uint64_t F = frame0[n];
+    VsPitchArgs a = {};
+    a.n_rows = (uint32_t)n; a.n_frames = F; a.warp_doubles = warp_doubles;
+    a.warps = (uint32_t)std::min<size_t>(4, (227 * 1024) / (warp_doubles * sizeof(double)));   /* the per-block cap of sm_100 */
+    a.f_min = op.f_min_hz; a.voicing = op.voicing_threshold; a.silence = op.silence_threshold; a.octave_cost = op.octave_cost;
+
+    /* scratch: rows | frame prefix | tables | per-frame candidates | stats | frame records */
+    Scratch sc;
+    const size_t o_rows = sc.take(n * sizeof(VsPitchRow)), o_pre = sc.take((n + 1) * sizeof(uint64_t));
+    const size_t o_tab = sc.take(tab.size() * sizeof(double)), o_cand = sc.take(F * sizeof(VsPitchCand));
+    const size_t o_st = sc.take(n * sizeof(vs_pitch_stats)), o_fr = sc.take(frames ? F * sizeof(vs_pitch_frame) : 0);
+    DeviceGuard restore_device;
+    PcmDev<const int16_t> d;
+    if ((rc = pcm_call_begin(ctx, pcm, span, sc.bytes, d))) return rc;
+    a.pcm = d.pcm;
+    a.rows = (const VsPitchRow *)(d.scratch + o_rows);
+    a.frame0 = (const uint64_t *)(d.scratch + o_pre);
+    a.tab = (const double *)(d.scratch + o_tab);
+    a.cand = (VsPitchCand *)(d.scratch + o_cand);
+    vs_pitch_stats *d_stats = (vs_pitch_stats *)(d.scratch + o_st);
+    vs_pitch_frame *d_frames = frames ? (vs_pitch_frame *)(d.scratch + o_fr) : nullptr;
+    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsPitchRow), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
+    CU(vs_launch_pitch(a, d_stats, d_frames, d.st));
+    CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_pitch_stats), cudaMemcpyDeviceToHost, d.st));
     /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
     auto records = [&](size_t i) { return RowCopy{frame0[i], frame_offsets ? frame_offsets[i] : frame0[i], nfr[i]}; };
     if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;

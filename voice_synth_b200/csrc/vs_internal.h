@@ -205,4 +205,37 @@ struct VsFormantArgs {
     double              seed_re[VS_FMT_MAX_ORDER], seed_im[VS_FMT_MAX_ORDER];   /* root-finder start points */
 };
 
+/* pitch analysis (vs_pitch_batch): one entry per stream */
+struct VsPitchRow {
+    uint64_t off;          /* samples, relative to the pcm pointer                                      */
+    uint32_t Nw, H;        /* window length and frame step                                              */
+    uint32_t tau_lo, tau_hi;
+    uint32_t tab;          /* offset of the stream's table: w[0..Nw), then r_w(0) / r_w(tau) for
+                              tau = tau_lo-1 .. tau_hi+1                                                */
+    uint32_t reserved;
+    double   fs;
+};
+
+/* what the frame kernel leaves for the stats kernel, per frame */
+struct VsPitchCand {
+    double   tau, r;       /* tau* and r* of the winning candidate (NaN for SILENT and NOPEAK)          */
+    double   peak;         /* P_f                                                                       */
+    uint32_t flags;        /* VS_PITCH_SILENT | VS_PITCH_NOPEAK                                         */
+    uint32_t reserved;
+};
+
+/* the launch arguments of the two pitch kernels */
+struct VsPitchArgs {
+    const int16_t    *pcm;
+    const VsPitchRow *rows;
+    const uint64_t   *frame0;       /* [n_rows + 1]: global index of each stream's first frame (prefix sum)     */
+    const double     *tab;          /* windows and lag corrections, one table per distinct (Nw, tau_lo, tau_hi) */
+    VsPitchCand      *cand;         /* [n_frames]                                                               */
+    uint32_t          n_rows;
+    uint32_t          warps;        /* warps per CTA of the frame kernel (1..4: the shared memory must fit)     */
+    uint32_t          warp_doubles; /* shared-memory stride of a warp, in doubles                               */
+    uint64_t          n_frames;
+    double            f_min, voicing, silence, octave_cost;
+};
+
 #endif
