@@ -62,6 +62,7 @@ def lib():
         L.vso_vowel.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_void_p]
         L.vso_vowel_noise.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_float, C.c_float,
                                       C.c_int64, C.c_uint32, C.c_void_p]
+        L.vso_noise.argtypes = [C.c_void_p, C.c_size_t, C.c_float, C.c_int64, C.c_uint32]
         _lib = L
     return _lib
 
@@ -114,6 +115,15 @@ def vowel_noise(flow, preset, snr_db, seed, gain=10.0, pre=1.0, fs=22050):
     rc = lib().vso_vowel_noise(flow.ctypes.data, flow.size, ord(preset), gain, pre, snr_db, fs, seed, out.ctypes.data)
     if rc:
         raise RuntimeError(f"vso_vowel_noise rc={rc}")
+    return out
+
+
+def noise(pcm, snr_db, seed, fs=22050):
+    """`vowel -n`'s output noise on already filtered PCM (the second half of vowel_noise): a new array"""
+    out = np.array(pcm, dtype=np.int16, copy=True, order="C")
+    rc = lib().vso_noise(out.ctypes.data, out.size, snr_db, fs, seed)
+    if rc:
+        raise RuntimeError(f"vso_noise rc={rc}")
     return out
 
 

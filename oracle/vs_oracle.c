@@ -278,6 +278,11 @@ int vso_vowel_noise(const int16_t *in, size_t n, int preset_key, float gain, flo
                     float snr_db_arg, int64_t fs, uint32_t seed, int16_t *out)
 {
     if (vso_vowel(in, n, preset_key, gain, pre, out, NULL)) return -1;
+    return vso_noise(out, n, snr_db_arg, fs, seed);
+}
+
+int vso_noise(int16_t *out, size_t n, float snr_db_arg, int64_t fs, uint32_t seed)
+{
     if (!(snr_db_arg > 0)) return -1;                                                  /* :141-143 */
     float snr = (float)pow(10, (double)(snr_db_arg / 10));
     int ms1 = (int)((uint64_t)fs * 0.001 / 2.0) * 2;                                   /* :361 */

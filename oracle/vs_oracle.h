@@ -65,6 +65,8 @@ int    vso_vowel(const int16_t *in, size_t n, int preset_key, float gain, float 
 /* vowel -n (vowel_new.c:302-324): per-frame output noise, frame = 50*((int)(fs*0.001/2.0)*2). */
 int    vso_vowel_noise(const int16_t *in, size_t n, int preset_key, float gain, float pre,
                        float snr_db_arg, int64_t fs, uint32_t seed, int16_t *out);
+/* vso_vowel_noise's second half: the output noise of `vowel -n`, in place on already filtered PCM */
+int    vso_noise(int16_t *out, size_t n, float snr_db, int64_t fs, uint32_t seed);
 int16_t vso_round2int(double x);                                     /* vowel_new.c:413-427 */
 
 #ifdef __cplusplus

@@ -43,7 +43,20 @@ def _formant_tracts(L, nt):
 
 SHAPES = ["cfg2", "cfg3_shard", "cfg5_slice", "flow_cfg2", "flow_cfg3_shard", "filter_only", "tracts_10", "tracts_128",
           "no_chunks", "fixed_chunks", "flow_fixed_chunks", "exact", "slab_97", "ragged", "period_log",
-          "simple_gen", "flow_simple_gen", "raw", "gain_10_5", "flow_exact", "kvar"]
+          "simple_gen", "flow_simple_gen", "raw", "gain_10_5", "flow_exact", "kvar",
+          "limit_filter", "limit_filter_chunk_2e27", "limit_filter_no_chunks", "limit_flow", "limit_flow_no_chunks",
+          "limit_flow_simple_gen", "limit_flow_noise", "limit_synth", "limit_synth_no_chunks", "limit_tracts_10",
+          "limit_tracts_10_no_chunks"]
+
+# The longest rows the ABI accepts: 2^31 - 1 samples of caller PCM, and the longest flow (float)fs * dur can give,
+# 2^31 - 128 samples (16 kHz for 134217.71875 s)
+LIMIT_NSAMP = 2**31 - 1
+LIMIT_FLOW_NSAMP = 2**31 - 128
+
+
+def limit_flow_params(noise=0.0):
+    """one voice of LIMIT_FLOW_NSAMP samples: strictly periodic (160 samples a period), with glottal noise if noise > 0"""
+    return api.FlowParams(1, fs=16000, dur=134217.71875, F0=100.0, noise=noise, seed=7, flags=4 if noise > 0 else 0)
 
 
 def shapes(L):
@@ -62,6 +75,10 @@ def shapes(L):
     p_kvar = p2.select(np.arange(p2.n))
     p_kvar.Kvar[::7] = 0.3
     sub = np.arange(1024)
+    p_lim = limit_flow_params()
+    f_lim = api.FilterParams(1, preset="u")
+    t_lim = api.TractParams(1, _preset_tracts(L), tract=[workloads.PRESETS.index("u")])     # the preset 'u' as a tract
+    p_lim_noise = limit_flow_params(noise=10.0)
     p_sub, f_sub = p2.select(sub), f2.select(sub)
     ns_sub = _nsamples(L, p_sub)
     ragged = np.concatenate([[0], np.cumsum(ns_sub[:-1] + rng.integers(0, 300, 1023).astype(np.uint64))]).astype(np.uint64) + 3
@@ -91,6 +108,17 @@ def shapes(L):
         "gain_10_5": dict(d, p=p2, f=f_gain),
         "flow_exact": dict(d, mode=FLOW, p=p2, exact=1),
         "kvar": dict(d, p=p_kvar, f=f2),
+        "limit_filter": dict(d, mode=FILTER, p=None, f=f_lim, nsamp=[LIMIT_NSAMP]),
+        "limit_filter_chunk_2e27": dict(d, mode=FILTER, p=None, f=f_lim, nsamp=[LIMIT_NSAMP], chunk=2**27),
+        "limit_filter_no_chunks": dict(d, mode=FILTER, p=None, f=f_lim, nsamp=[LIMIT_NSAMP], chunk=-1),
+        "limit_flow": dict(d, mode=FLOW, p=p_lim),
+        "limit_flow_no_chunks": dict(d, mode=FLOW, p=p_lim, chunk=-1),
+        "limit_flow_simple_gen": dict(d, mode=FLOW, p=p_lim, simple_gen=1),
+        "limit_flow_noise": dict(d, mode=FLOW, p=p_lim_noise),
+        "limit_synth": dict(d, p=p_lim, f=f_lim),
+        "limit_synth_no_chunks": dict(d, p=p_lim, f=f_lim, chunk=-1),
+        "limit_tracts_10": dict(d, p=p_lim, f=t_lim),
+        "limit_tracts_10_no_chunks": dict(d, p=p_lim, f=t_lim, chunk=-1),
     }
 
 
@@ -128,6 +156,17 @@ KERNELS = {
     "gain_10_5":          (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_FMA, 0, 0, 0, FAST, 5),
     "flow_exact":         (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_EXACT, 0, 0, 0, FAST, 41),
     "kvar":               (TAB_FULL, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 1, SIMPLE, 0),
+    "limit_filter":       (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "limit_filter_chunk_2e27": (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "limit_filter_no_chunks": (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "limit_flow":         (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 33),
+    "limit_flow_no_chunks": (TAB_C8, 1, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 33),
+    "limit_flow_simple_gen": (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, SIMPLE, 0),
+    "limit_flow_noise":   (TAB_N16, 0, 0, 10, 32, PULSE, 512, F_INT, 0, 1, 0, FAST, 3),
+    "limit_synth":        (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "limit_synth_no_chunks": (TAB_C8, 0, 0, 10, 32, LEAN, 1024, F_INT, 0, 0, 0, FAST, 1),
+    "limit_tracts_10":    (TAB_C8, 0, 1, 128, 128, LEAN, 1024, F_INT, 0, 0, 0, FAST, 65),
+    "limit_tracts_10_no_chunks": (TAB_C8, 0, 1, 128, 128, LEAN, 1024, F_INT, 0, 0, 0, FAST, 65),
 }
 
 # VS_OPT_PLAN_WARPS, streams, glottal noise, period log, busy, burst -> the plan kernel's warp form
@@ -144,9 +183,9 @@ PLAN_WARPS = [
 ]
 
 
-@pytest.fixture(scope="module")
-def shim(tmp_path_factory):
-    out = tmp_path_factory.mktemp("batch_plan") / "libbatch_plan_shim.so"
+def build_shim(out_dir):
+    """the planner and the shim as a shared library in out_dir"""
+    out = pathlib.Path(out_dir) / "libbatch_plan_shim.so"
     subprocess.run(["g++", "-O3", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-o", str(out),
                     str(ROOT / "tests" / "tools" / "batch_plan_shim.cpp"), str(ROOT / "voice_synth_b200" / "csrc" / "vs_batch_plan.cpp")],
                    check=True)
@@ -159,6 +198,11 @@ def shim(tmp_path_factory):
     L.shim_plan_warps.argtypes = [C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_uint]
     L.vs_flow_max_periods.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p]
     return L
+
+
+@pytest.fixture(scope="module")
+def shim(tmp_path_factory):
+    return build_shim(tmp_path_factory.mktemp("batch_plan"))
 
 
 @pytest.fixture(scope="module")

@@ -84,25 +84,30 @@ __global__ void __launch_bounds__(VS_FLOWROWS_WARPS * 32, 4) vs_flow_rows_kernel
                 const int up = __shfl_up_sync(VS_FULL, incl, o);
                 if (lane >= o) incl += up;
             }
-            const int start = sb + incl - T;
+            /* a period that starts or ends past 2^31 - 1 is clipped to it: rows end at or before it (VS_EOVERLAP) */
+            const int start = (int)min((long long)sb + incl - T, 0x7fffffffLL);
+            const int end = (int)min((long long)sb + incl, 0x7fffffffLL);
             const double Ad = (double)__uint_as_float(e.x);
             const int fv = max(vs_ceil_magic(__dmul_rn(Ad, h0)), DCs);
             __syncwarp();                                   /* the previous batch has been read by every lane */
             ent[lane] = make_uint4((uint32_t)start, (uint32_t)(T - 1), (uint32_t)__double2loint(Ad), (uint32_t)__double2hiint(Ad));
             first[lane] = fv;
-            if (lane == 31) { ent[32] = make_uint4((uint32_t)(start + T), 0xffffffffu, 0u, 0u); first[32] = DCs; }
+            if (lane == 31) { ent[32] = make_uint4((uint32_t)end, 0xffffffffu, 0u, 0u); first[32] = DCs; }
             __syncwarp();
             more = qb + 32u < np;
             /* with more periods to come the batch's last one only serves as the `next` of a straddling pair */
-            blimit = __shfl_sync(VS_FULL, more ? start : start + T, 31);
+            blimit = __shfl_sync(VS_FULL, more ? start : end, 31);
         };
         load_batch();
 
-        /* steps are anchored on the 128-byte lines of the row's own address */
+        /* steps are anchored on the 128-byte lines of the row's own address.  A row can end at 2^31 - 128 (the most
+         * (float)fs * dur gives): the step's bounds come from the samples left, M + VS_SPAN can pass 2^31.  Positions of
+         * a lane's pairs past the row's end are computed modulo 2^32 and never stored. */
         const int ph64 = (int)((reinterpret_cast<uintptr_t>(orow) >> 1) & 63);
         int P = 0;                                          /* batch index of the period that contains the previous step's last sample */
-        for (int M = lo - ((ph64 + lo) & 63); M < hi; M += VS_SPAN) {
-            const int Mend = min(M + VS_SPAN, hi);
+        for (int M = lo - ((ph64 + lo) & 63);; M += VS_SPAN) {
+            const uint32_t left = (uint32_t)hi - (uint32_t)M;                /* > 0: samples of the row from M on */
+            const int Mend = left > VS_SPAN ? M + VS_SPAN : hi;
             if (Mend > blimit && more) {                    /* re-base the batch on the current period */
                 qb += (uint32_t)P;
                 sb = (int)ent[P].x;
@@ -115,16 +120,16 @@ __global__ void __launch_bounds__(VS_FLOWROWS_WARPS * 32, 4) vs_flow_rows_kernel
             }
             /* the period of each of the lane's four pairs: P + the period starts since then at or before the pair */
             const int Mlast = Mend - 1;
-            const int m0 = M + 2 * lane;
+            const uint32_t m0 = (uint32_t)M + 2u * (uint32_t)lane;
             int pu[4] = {P, P, P, P};
             {
                 int j = P + 1;
                 int bnd = (int)ent[j].x;
                 while (bnd <= Mlast) {
-                    vs_count_le(pu[0], bnd, m0);
-                    vs_count_le(pu[1], bnd, m0 + 64);
-                    vs_count_le(pu[2], bnd, m0 + 128);
-                    vs_count_le(pu[3], bnd, m0 + 192);
+                    vs_count_le(pu[0], bnd, (int)m0);
+                    vs_count_le(pu[1], bnd, (int)(m0 + 64u));
+                    vs_count_le(pu[2], bnd, (int)(m0 + 128u));
+                    vs_count_le(pu[3], bnd, (int)(m0 + 192u));
                     j++;
                     bnd = (int)ent[j].x;
                 }
@@ -137,7 +142,7 @@ __global__ void __launch_bounds__(VS_FLOWROWS_WARPS * 32, 4) vs_flow_rows_kernel
 #pragma unroll
             for (int u = 0; u < 4; u++) {
                 const uint4 e0 = ent[pu[u]];
-                const uint32_t i0 = (uint32_t)(m0 + 64 * u) - e0.x;      /* "negative" before the row's first period */
+                const uint32_t i0 = m0 + 64u * u - e0.x;    /* "negative" before the row's first period */
                 A[u] = __hiloint2double((int)e0.w, (int)e0.z);
                 str[u] = (int)i0 >= (int)e0.y;              /* the pair's second sample opens the next period */
                 const uint32_t ic = min(i0, n2);            /* beyond the open phase the table is zero */
@@ -152,18 +157,20 @@ __global__ void __launch_bounds__(VS_FLOWROWS_WARPS * 32, 4) vs_flow_rows_kernel
                 x1[u] = max(vs_ceil_magic(__dmul_rn(A[u], f[u].y)), DCs);
                 if (str[u]) x1[u] = first[pu[u] + 1];
             }
-            if (M >= lo && M + VS_SPAN <= hi) {
+            if (M >= lo && left >= VS_SPAN) {
                 uint32_t *const o32 = reinterpret_cast<uint32_t *>(orow + m0);
 #pragma unroll
                 for (int u = 0; u < 4; u++) o32[32 * u] = __byte_perm((uint32_t)x0[u], (uint32_t)x1[u], 0x5410);
-            } else {                                        /* a stream's first or last step */
+            } else {                                        /* a stream's first or last step: the step's samples [klo, left) are the row's */
+                const int klo = lo - M;
 #pragma unroll
                 for (int u = 0; u < 4; u++) {
-                    const int m = m0 + 64 * u;
-                    if (m >= lo && m < hi) orow[m] = (int16_t)x0[u];
-                    if (m + 1 >= lo && m + 1 < hi) orow[m + 1] = (int16_t)x1[u];
+                    const int k = 2 * lane + 64 * u;
+                    if (k >= klo && (uint32_t)k < left) orow[M + k] = (int16_t)x0[u];
+                    if (k + 1 >= klo && (uint32_t)k + 1u < left) orow[M + k + 1] = (int16_t)x1[u];
                 }
             }
+            if (left <= VS_SPAN) break;
         }
     }
 }

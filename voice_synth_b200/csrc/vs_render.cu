@@ -93,12 +93,13 @@ __device__ __forceinline__ void vs_pair_barrier(int pair)
 }
 
 /* ---- F: one lane, one row: the order-22 recurrence (vowel_new.c:266-289) window after window, in place ------- *
+ * rrow, rlo, rhi: the raw output row and the row's [lo, hi), all counted from the lane's first window (blk0).
  * Coefficients: PRESET >= 0 reads c_ncoef[PRESET] at literal constant-bank addresses; PRESET < 0 reads tcoef[0..21]
  * (= -A[1..22]) inside the kernel's parameter block (the tract kernels).  The operations and their order are the
  * same either way. */
 template <int WIN, int NT, int FILT, bool RAW, int PRESET>
 __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane's row in tile 0 */, const int pair, const int nwin,
-                                               const double gaind, const double pred, double *rrow, const int blk0, const int lo, const int hi,
+                                               const double gaind, const double pred, double *rrow, const uint32_t rlo, const uint32_t rhi,
                                                const double *tcoef)
 {
 #define VS_NC(j) (PRESET >= 0 ? c_ncoef[PRESET < 0 ? 0 : PRESET][j] : tcoef[(j) - 1])
@@ -110,7 +111,9 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
     /* FILT_INT: the bytes {-pre, 1} of a two-way 16x8 dot product (pre is 0 or 1) */
     const int pre_b = (int)(((uint32_t)-(int)pred & 0xffu) | 0x100u);
     uint32_t w_prev = 0;                                    /* the last input word read: its high half is x[n-1] */
-    int mbase = blk0, ti = 0;
+    uint32_t mbase = 0;                                     /* the group's first sample, counted from blk0 (see nwin) */
+    double *rgrp = rrow;                                    /* its raw output, advanced with it (a 64-bit pointer) */
+    int ti = 0;
 
     vs_pair_barrier(pair);                                  /* window 0 generated */
     for (int w = 0; w < nwin; w++) {
@@ -158,8 +161,8 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
                      * saturating pack and a 16x2 maximum below */
                     qv[u] = FILT == VS_FILT_EXACT ? vs_round2int(v) : __double2int_rn(v);
                     if (RAW) {
-                        const int m = mbase + u;
-                        if (rrow && m >= lo && m < hi) rrow[m] = v;
+                        const uint32_t m = mbase + u;
+                        if (rrow && m >= rlo && m < rhi) rgrp[u] = v;
                     }
                 }
 #pragma unroll
@@ -171,6 +174,7 @@ __device__ __forceinline__ void vs_filter_rows(unsigned char *tiles /* the lane'
                 *piece = make_uint4(ow[0], ow[1], ow[2], ow[3]);
                 w_prev = xw[3];
                 mbase += VS_GROUP;
+                if (RAW) rgrp += VS_GROUP;
             }
         }
         vs_fence_async();                                   /* the TMA engine will read what this lane wrote */
@@ -259,7 +263,11 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
     /* windows are anchored on the 16-byte grid of the row's own address in HBM */
     const int phase = (int)((reinterpret_cast<uintptr_t>(orow) >> 1) & 7);
     const int blk0 = nstart - ((phase + nstart) & 7);
-    int nwin = active ? (hi - blk0 + WIN - 1) / WIN : 0;
+    /* Per window, positions are counted from blk0 in unsigned arithmetic: a row may end at 2^31 - 1 and be unchunked
+     * (blk0 down to -7), and the warp runs every lane to its longest row, so blk0 + w * WIN can pass 2^31 where
+     * (uint32_t)w * WIN cannot (it stays below 2^31 + 2 * WIN). */
+    const uint32_t rnst = (uint32_t)(nstart - blk0), rlo = (uint32_t)lo - (uint32_t)blk0, rhi = (uint32_t)hi - (uint32_t)blk0;
+    int nwin = active ? (int)((rhi + (WIN - 1)) / WIN) : 0;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) nwin = max(nwin, __shfl_xor_sync(VS_FULL, nwin, o));
 
@@ -271,13 +279,13 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
      * =================================================================================================== */
     if (is_f) {
         const double gaind = active ? (double)st->gain : 0.0, pred = active ? (double)st->pre : 0.0;
-        double *rrow = (RAW && active && a.raw_out) ? a.raw_out + st->out_off : nullptr;
+        double *rrow = (RAW && active && a.raw_out) ? a.raw_out + st->out_off + blk0 : nullptr;
         unsigned char *tiles = smem + tile_off + (uint32_t)lane * TSB;
-        if constexpr (TRACT) vs_filter_rows<WIN, NT, FILT, RAW, -1>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, tcoef);
+        if constexpr (TRACT) vs_filter_rows<WIN, NT, FILT, RAW, -1>(tiles, pair, nwin, gaind, pred, rrow, rlo, rhi, tcoef);
         else switch (preset) {
-#define VS_F_CASE(P) case P: vs_filter_rows<WIN, NT, FILT, RAW, P>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, nullptr); break;
+#define VS_F_CASE(P) case P: vs_filter_rows<WIN, NT, FILT, RAW, P>(tiles, pair, nwin, gaind, pred, rrow, rlo, rhi, nullptr); break;
             VS_F_CASE(0) VS_F_CASE(1) VS_F_CASE(2) VS_F_CASE(3) VS_F_CASE(4) VS_F_CASE(5) VS_F_CASE(6) VS_F_CASE(7) VS_F_CASE(8)
-            default: vs_filter_rows<WIN, NT, FILT, RAW, 9>(tiles, pair, nwin, gaind, pred, rrow, blk0, lo, hi, nullptr); break;
+            default: vs_filter_rows<WIN, NT, FILT, RAW, 9>(tiles, pair, nwin, gaind, pred, rrow, rlo, rhi, nullptr); break;
 #undef VS_F_CASE
         }
         continue;
@@ -560,19 +568,20 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
              * latency per window.  Any other layout, and the pieces that straddle the row's ends, go sample by
              * sample. */
             unsigned char *trow = tbase + (uint32_t)lane * TSB;
-            const int wb = blk0 + w * WIN;
-            const bool aligned = ((reinterpret_cast<uintptr_t>(fin + blk0)) & 15) == 0;
+            const int16_t *fb = fin + blk0;                 /* positions from here on count from blk0 */
+            const uint32_t wb = (uint32_t)w * WIN;
+            const bool aligned = ((reinterpret_cast<uintptr_t>(fb)) & 15) == 0;
             uint4 pc[NGRP];
 #pragma unroll
             for (int g = 0; g < NGRP; g++) {
-                const int m0 = wb + g * VS_GROUP;
-                if (aligned && m0 >= nstart && m0 + VS_GROUP <= hi) pc[g] = __ldg(reinterpret_cast<const uint4 *>(fin + m0));
+                const uint32_t m0 = wb + g * VS_GROUP;
+                if (aligned && m0 >= rnst && m0 + VS_GROUP <= rhi) pc[g] = __ldg(reinterpret_cast<const uint4 *>(fb + m0));
                 else {
                     uint32_t h[VS_GROUP];
 #pragma unroll
                     for (int u = 0; u < VS_GROUP; u++) {
-                        const int m = m0 + u;
-                        h[u] = (m >= nstart && m < hi) ? (uint32_t)(uint16_t)__ldg(fin + m) : 0u;
+                        const uint32_t m = m0 + u;
+                        h[u] = (m >= rnst && m < rhi) ? (uint32_t)(uint16_t)__ldg(fb + m) : 0u;
                     }
                     pc[g] = make_uint4(h[0] | (h[1] << 16), h[2] | (h[3] << 16), h[4] | (h[5] << 16), h[6] | (h[7] << 16));
                 }
@@ -612,19 +621,20 @@ vs_render_kernel(const VsRenderArgs a, const __grid_constant__ VsTractParam<TRAC
     /* ---- W: a finished window leaves through the TMA engine: per lane one bulk copy of its row's whole 16-byte
      * pieces inside [lo, hi); the few samples of a stream's unaligned first / last piece go as 2-byte stores ---- */
     auto store_window = [&](const int w, const int ti) {
-        const int wb = blk0 + w * WIN;
-        const int a0 = max(wb, lo), b0 = min(wb + WIN, hi);
+        int16_t *ob = orow + blk0;                          /* positions count from blk0, the window's start is a multiple of 8 */
+        const uint32_t wb = (uint32_t)w * WIN;
+        const uint32_t a0 = max(wb, rlo), b0 = min(wb + WIN, rhi);
 #ifdef VS_DEBUG_BOUNDS
-        if (b0 > a0 && (orow == nullptr || a0 < 0 || b0 - wb > WIN || a0 < wb)) { atomicExch(a.status, -120); return; }
+        if (b0 > a0 && (orow == nullptr || b0 - wb > WIN || a0 < wb)) { atomicExch(a.status, -120); return; }
 #endif
         if (b0 > a0) {
             const uint32_t trow = tile_off + (uint32_t)ti * TILE + (uint32_t)lane * TSB;
-            const int a8 = wb + ((a0 - wb + 7) & ~7), b8 = wb + ((b0 - wb) & ~7);
-            if (b8 > a8 && !(a.debug & 1)) vs_bulk_s2g(orow + a8, smem_base + trow + (uint32_t)(a8 - wb) * 2u, (uint32_t)(b8 - a8) * 2u);
+            const uint32_t a8 = (a0 + 7u) & ~7u, b8 = b0 & ~7u;
+            if (b8 > a8 && !(a.debug & 1)) vs_bulk_s2g(ob + a8, smem_base + trow + (a8 - wb) * 2u, (b8 - a8) * 2u);
             const int16_t *tr = reinterpret_cast<const int16_t *>(smem + trow);
-            const int hend = min(a8, b0);
-            for (int m = a0; m < hend; m++) orow[m] = tr[m - wb];
-            for (int m = max(b8, hend); m < b0; m++) orow[m] = tr[m - wb];
+            const uint32_t hend = min(a8, b0);
+            for (uint32_t m = a0; m < hend; m++) ob[m] = tr[m - wb];
+            for (uint32_t m = max(b8, hend); m < b0; m++) ob[m] = tr[m - wb];
         }
         vs_bulk_commit();
     };
