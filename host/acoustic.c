@@ -16,7 +16,11 @@
  *   acoustic -P file.wav [file.wav ...]                    pitch and harmonicity of vowel PCM (vs_pitch_batch, default
  *                                                          options: 75-600 Hz, 3 periods per window, 10 ms hop)
  * One line per file:  name  fs  samples  frames  voiced  F0_mean[Hz]  F0_sd[Hz]  HNR_mean[dB]   (nan where no frame is
- *    voiced, resp. periodic) */
+ *    voiced, resp. periodic)
+ *
+ *   acoustic -V file.wav [file.wav ...]                    voice report of vowel PCM (vs_vowel_report_batch, default pitch
+ *                                                          options): period marks by cross-correlation, then the report
+ * One line per file: the columns of -x, then the voiced run the marks lie in: first frame, frames, first sample, samples */
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -26,7 +30,7 @@
 
 int main(int argc, char **argv)
 {
-    int lo = 0, hi = 0, a = 1, report = 0, formants = 0, pitch = 0, order = 14;
+    int lo = 0, hi = 0, a = 1, report = 0, formants = 0, pitch = 0, vowel = 0, order = 14;
     for (;;) {
         if (a < argc && strcmp(argv[a], "-x") == 0) {
             report = 1;
@@ -36,6 +40,9 @@ int main(int argc, char **argv)
             a += 1;
         } else if (a < argc && strcmp(argv[a], "-P") == 0) {
             pitch = 1;
+            a += 1;
+        } else if (a < argc && strcmp(argv[a], "-V") == 0) {
+            vowel = report = 1;
             a += 1;
         } else if (a + 1 < argc && strcmp(argv[a], "-p") == 0) {
             order = atoi(argv[a + 1]);
@@ -51,7 +58,8 @@ int main(int argc, char **argv)
         printf("usage: acoustic [-l lo] [-h hi] [-x] file.wav [file.wav ...]   (lo <= hi: thresholds of the onset trigger;"
                " -x: voice report columns)\n"
                "       acoustic -F [-p order] file.wav [file.wav ...]          (formants of vowel PCM; order even, 2..32)\n"
-               "       acoustic -P file.wav [file.wav ...]                     (pitch and harmonicity of vowel PCM)\n");
+               "       acoustic -P file.wav [file.wav ...]                     (pitch and harmonicity of vowel PCM)\n"
+               "       acoustic -V file.wav [file.wav ...]                     (voice report of vowel PCM)\n");
         return 0;
     }
     const size_t n = (size_t)(argc - a);
@@ -105,7 +113,13 @@ int main(int argc, char **argv)
     }
     vs_flow_stats *st = (vs_flow_stats *)calloc(n, sizeof *st);
     vs_flow_report *rp = report ? (vs_flow_report *)calloc(n, sizeof *rp) : NULL;
-    rc = report ? vs_flow_report_batch(ctx, flow, offs, ns, fs, tl, th, n, rp) : vs_flow_analyze_batch(ctx, flow, offs, ns, fs, tl, th, n, st);
+    vs_vowel_report *vr = vowel ? (vs_vowel_report *)calloc(n, sizeof *vr) : NULL;
+    if (vowel) {
+        rc = vs_vowel_report_batch(ctx, flow, offs, ns, fs, n, NULL, vr, NULL, NULL);
+        for (size_t i = 0; i < n && !rc; i++) rp[i] = vr[i].rep;
+    } else {
+        rc = report ? vs_flow_report_batch(ctx, flow, offs, ns, fs, tl, th, n, rp) : vs_flow_analyze_batch(ctx, flow, offs, ns, fs, tl, th, n, st);
+    }
     if (rc) { fprintf(stderr, "acoustic: %s (%s)\n", vs_strerror(rc), vs_last_error(ctx)); return 1; }
     for (size_t i = 0; i < n; i++) {
         if (report) st[i] = rp[i].base;
@@ -119,6 +133,7 @@ int main(int argc, char **argv)
             printf(" %.3f %.4f %.4f %.4f %.4f %.4f %.4f %.4f %.4f %.3f", rp[i].jitter_abs_us, rp[i].jitter_rap_pct, rp[i].jitter_ppq5_pct,
                    rp[i].jitter_ddp_pct, rp[i].shimmer_db, rp[i].shimmer_apq3_pct, rp[i].shimmer_apq5_pct, rp[i].shimmer_apq11_pct,
                    rp[i].shimmer_dda_pct, rp[i].hnr_db);
+        if (vowel) printf(" %u %u %u %u", vr[i].run_frame, vr[i].run_frames, vr[i].run_start, vr[i].run_len);
         printf("\n");
     }
     vs_ctx_destroy(ctx);

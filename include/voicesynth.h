@@ -363,6 +363,50 @@ int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, con
                    size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames,
                    const uint64_t *frame_offsets);
 
+/* Voice report of vowel PCM (the jitter and shimmer axes of rendered vowels, which vs_flow_report_batch measures only on
+ * glottal flow): period marks by cross-correlation guided by the pitch track, in the spirit of Praat's "To PointProcess
+ * (periodic, cc)", then the voice report above on those marks.  The definitions are the library's own; they make every
+ * mark an exact integer decided by exact integer sums.  tests/vowel_report_ref.py restates them in numpy.  Per stream,
+ * with x the PCM, fs its rate and the options o (NULL: the defaults of vs_pitch_opts):
+ *   track      the frames of vs_pitch_batch with the same options, and its Nw and H;
+ *   run        the longest sequence of consecutive VS_PITCH_VOICED frames f_a .. f_b (the first of equal ones); its
+ *              samples are [s, e) = [f_a H, f_b H + Nw).  No voiced frame: run_frames = 0, no mark, and rep is the report
+ *              of an empty onset list (onsets = cycles = 0, every quotient NaN);
+ *   period     T(t) = fs / (double)f0_hz with f0_hz the float frame record of frame f = clamp(floor((t - floor(Nw/2) +
+ *              floor(H/2)) / H), f_a, f_b) (integer arithmetic), and L(t) = lround(T(t));
+ *   anchor     m_0 = the first index of max |x| in [c - floor(L(c)/2), c - floor(L(c)/2) + L(c)), the period around the
+ *              centre c = s + floor(Nw/2) of the run's first frame (a voiced frame's window may begin in silence);
+ *   step       from m_k, with T = T(m_k) and L = lround(T), and only while every candidate's period lies in the run
+ *              (m_k + lround(VS_MARK_STEP_MAX T) + L <= e): the candidates are the m in
+ *              [m_k + lround(VS_MARK_STEP_MIN T), m_k + lround(VS_MARK_STEP_MAX T)];
+ *              C(m) = sum_{j<L} x[m_k+j] x[m+j] and E(p) = sum_{j<L} x[p+j]^2, exact integers;
+ *              r(m) = C(m) / sqrt((double)E(m_k) (double)E(m)) (IEEE multiply, square root and divide; 0 when the
+ *              product is 0).  The largest r wins, a tie goes to the smaller m; m_k+1 is the winner unless there is no
+ *              candidate or the best r <= 0, which ends the marks;
+ *   report     the marks m_0 < ... < m_K-1 (stream coordinates) are the onsets of the vs_flow_report definitions, with
+ *              x the PCM: base.onsets = K, base.cycles = K - 1, the peaks P_k the largest sample of each period, the
+ *              quotients and the cycle-synchronous HNR.
+ * vs_vowel_mark_slots bounds the marks of a stream (base.flags is never VS_STATS_OVERFLOW): with tau_lo of the pitch
+ * geometry every step is at least lround(VS_MARK_STEP_MIN T_lo) >= 1 samples, T_lo = (tau_lo - 1/2) (1 - 2^-20) below
+ * any period a frame record can publish; a stream of n >= Nw samples has at most (n - 1) / step + 1 marks, 0 below Nw.
+ * Errors (vs_vowel_mark_slots returns the same ones, in the same order): NULL ctx / pcm / nsamp / out -> VS_EINVAL, then
+ * those of vs_pitch_batch.  Input, offsets and staging are as for vs_pitch_batch.  marks (nullable) and mark_offsets are
+ * host memory: stream i's base.onsets marks go to marks + mark_offsets[i] (mark_offsets NULL: the prefix sum of the
+ * slots, densely packed); marks NULL: no marks are written, out is the same. */
+#define VS_MARK_STEP_MIN 0.8
+#define VS_MARK_STEP_MAX 1.25
+typedef struct vs_vowel_report {      /* 96 bytes */
+    vs_flow_report rep;               /* the voice report over the marks: rep.base.onsets = marks, .cycles = periods */
+    uint32_t run_frame, run_frames;   /* the analysed voiced run, in pitch frames; run_frames 0: no voiced frame     */
+    uint32_t run_start, run_len;      /* the same run in samples                                                    */
+} vs_vowel_report;
+
+/* host only: validates exactly as vs_vowel_report_batch does; per stream the number of mark slots it may fill */
+int vs_vowel_mark_slots(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *slots_out);
+int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp,
+                          const int32_t *fs, size_t n, const vs_pitch_opts *o, vs_vowel_report *out,
+                          uint32_t *marks, const uint64_t *mark_offsets);
+
 /* SURVEY 8f N1 -- `vowel -n`: white noise added to already filtered PCM, IN PLACE (vowel_new.c:302-324).
  * Per stream and per frame of 50*((int)(fs*0.001/2.0)*2) samples: float power of the frame, uniform
  * noise of width sqrt(12*power/snr) drawn with random() seeded by srandom(seed[i]) (vowel_new.c:234),

@@ -9,7 +9,8 @@ EXPORTS = ["vs_abi_version", "vs_device_count", "vs_strerror", "vs_last_error", 
            "vs_flow_nsamples", "vs_flow_max_periods", "vs_flow_validate", "vs_filter_warmup",
            "vs_flowgen_batch", "vs_vowel_filter_batch", "vs_synth_batch", "vs_vowel_noise_batch", "vs_flow_analyze_batch",
            "vs_flow_report_batch", "vs_synth_batch_tract", "vs_vowel_filter_batch_tract", "vs_tract_from_formants", "vs_tract_from_preset",
-           "vs_formant_frames", "vs_formant_batch", "vs_pitch_frames", "vs_pitch_batch"]
+           "vs_formant_frames", "vs_formant_batch", "vs_pitch_frames", "vs_pitch_batch",
+           "vs_vowel_mark_slots", "vs_vowel_report_batch"]
 
 
 class FlowParamsC(C.Structure):
@@ -101,5 +102,8 @@ def load():
     L.vs_pitch_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     L.vs_pitch_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p]
+    L.vs_vowel_mark_slots.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    L.vs_vowel_report_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L

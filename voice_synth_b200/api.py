@@ -48,6 +48,9 @@ PITCH_STATS_DTYPE = np.dtype([("frames", "<u4"), ("periodic", "<u4"), ("voiced",
 assert PITCH_STATS_DTYPE.itemsize == 48
 PITCH_DEFAULTS = dict(f_min_hz=75.0, f_max_hz=600.0, periods=3.0, hop_ms=10.0, voicing_threshold=0.45, silence_threshold=0.03,
                       octave_cost=0.01)
+VOWEL_REPORT_DTYPE = np.dtype([("rep", FLOW_REPORT_DTYPE), ("run_frame", "<u4"), ("run_frames", "<u4"), ("run_start", "<u4"),
+                               ("run_len", "<u4")])
+assert VOWEL_REPORT_DTYPE.itemsize == 96
 
 _FLOW_FIELDS = [("dur", np.float32, 1.0), ("jitter", np.float32, 0.0), ("shimmer", np.float32, 0.0),
                 ("cq", np.float32, 0.55), ("K", np.float32, 0.65), ("Kvar", np.float32, 0.0), ("F0", np.float32, 120.0),
@@ -336,6 +339,18 @@ def pitch_frames(nsamp, fs=None, opts=None):
     return out
 
 
+def vowel_mark_slots(nsamp, fs=None, opts=None):
+    """mark slots per stream of vs_vowel_report_batch (host only, validates like the batch call; raises VsError)"""
+    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+    rate = _per_stream(fs, np.int32, len(ns))
+    o = pitch_opts(opts)
+    out = np.zeros(len(ns), dtype=np.uint64)
+    rc = _lib.load().vs_vowel_mark_slots(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
+    if rc:
+        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
+    return out
+
+
 def _per_stream(x, dtype, n):
     """a per-stream argument as n contiguous values of dtype (a scalar stands for every stream); None stays None (NULL)"""
     return None if x is None else np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=dtype), (n,)))
@@ -510,6 +525,26 @@ class Context:
         if want_frames:
             return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
         return st
+
+    def vowel_report_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_marks=False):
+        """voice report of vowel PCM (vs_vowel_report_batch): per stream the report over its period marks and the voiced
+        run they lie in (VOWEL_REPORT_DTYPE) and, with want_marks, the list of each stream's marks (uint32, stream
+        coordinates).  pcm: numpy array or device tensor; opts: None (the defaults) or a dict of the vs_pitch_opts fields
+        to change."""
+        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+        n = len(ns)
+        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
+        o = pitch_opts(opts)
+        out = np.zeros(n, dtype=VOWEL_REPORT_DTYPE)
+        mk, mo = None, None
+        if want_marks:
+            mo = np.concatenate([[0], np.cumsum(vowel_mark_slots(ns, fs, opts))]).astype(np.uint64)
+            mk = np.zeros(int(mo[-1]), dtype=np.uint32)
+        self._check(self.L.vs_vowel_report_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
+                                                 None if o is None else C.byref(o), out.ctypes.data, _ptr(mk), None))
+        if want_marks:
+            return out, [mk[int(mo[i]): int(mo[i]) + int(out[i]["rep"]["base"]["onsets"])] for i in range(n)]
+        return out
 
     def synth_batch(self, p, f, out=None, offsets=None, want_raw=False):
         """f: FilterParams (the presets) or TractParams (caller-defined tracts, vs_synth_batch_tract)."""

@@ -9,7 +9,8 @@
  *                      -- two ballots and one unsigned compare of the masked masks.  Onsets are written compactly.
  *   vs_cycles_kernel   one warp per stream, lanes along the cycles: length and peak of each cycle, exact integer
  *                      sums of lengths, peaks and absolute first differences, statistics in FP64 by lane 0.
- *   vs_report_kernel   the voice report on top of them (vs_flow_report_batch), below.
+ *   vs_report_kernel   the voice report on top of them (vs_flow_report_batch; vs_vowel_report_batch runs the cycles
+ *                      and report kernels on the period marks of vs_marks.cu), below.
  */
 #include "vs_device.cuh"
 
@@ -297,13 +298,26 @@ __global__ void __launch_bounds__(VS_AN_NT) vs_report_kernel(const int16_t *__re
     }
 }
 
-/* the two analysis kernels, then the report kernel; peaks: one slot per onset slot */
+/* the cycles and report kernels on onset lists already in place (the onset kernel's, or the period marks of
+ * vs_vowel_report_batch); peaks: one slot per onset slot */
+cudaError_t vs_launch_report_onsets(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, const uint32_t *onsets,
+                                    const uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s)
+{
+    const unsigned grid = (n_rows + VS_AN_NT / 32 - 1) / (VS_AN_NT / 32);
+    vs_cycles_kernel<<<grid, VS_AN_NT, 0, s>>>(x, rows, n_rows, onsets, counts, stats);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    vs_report_kernel<<<grid, VS_AN_NT, 0, s>>>(x, rows, n_rows, onsets, stats, peaks, out);
+    return cudaGetLastError();
+}
+
+/* the onset kernel, then the cycles and report kernels */
 cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
                              vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s)
 {
-    cudaError_t e = vs_launch_analyze(flow, rows, n_rows, onsets, counts, stats, s);
-    if (e != cudaSuccess) return e;
     const unsigned grid = (n_rows + VS_AN_NT / 32 - 1) / (VS_AN_NT / 32);
-    vs_report_kernel<<<grid, VS_AN_NT, 0, s>>>(flow, rows, n_rows, onsets, stats, peaks, out);
-    return cudaGetLastError();
+    vs_onsets_kernel<<<grid, VS_AN_NT, 0, s>>>(flow, rows, n_rows, onsets, counts);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    return vs_launch_report_onsets(flow, rows, n_rows, onsets, counts, stats, peaks, out, s);
 }

@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <array>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -27,8 +28,11 @@ cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uin
                               vs_flow_stats *out, cudaStream_t s);
 cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
                              vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
+cudaError_t vs_launch_report_onsets(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, const uint32_t *onsets,
+                                    const uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
 cudaError_t vs_launch_formants(const VsFormantArgs &a, vs_formant_stats *stats, vs_formant_frame *frames, cudaStream_t s);
 cudaError_t vs_launch_pitch(const VsPitchArgs &a, vs_pitch_stats *stats, vs_pitch_frame *frames, cudaStream_t s);
+cudaError_t vs_launch_marks(const VsMarkArgs &a, cudaStream_t s);
 
 namespace {
 
@@ -324,7 +328,12 @@ int slot_reserve(vs_ctx *ctx, Slot &sl, const Call &c, unsigned cp, size_t ns, c
     if ((rc = ring_pin(sl.h_chunks, nc * sizeof(VsChunk)))) return rc;
     if ((rc = ring_pin(sl.h_order, nrows * sizeof(uint32_t) + 16))) return rc;
     if ((rc = ring_pin(sl.h_nper, ns * sizeof(uint32_t)))) return rc;
-    if ((rc = ring_pin(sl.h_status, sizeof(int32_t)))) return rc;
+    if (!sl.h_status[cp].p) {
+        /* vs_sync reads the error flag of every ring slot, also of those no call has used yet: they must read 0, not
+         * whatever the fresh pinned allocation held */
+        if ((rc = ring_pin(sl.h_status, sizeof(int32_t)))) return rc;
+        for (PinBuf &b : sl.h_status) *(int32_t *)b.p = 0;
+    }
     return VS_OK;
 }
 
@@ -1217,28 +1226,35 @@ int vs_pitch_frames(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t
     return pitch_geometry(o, nsamp, fs, n, oo, nullptr, frames_out, nullptr);
 }
 
-int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
-                   size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames, const uint64_t *frame_offsets)
-{
-    if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
-    vs_pitch_opts op;
-    std::vector<VsPitchRow> rows(n);
-    std::vector<uint64_t> nfr(n);
-    int rc = pitch_geometry(o, nsamp, fs, n, op, rows.data(), nfr.data(), &ctx->err);
-    if (rc) return rc;
-    if (n == 0) return VS_OK;
-
-    /* the frame prefix and one table per distinct (Nw, tau_lo, tau_hi), host libm in double: the window w[0..Nw), then
-     * r_w(0) / r_w(tau) for tau = tau_lo-1 .. tau_hi+1, each r_w summed in index order */
-    const double pi = 3.14159265358979323846;
-    std::vector<uint64_t> frame0(n + 1, 0);
+/* the pitch track of vs_pitch_batch and vs_vowel_report_batch: the frame prefix, one table per distinct (Nw, tau_lo,
+ * tau_hi) (host libm in double: the window w[0..Nw), then r_w(0) / r_w(tau) for tau = tau_lo-1 .. tau_hi+1, each r_w
+ * summed in index order), the rows placed in the PCM, the kernels' arguments but for the device pointers, and their
+ * scratch: rows | frame prefix | tables | per-frame candidates */
+struct PitchTrack {
+    std::vector<VsPitchRow> rows;
+    std::vector<uint64_t> nfr, frame0;
     std::vector<double> tab;
+    Span span;
+    VsPitchArgs a = {};
+    size_t o_rows, o_pre, o_tab, o_cand;
+};
+static int pitch_track(const vs_pitch_opts *o, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs, size_t n,
+                       PitchTrack &p, Scratch &sc, std::string *err)
+{
+    vs_pitch_opts op;
+    p.rows.resize(n);
+    p.nfr.resize(n);
+    const int rc = pitch_geometry(o, nsamp, fs, n, op, p.rows.data(), p.nfr.data(), err);
+    if (rc || n == 0) return rc;
+    const double pi = 3.14159265358979323846;
+    p.frame0.assign(n + 1, 0);
     std::map<std::array<uint32_t, 3>, uint32_t> tab_at;
     uint32_t warp_doubles = 0;
     for (size_t i = 0; i < n; i++) {
-        VsPitchRow &r = rows[i];
-        const auto ins = tab_at.insert({{r.Nw, r.tau_lo, r.tau_hi}, (uint32_t)tab.size()});
+        VsPitchRow &r = p.rows[i];
+        const auto ins = tab_at.insert({{r.Nw, r.tau_lo, r.tau_hi}, (uint32_t)p.tab.size()});
         if (ins.second) {
+            std::vector<double> &tab = p.tab;
             const size_t w0 = tab.size();
             for (uint32_t m = 0; m < r.Nw; m++) tab.push_back(0.5 - 0.5 * std::cos(2.0 * pi * ((double)m + 0.5) / (double)r.Nw));
             auto rw = [&](uint32_t tau) {
@@ -1251,39 +1267,148 @@ int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, con
         }
         r.tab = ins.first->second;
         warp_doubles = std::max(warp_doubles, (r.Nw + 32 + (r.tau_hi - r.tau_lo + 3) + 1) & ~1u);
-        frame0[i + 1] = frame0[i] + nfr[i];
+        p.frame0[i + 1] = p.frame0[i] + p.nfr[i];
     }
-    const Span span = place_rows(offsets, nsamp, rows);
-    const uint64_t F = frame0[n];
-    VsPitchArgs a = {};
-    a.n_rows = (uint32_t)n; a.n_frames = F; a.warp_doubles = warp_doubles;
+    p.span = place_rows(offsets, nsamp, p.rows);
+    VsPitchArgs &a = p.a;
+    a.n_rows = (uint32_t)n; a.n_frames = p.frame0[n]; a.warp_doubles = warp_doubles;
     a.warps = (uint32_t)std::min<size_t>(4, (227 * 1024) / (warp_doubles * sizeof(double)));   /* the per-block cap of sm_100 */
     a.f_min = op.f_min_hz; a.voicing = op.voicing_threshold; a.silence = op.silence_threshold; a.octave_cost = op.octave_cost;
+    p.o_rows = sc.take(n * sizeof(VsPitchRow)); p.o_pre = sc.take((n + 1) * sizeof(uint64_t));
+    p.o_tab = sc.take(p.tab.size() * sizeof(double)); p.o_cand = sc.take(a.n_frames * sizeof(VsPitchCand));
+    return VS_OK;
+}
 
-    /* scratch: rows | frame prefix | tables | per-frame candidates | stats | frame records */
+/* points the pitch kernels' arguments into the call's scratch and uploads rows, frame prefix and tables */
+static int pitch_upload(vs_ctx *ctx, PitchTrack &p, const PcmDev<const int16_t> &d)
+{
+    const size_t n = p.rows.size();
+    VsPitchArgs &a = p.a;
+    a.pcm = d.pcm;
+    a.rows = (const VsPitchRow *)(d.scratch + p.o_rows);
+    a.frame0 = (const uint64_t *)(d.scratch + p.o_pre);
+    a.tab = (const double *)(d.scratch + p.o_tab);
+    a.cand = (VsPitchCand *)(d.scratch + p.o_cand);
+    CU(cudaMemcpyAsync((void *)a.rows, p.rows.data(), n * sizeof(VsPitchRow), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.frame0, p.frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
+    CU(cudaMemcpyAsync((void *)a.tab, p.tab.data(), p.tab.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
+    return VS_OK;
+}
+
+int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                   size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames, const uint64_t *frame_offsets)
+{
+    if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
+    PitchTrack p;
     Scratch sc;
-    const size_t o_rows = sc.take(n * sizeof(VsPitchRow)), o_pre = sc.take((n + 1) * sizeof(uint64_t));
-    const size_t o_tab = sc.take(tab.size() * sizeof(double)), o_cand = sc.take(F * sizeof(VsPitchCand));
+    int rc = pitch_track(o, offsets, nsamp, fs, n, p, sc, &ctx->err);
+    if (rc) return rc;
+    if (n == 0) return VS_OK;
+    /* scratch, after the track's: stats | frame records */
+    const uint64_t F = p.frame0[n];
     const size_t o_st = sc.take(n * sizeof(vs_pitch_stats)), o_fr = sc.take(frames ? F * sizeof(vs_pitch_frame) : 0);
     DeviceGuard restore_device;
     PcmDev<const int16_t> d;
-    if ((rc = pcm_call_begin(ctx, pcm, span, sc.bytes, d))) return rc;
-    a.pcm = d.pcm;
-    a.rows = (const VsPitchRow *)(d.scratch + o_rows);
-    a.frame0 = (const uint64_t *)(d.scratch + o_pre);
-    a.tab = (const double *)(d.scratch + o_tab);
-    a.cand = (VsPitchCand *)(d.scratch + o_cand);
+    if ((rc = pcm_call_begin(ctx, pcm, p.span, sc.bytes, d))) return rc;
     vs_pitch_stats *d_stats = (vs_pitch_stats *)(d.scratch + o_st);
     vs_pitch_frame *d_frames = frames ? (vs_pitch_frame *)(d.scratch + o_fr) : nullptr;
-    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsPitchRow), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
-    CU(vs_launch_pitch(a, d_stats, d_frames, d.st));
+    if ((rc = pitch_upload(ctx, p, d))) return rc;
+    CU(vs_launch_pitch(p.a, d_stats, d_frames, d.st));
     CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_pitch_stats), cudaMemcpyDeviceToHost, d.st));
     /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
-    auto records = [&](size_t i) { return RowCopy{frame0[i], frame_offsets ? frame_offsets[i] : frame0[i], nfr[i]}; };
+    auto records = [&](size_t i) { return RowCopy{p.frame0[i], frame_offsets ? frame_offsets[i] : p.frame0[i], p.nfr[i]}; };
     if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;
     CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are pageable host memory */
+    return VS_OK;
+}
+
+/* the mark slots of a stream (vs_vowel_mark_slots): every step is at least lround(VS_MARK_STEP_MIN T_lo) samples */
+static uint64_t mark_slots(uint64_t n, const VsPitchRow &r)
+{
+    if (n < r.Nw) return 0;
+    const double t_lo = ((double)r.tau_lo - 0.5) * (1.0 - 0x1p-20);
+    const uint64_t step = (uint64_t)std::llround(VS_MARK_STEP_MIN * t_lo);
+    return (n - 1) / step + 1;
+}
+
+int vs_vowel_mark_slots(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t *fs, size_t n, uint64_t *slots_out)
+{
+    if (!nsamp || !slots_out) return VS_EINVAL;
+    vs_pitch_opts oo;
+    std::vector<VsPitchRow> rows(n);
+    const int rc = pitch_geometry(o, nsamp, fs, n, oo, rows.data(), slots_out, nullptr);
+    if (rc) return rc;
+    for (size_t i = 0; i < n; i++) slots_out[i] = mark_slots(nsamp[i], rows[i]);
+    return VS_OK;
+}
+
+static_assert(sizeof(vs_vowel_report) == 96 && sizeof(VsMarkRun) == 16 &&
+              offsetof(vs_vowel_report, run_frame) == sizeof(vs_flow_report), "vs_vowel_report = report | VsMarkRun");
+
+int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
+                          size_t n, const vs_pitch_opts *o, vs_vowel_report *out, uint32_t *marks, const uint64_t *mark_offsets)
+{
+    if (!ctx || !pcm || !nsamp || !out) return VS_EINVAL;
+    PitchTrack p;
+    Scratch sc;
+    int rc = pitch_track(o, offsets, nsamp, fs, n, p, sc, &ctx->err);
+    if (rc) return rc;
+    if (n == 0) return VS_OK;
+
+    /* the report's rows: each stream's onset list holds its mark slots.  The stage of the marks kernel holds a reference
+     * period and the span of its candidates: lround(VS_MARK_STEP_MAX T) + lround(T) <= 2.25 T + 1 samples, with every
+     * period a frame can publish below tau_hi + 1 */
+    std::vector<VsAnalyzeRow> arows(n);
+    uint64_t slots = 0;
+    uint32_t tau_max = 0;
+    for (size_t i = 0; i < n; i++) {
+        const uint64_t cap = mark_slots(nsamp[i], p.rows[i]);
+        arows[i] = {p.rows[i].off, slots, (uint32_t)nsamp[i], (uint32_t)cap, fs ? fs[i] : 22050, 0, 0};
+        slots += cap;
+        tau_max = std::max(tau_max, p.rows[i].tau_hi);
+    }
+    const double t_hi = ((double)tau_max + 1.0) * (1.0 + 0x1p-20);
+    const uint32_t stage = ((uint32_t)std::ceil((VS_MARK_STEP_MAX + 1.0) * t_hi) + 2u + 7u) & ~7u;
+
+    /* scratch, after the track's: pitch stats | frame records | report rows | mark counts | stats | marks | peaks |
+     * reports | runs */
+    const uint64_t F = p.frame0[n];
+    const size_t o_pst = sc.take(n * sizeof(vs_pitch_stats)), o_fr = sc.take(F * sizeof(vs_pitch_frame));
+    const size_t o_rows = sc.take(n * sizeof(VsAnalyzeRow)), o_cnt = sc.take(n * sizeof(uint32_t));
+    const size_t o_st = sc.take(n * sizeof(vs_flow_stats)), o_marks = sc.take(slots * sizeof(uint32_t));
+    const size_t o_peaks = sc.take(slots * sizeof(int32_t)), o_rep = sc.take(n * sizeof(vs_flow_report));
+    const size_t o_run = sc.take(n * sizeof(VsMarkRun));
+    DeviceGuard restore_device;
+    PcmDev<const int16_t> d;
+    if ((rc = pcm_call_begin(ctx, pcm, p.span, sc.bytes, d))) return rc;
+    if ((rc = pitch_upload(ctx, p, d))) return rc;
+    VsMarkArgs m = {};
+    m.pcm = d.pcm; m.prows = p.a.rows; m.frame0 = p.a.frame0; m.frames = d.scratch + o_fr;
+    m.arows = (const VsAnalyzeRow *)(d.scratch + o_rows);
+    m.marks = (uint32_t *)(d.scratch + o_marks);
+    m.counts = (uint32_t *)(d.scratch + o_cnt);
+    m.run = (VsMarkRun *)(d.scratch + o_run);
+    m.n_rows = (uint32_t)n; m.stage = stage;
+    vs_flow_report *d_rep = (vs_flow_report *)(d.scratch + o_rep);
+    CU(cudaMemcpyAsync(d.scratch + o_rows, arows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, d.st));
+    CU(vs_launch_pitch(p.a, (vs_pitch_stats *)(d.scratch + o_pst), (vs_pitch_frame *)(d.scratch + o_fr), d.st));
+    CU(vs_launch_marks(m, d.st));
+    CU(vs_launch_report_onsets(d.pcm, m.arows, (uint32_t)n, m.marks, m.counts, (vs_flow_stats *)(d.scratch + o_st),
+                               (int32_t *)(d.scratch + o_peaks), d_rep, d.st));
+    /* the report and the run side by side in each 96-byte record */
+    CU(cudaMemcpy2DAsync(out, sizeof(vs_vowel_report), d_rep, sizeof(vs_flow_report), sizeof(vs_flow_report), n,
+                         cudaMemcpyDeviceToHost, d.st));
+    CU(cudaMemcpy2DAsync(&out->run_frame, sizeof(vs_vowel_report), m.run, sizeof(VsMarkRun), sizeof(VsMarkRun), n,
+                         cudaMemcpyDeviceToHost, d.st));
+    CU(cudaStreamSynchronize(d.st));                          /* the mark counts, `arows` and `out` are pageable host memory */
+    if (marks) {
+        /* stream i's marks: its slots on the device, mark_offsets[i] (NULL: the same dense prefix) on the host */
+        auto rows = [&](size_t i) {
+            return RowCopy{arows[i].ons_off, mark_offsets ? mark_offsets[i] : arows[i].ons_off, std::min<uint64_t>(out[i].rep.base.onsets, arows[i].cap)};
+        };
+        if ((rc = copy_rows_home(ctx, marks, m.marks, n, rows, d.st))) return rc;
+        CU(cudaStreamSynchronize(d.st));
+    }
     return VS_OK;
 }
 

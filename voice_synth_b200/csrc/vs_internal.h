@@ -238,4 +238,25 @@ struct VsPitchArgs {
     double            f_min, voicing, silence, octave_cost;
 };
 
+/* period marks (vs_vowel_report_batch): the voiced run a stream's marks lie in, as vs_vowel_report holds it */
+struct VsMarkRun {
+    uint32_t frame, frames;   /* first pitch frame and frame count of the run                             */
+    uint32_t start, len;      /* its samples                                                              */
+};
+
+/* the launch arguments of the marks kernel: the pitch call's geometry and frame records in, onset lists out */
+struct VsMarkArgs {
+    const int16_t      *pcm;
+    const VsPitchRow   *prows;      /* Nw, H and fs of each stream                                              */
+    const uint64_t     *frame0;     /* [n_rows + 1]: each stream's first frame record (prefix sum)              */
+    const void         *frames;     /* vs_pitch_frame[n_frames], as vs_pitch_batch returns them                 */
+    const VsAnalyzeRow *arows;      /* row offset, onset-list slot and capacity of each stream                  */
+    uint32_t           *marks;      /* the onset lists of the report kernels                                   */
+    uint32_t           *counts;     /* [n_rows] marks per stream                                                */
+    VsMarkRun          *run;        /* [n_rows]                                                                  */
+    uint32_t            n_rows;
+    uint32_t            stage;      /* int16 samples of shared memory per warp: the longest reference period plus
+                                       the span of its candidates                                              */
+};
+
 #endif
