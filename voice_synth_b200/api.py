@@ -295,60 +295,51 @@ def flow_nsamples(p):
     return out
 
 
+def _opts(struct, defaults, what, opts):
+    """struct from a dict of the fields to change (the rest keep defaults); None stays None (NULL)"""
+    if opts is None or isinstance(opts, struct):
+        return opts
+    unknown = set(opts) - set(defaults)
+    if unknown:
+        raise ValueError(f"unknown {what} options {sorted(unknown)}")
+    return struct(**{**defaults, **opts})
+
+
 def formant_opts(opts=None):
     """vs_formant_opts from a dict of the fields to change (the rest keep FORMANT_DEFAULTS); None stays None (NULL)"""
-    if opts is None or isinstance(opts, FormantOptsC):
-        return opts
-    unknown = set(opts) - set(FORMANT_DEFAULTS)
-    if unknown:
-        raise ValueError(f"unknown formant options {sorted(unknown)}")
-    return FormantOptsC(**{**FORMANT_DEFAULTS, **opts})
-
-
-def formant_frames(nsamp, fs=None, opts=None):
-    """frames per stream of vs_formant_batch (host only, validates like the batch call; raises VsError)"""
-    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-    rate = _per_stream(fs, np.int32, len(ns))
-    o = formant_opts(opts)
-    out = np.zeros(len(ns), dtype=np.uint64)
-    rc = _lib.load().vs_formant_frames(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
-    if rc:
-        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
-    return out
+    return _opts(FormantOptsC, FORMANT_DEFAULTS, "formant", opts)
 
 
 def pitch_opts(opts=None):
     """vs_pitch_opts from a dict of the fields to change (the rest keep PITCH_DEFAULTS); None stays None (NULL)"""
-    if opts is None or isinstance(opts, PitchOptsC):
-        return opts
-    unknown = set(opts) - set(PITCH_DEFAULTS)
-    if unknown:
-        raise ValueError(f"unknown pitch options {sorted(unknown)}")
-    return PitchOptsC(**{**PITCH_DEFAULTS, **opts})
+    return _opts(PitchOptsC, PITCH_DEFAULTS, "pitch", opts)
+
+
+def _counts(call, to_c, nsamp, fs, opts):
+    """per-stream counts from a host-only call that validates like its batch call (raises VsError)"""
+    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+    rate = _per_stream(fs, np.int32, len(ns))
+    o = to_c(opts)
+    out = np.zeros(len(ns), dtype=np.uint64)
+    rc = call(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
+    if rc:
+        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
+    return out
+
+
+def formant_frames(nsamp, fs=None, opts=None):
+    """frames per stream of vs_formant_batch (host only, validates like the batch call; raises VsError)"""
+    return _counts(_lib.load().vs_formant_frames, formant_opts, nsamp, fs, opts)
 
 
 def pitch_frames(nsamp, fs=None, opts=None):
     """frames per stream of vs_pitch_batch (host only, validates like the batch call; raises VsError)"""
-    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-    rate = _per_stream(fs, np.int32, len(ns))
-    o = pitch_opts(opts)
-    out = np.zeros(len(ns), dtype=np.uint64)
-    rc = _lib.load().vs_pitch_frames(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
-    if rc:
-        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
-    return out
+    return _counts(_lib.load().vs_pitch_frames, pitch_opts, nsamp, fs, opts)
 
 
 def vowel_mark_slots(nsamp, fs=None, opts=None):
     """mark slots per stream of vs_vowel_report_batch (host only, validates like the batch call; raises VsError)"""
-    ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-    rate = _per_stream(fs, np.int32, len(ns))
-    o = pitch_opts(opts)
-    out = np.zeros(len(ns), dtype=np.uint64)
-    rc = _lib.load().vs_vowel_mark_slots(None if o is None else C.byref(o), ns.ctypes.data, _ptr(rate), len(ns), out.ctypes.data)
-    if rc:
-        raise VsError(rc, _lib.load().vs_strerror(rc).decode())
-    return out
+    return _counts(_lib.load().vs_vowel_mark_slots, pitch_opts, nsamp, fs, opts)
 
 
 def _per_stream(x, dtype, n):
@@ -488,42 +479,40 @@ class Context:
         self._check(call(self.h, _ptr(flow), _ptr(offs), ns.ctypes.data, _ptr(rate), _ptr(tl), _ptr(th), n, res.ctypes.data))
         return res
 
+    def _frame_wise(self, call, dtype, to_c, slots, rec_dtype, pcm, nsamp, offsets, fs, opts, want_records):
+        """a frame-wise call: per stream its results (dtype) and, with want_records, its records (rec_dtype) at the
+        dense prefix of slots(nsamp, fs, opts).  Returns the results, the records and that prefix."""
+        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
+        n = len(ns)
+        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
+        o = to_c(opts)
+        res = np.zeros(n, dtype=dtype)
+        rec, ro = None, None
+        if want_records:
+            ro = np.concatenate([[0], np.cumsum(slots(ns, fs, opts))]).astype(np.uint64)
+            rec = np.zeros(int(ro[-1]), dtype=rec_dtype)
+        self._check(call(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n, None if o is None else C.byref(o),
+                         res.ctypes.data, _ptr(rec), None))
+        return res, rec, ro
+
     def formant_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_frames=False):
         """formant analysis (vs_formant_batch): per-stream statistics (FORMANT_STATS_DTYPE) and, with want_frames, the
         list of each stream's frame records (FORMANT_FRAME_DTYPE).  pcm: numpy array or device tensor; opts: None (the
         defaults) or a dict of the vs_formant_opts fields to change."""
-        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-        n = len(ns)
-        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
-        o = formant_opts(opts)
-        st = np.zeros(n, dtype=FORMANT_STATS_DTYPE)
-        fr, fo = None, None
+        st, fr, fo = self._frame_wise(self.L.vs_formant_batch, FORMANT_STATS_DTYPE, formant_opts, formant_frames,
+                                      FORMANT_FRAME_DTYPE, pcm, nsamp, offsets, fs, opts, want_frames)
         if want_frames:
-            fo = np.concatenate([[0], np.cumsum(formant_frames(ns, fs, opts))]).astype(np.uint64)
-            fr = np.zeros(int(fo[-1]), dtype=FORMANT_FRAME_DTYPE)
-        self._check(self.L.vs_formant_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
-                                            None if o is None else C.byref(o), st.ctypes.data, _ptr(fr), None))
-        if want_frames:
-            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
+            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(len(st))]
         return st
 
     def pitch_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_frames=False):
         """pitch and harmonicity (vs_pitch_batch): per-stream statistics (PITCH_STATS_DTYPE) and, with want_frames, the
         list of each stream's frame records (PITCH_FRAME_DTYPE).  pcm: numpy array or device tensor; opts: None (the
         defaults) or a dict of the vs_pitch_opts fields to change."""
-        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-        n = len(ns)
-        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
-        o = pitch_opts(opts)
-        st = np.zeros(n, dtype=PITCH_STATS_DTYPE)
-        fr, fo = None, None
+        st, fr, fo = self._frame_wise(self.L.vs_pitch_batch, PITCH_STATS_DTYPE, pitch_opts, pitch_frames, PITCH_FRAME_DTYPE,
+                                      pcm, nsamp, offsets, fs, opts, want_frames)
         if want_frames:
-            fo = np.concatenate([[0], np.cumsum(pitch_frames(ns, fs, opts))]).astype(np.uint64)
-            fr = np.zeros(int(fo[-1]), dtype=PITCH_FRAME_DTYPE)
-        self._check(self.L.vs_pitch_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
-                                          None if o is None else C.byref(o), st.ctypes.data, _ptr(fr), None))
-        if want_frames:
-            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(n)]
+            return st, [fr[int(fo[i]): int(fo[i + 1])] for i in range(len(st))]
         return st
 
     def vowel_report_batch(self, pcm, nsamp, offsets=None, fs=None, opts=None, want_marks=False):
@@ -531,19 +520,10 @@ class Context:
         run they lie in (VOWEL_REPORT_DTYPE) and, with want_marks, the list of each stream's marks (uint32, stream
         coordinates).  pcm: numpy array or device tensor; opts: None (the defaults) or a dict of the vs_pitch_opts fields
         to change."""
-        ns = np.ascontiguousarray(nsamp, dtype=np.uint64)
-        n = len(ns)
-        offs, rate = (_per_stream(x, dt, n) for x, dt in ((offsets, np.uint64), (fs, np.int32)))
-        o = pitch_opts(opts)
-        out = np.zeros(n, dtype=VOWEL_REPORT_DTYPE)
-        mk, mo = None, None
+        out, mk, mo = self._frame_wise(self.L.vs_vowel_report_batch, VOWEL_REPORT_DTYPE, pitch_opts, vowel_mark_slots,
+                                       np.uint32, pcm, nsamp, offsets, fs, opts, want_marks)
         if want_marks:
-            mo = np.concatenate([[0], np.cumsum(vowel_mark_slots(ns, fs, opts))]).astype(np.uint64)
-            mk = np.zeros(int(mo[-1]), dtype=np.uint32)
-        self._check(self.L.vs_vowel_report_batch(self.h, _ptr(pcm), _ptr(offs), ns.ctypes.data, _ptr(rate), n,
-                                                 None if o is None else C.byref(o), out.ctypes.data, _ptr(mk), None))
-        if want_marks:
-            return out, [mk[int(mo[i]): int(mo[i]) + int(out[i]["rep"]["base"]["onsets"])] for i in range(n)]
+            return out, [mk[int(mo[i]): int(mo[i]) + int(out[i]["rep"]["base"]["onsets"])] for i in range(len(out))]
         return out
 
     def synth_batch(self, p, f, out=None, offsets=None, want_raw=False):

@@ -49,13 +49,6 @@ __global__ void __launch_bounds__(VS_AN_NT) vs_onsets_kernel(const int16_t *flow
     if (lane == 0) counts[s] = count;
 }
 
-__device__ __forceinline__ long long vs_warp_sum(long long v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(VS_FULL, v, o);
-    return v;
-}
-
 __global__ void __launch_bounds__(VS_AN_NT) vs_cycles_kernel(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows,
                                                              const uint32_t *onsets, const uint32_t *counts, vs_flow_stats *out)
 {
@@ -112,17 +105,6 @@ __global__ void __launch_bounds__(VS_AN_NT) vs_cycles_kernel(const int16_t *flow
     }
 }
 
-cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
-                              vs_flow_stats *out, cudaStream_t s)
-{
-    const unsigned grid = (n_rows + VS_AN_NT / 32 - 1) / (VS_AN_NT / 32);
-    vs_onsets_kernel<<<grid, VS_AN_NT, 0, s>>>(flow, rows, n_rows, onsets, counts);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    vs_cycles_kernel<<<grid, VS_AN_NT, 0, s>>>(flow, rows, n_rows, onsets, counts, out);
-    return cudaGetLastError();
-}
-
 /* ---- voice report (vs_flow_report_batch): Praat's jitter and shimmer quotients and a cycle-averaged HNR ----------
  *   vs_report_kernel   one warp per stream, after the two kernels above, whose onset lists and statistics it reads.
  *                      HNR pass: lanes along j, 32*VS_RPT_R values of j per tile held as int64 S_j in registers
@@ -167,8 +149,7 @@ __device__ __forceinline__ VsWinSums vs_window_sums(uint32_t K, int lane, V v)
     if (!PEAKS) w.d1 = vs_warp_sum(w.d1);
     if (PEAKS) {
         w.n11 = vs_warp_sum(w.n11);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) w.db += __shfl_xor_sync(VS_FULL, w.db, o);
+        w.db = vs_warp_sum(w.db);
         w.nonpos = __any_sync(VS_FULL, w.nonpos);
     }
     return w;
@@ -198,12 +179,11 @@ __global__ void __launch_bounds__(VS_AN_NT) vs_report_kernel(const int16_t *__re
     const uint32_t s = blockIdx.x * (VS_AN_NT / 32) + (threadIdx.x >> 5);
     if (s >= n_rows) return;
     const VsAnalyzeRow r = rows[s];
-    const float qnan = __int_as_float(0x7fc00000);
     vs_flow_report rep;
     rep.base = stats[s];
-    rep.jitter_abs_us = rep.jitter_rap_pct = rep.jitter_ppq5_pct = rep.jitter_ddp_pct = qnan;
-    rep.shimmer_db = rep.shimmer_apq3_pct = rep.shimmer_apq5_pct = rep.shimmer_apq11_pct = rep.shimmer_dda_pct = qnan;
-    rep.hnr_db = qnan;
+    rep.jitter_abs_us = rep.jitter_rap_pct = rep.jitter_ppq5_pct = rep.jitter_ddp_pct = VS_QNAN_F;
+    rep.shimmer_db = rep.shimmer_apq3_pct = rep.shimmer_apq5_pct = rep.shimmer_apq11_pct = rep.shimmer_dda_pct = VS_QNAN_F;
+    rep.hnr_db = VS_QNAN_F;
     rep.hnr_len = 0; rep.reserved = 0;
     const uint32_t K = rep.base.cycles;                     /* 0 when the onset list overflowed */
     if ((rep.base.flags & VS_STATS_OVERFLOW) || K == 0) {
@@ -298,26 +278,20 @@ __global__ void __launch_bounds__(VS_AN_NT) vs_report_kernel(const int16_t *__re
     }
 }
 
-/* the cycles and report kernels on onset lists already in place (the onset kernel's, or the period marks of
- * vs_vowel_report_batch); peaks: one slot per onset slot */
-cudaError_t vs_launch_report_onsets(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, const uint32_t *onsets,
-                                    const uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s)
+/* the onset kernel when find_onsets (otherwise the onset lists are in place already: the period marks of
+ * vs_vowel_report_batch), then the cycles kernel and, when peaks and out are given, the report kernel (peaks: one slot
+ * per onset slot) */
+cudaError_t vs_launch_analyze(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, bool find_onsets, uint32_t *onsets,
+                              uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s)
 {
     const unsigned grid = (n_rows + VS_AN_NT / 32 - 1) / (VS_AN_NT / 32);
+    cudaError_t e;
+    if (find_onsets) {
+        vs_onsets_kernel<<<grid, VS_AN_NT, 0, s>>>(x, rows, n_rows, onsets, counts);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
     vs_cycles_kernel<<<grid, VS_AN_NT, 0, s>>>(x, rows, n_rows, onsets, counts, stats);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
+    if ((e = cudaGetLastError()) != cudaSuccess || !peaks || !out) return e;
     vs_report_kernel<<<grid, VS_AN_NT, 0, s>>>(x, rows, n_rows, onsets, stats, peaks, out);
     return cudaGetLastError();
-}
-
-/* the onset kernel, then the cycles and report kernels */
-cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
-                             vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s)
-{
-    const unsigned grid = (n_rows + VS_AN_NT / 32 - 1) / (VS_AN_NT / 32);
-    vs_onsets_kernel<<<grid, VS_AN_NT, 0, s>>>(flow, rows, n_rows, onsets, counts);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    return vs_launch_report_onsets(flow, rows, n_rows, onsets, counts, stats, peaks, out, s);
 }

@@ -24,12 +24,8 @@ cudaError_t vs_render_init_device();
 cudaError_t vs_launch_flow_rows(const VsRenderArgs &a, cudaStream_t s);
 cudaError_t vs_launch_fp64_peak(double *scratch, int blocks, int iters, cudaStream_t s);
 cudaError_t vs_launch_vnoise(int16_t *pcm, const VsNoiseRow *rows, uint32_t n_rows, cudaStream_t s);
-cudaError_t vs_launch_analyze(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
-                              vs_flow_stats *out, cudaStream_t s);
-cudaError_t vs_launch_report(const int16_t *flow, const VsAnalyzeRow *rows, uint32_t n_rows, uint32_t *onsets, uint32_t *counts,
-                             vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
-cudaError_t vs_launch_report_onsets(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, const uint32_t *onsets,
-                                    const uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
+cudaError_t vs_launch_analyze(const int16_t *x, const VsAnalyzeRow *rows, uint32_t n_rows, bool find_onsets, uint32_t *onsets,
+                              uint32_t *counts, vs_flow_stats *stats, int32_t *peaks, vs_flow_report *out, cudaStream_t s);
 cudaError_t vs_launch_formants(const VsFormantArgs &a, vs_formant_stats *stats, vs_formant_frame *frames, cudaStream_t s);
 cudaError_t vs_launch_pitch(const VsPitchArgs &a, vs_pitch_stats *stats, vs_pitch_frame *frames, cudaStream_t s);
 cudaError_t vs_launch_marks(const VsMarkArgs &a, cudaStream_t s);
@@ -774,6 +770,67 @@ int copy_rows_home(vs_ctx *ctx, T *dst, const T *src, size_t n, Row row, cudaStr
     return VS_OK;
 }
 
+/* ---- frame-wise calls on PCM: formants, pitch, vowel report ------------------------------------------------------ */
+const double pi = 3.14159265358979323846;
+
+/* stream i's frame step h = lround(hl), hl the step in samples, and its frame count for a window of nw samples */
+int frame_step(std::string *err, size_t i, double hl, uint64_t nsamp, uint64_t nw, uint64_t &h, uint64_t &frames)
+{
+    if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
+    h = (uint64_t)std::lround(hl);
+    frames = nsamp >= nw ? (nsamp - nw) / h + 1 : 0;
+    return VS_OK;
+}
+
+/* the frame track of a frame-wise call: the rows (the call's geometry fills them but for off, which build() places in
+ * the PCM, and the table offset row.*tab_off), each stream's frame count, the frame prefix, the tables (one per
+ * distinct key(row), appended by fill(row, tab) and at offsets in order of first appearance), the span of the PCM, and
+ * the scratch: rows | frame prefix | tables */
+template <class Row>
+struct FrameTrack {
+    std::vector<Row> rows;
+    std::vector<uint64_t> nfr, frame0;
+    std::vector<double> tab;
+    Span span;
+    size_t o_rows = 0, o_pre = 0, o_tab = 0;
+
+    explicit FrameTrack(size_t n) : rows(n), nfr(n) {}
+    template <class Key, class Fill>
+    void build(const uint64_t *offsets, const uint64_t *nsamp, uint32_t Row::*tab_off, Key key, Fill fill, Scratch &sc)
+    {
+        const size_t n = rows.size();
+        frame0.assign(n + 1, 0);
+        std::map<decltype(key(rows[0])), uint32_t> tab_at;
+        for (size_t i = 0; i < n; i++) {
+            Row &r = rows[i];
+            const auto ins = tab_at.insert({key(r), (uint32_t)tab.size()});
+            if (ins.second) fill(r, tab);
+            r.*tab_off = ins.first->second;
+            frame0[i + 1] = frame0[i] + nfr[i];
+        }
+        span = place_rows(offsets, nsamp, rows);
+        o_rows = sc.take(n * sizeof(Row));
+        o_pre = sc.take((n + 1) * sizeof(uint64_t));
+        o_tab = sc.take(tab.size() * sizeof(double));
+    }
+    /* uploads rows, frame prefix and tables into the call's scratch */
+    int upload(vs_ctx *ctx, const PcmDev<const int16_t> &d) const
+    {
+        CU(cudaMemcpyAsync(d.scratch + o_rows, rows.data(), rows.size() * sizeof(Row), cudaMemcpyHostToDevice, d.st));
+        CU(cudaMemcpyAsync(d.scratch + o_pre, frame0.data(), frame0.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
+        CU(cudaMemcpyAsync(d.scratch + o_tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
+        return VS_OK;
+    }
+};
+
+/* stream i's count(i) records home: from pre[i] on the device to offsets[i] on the host (offsets NULL: the same dense
+ * prefix), merged into runs */
+template <class T, class Count>
+int records_home(vs_ctx *ctx, T *dst, const T *src, const uint64_t *pre, const uint64_t *offsets, size_t n, Count count, cudaStream_t st)
+{
+    return copy_rows_home(ctx, dst, src, n, [&](size_t i) { return RowCopy{pre[i], offsets ? offsets[i] : pre[i], count(i)}; }, st);
+}
+
 } // namespace
 
 /* ================================================================================================
@@ -1066,14 +1123,11 @@ static int flow_analysis(vs_ctx *ctx, const int16_t *flow, const uint64_t *offse
     uint32_t *d_cnt = (uint32_t *)(d.scratch + o_cnt), *d_ons = (uint32_t *)(d.scratch + o_ons);
     vs_flow_stats *d_st = (vs_flow_stats *)(d.scratch + o_st);
     CU(cudaMemcpyAsync(d.scratch + o_rows, rows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, d.st));
-    if (!report) {
-        CU(vs_launch_analyze(d.pcm, d_rows, (uint32_t)n, d_ons, d_cnt, d_st, d.st));
-        CU(cudaMemcpyAsync(stats, d_st, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, d.st));
-    } else {
-        vs_flow_report *d_rep = (vs_flow_report *)(d.scratch + o_rep);
-        CU(vs_launch_report(d.pcm, d_rows, (uint32_t)n, d_ons, d_cnt, d_st, (int32_t *)(d.scratch + o_peaks), d_rep, d.st));
-        CU(cudaMemcpyAsync(report, d_rep, n * sizeof(vs_flow_report), cudaMemcpyDeviceToHost, d.st));
-    }
+    int32_t *d_peaks = report ? (int32_t *)(d.scratch + o_peaks) : nullptr;
+    vs_flow_report *d_rep = report ? (vs_flow_report *)(d.scratch + o_rep) : nullptr;
+    CU(vs_launch_analyze(d.pcm, d_rows, (uint32_t)n, true, d_ons, d_cnt, d_st, d_peaks, d_rep, d.st));
+    if (!report) CU(cudaMemcpyAsync(stats, d_st, n * sizeof(vs_flow_stats), cudaMemcpyDeviceToHost, d.st));
+    else CU(cudaMemcpyAsync(report, d_rep, n * sizeof(vs_flow_report), cudaMemcpyDeviceToHost, d.st));
     CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are the caller's / pageable memory */
     return VS_OK;
 }
@@ -1107,10 +1161,9 @@ static int formant_geometry(const vs_formant_opts *in, const uint64_t *nsamp, co
         const long nw = wl > -1e9 && wl < 1e9 ? lround(wl) : -1;
         if (nw < (long)o.order + 1 || nw > VS_FORMANT_MAX_WIN)
             return vs_error(err, VS_ERANGE, "stream %zu: window of %ld samples, needs %u..%d", i, nw, o.order + 1, VS_FORMANT_MAX_WIN);
-        if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
-        const uint64_t h = (uint64_t)lround(hl);
+        uint64_t h = 0;
+        if (const int rc = frame_step(err, i, hl, nsamp[i], (uint64_t)nw, h, frames[i])) return rc;
         if (rows) rows[i] = {0, (uint32_t)nsamp[i], (uint32_t)nw, (uint32_t)h, 0, 0.0, (double)rate};
-        frames[i] = nsamp[i] >= (uint64_t)nw ? (nsamp[i] - (uint64_t)nw) / h + 1 : 0;
         return VS_OK;
     });
 }
@@ -1128,33 +1181,23 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
 {
     if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
     vs_formant_opts op;
-    std::vector<VsFormantRow> rows(n);
-    std::vector<uint64_t> nfr(n);
-    int rc = formant_geometry(o, nsamp, fs, n, op, rows.data(), nfr.data(), &ctx->err);
+    FrameTrack<VsFormantRow> ft(n);
+    int rc = formant_geometry(o, nsamp, fs, n, op, ft.rows.data(), ft.nfr.data(), &ctx->err);
     if (rc) return rc;
     if (n == 0) return VS_OK;
 
-    /* pre-emphasis, the frame prefix and one window table per distinct window length; host libm in double */
-    const double pi = 3.14159265358979323846;
-    std::vector<uint64_t> frame0(n + 1, 0);
-    std::vector<double> win;
-    std::vector<std::pair<uint32_t, uint32_t>> win_at;        /* (Nw, offset) */
+    /* pre-emphasis and one Hamming window per distinct window length; host libm in double */
     uint32_t max_nw = 0;
-    for (size_t i = 0; i < n; i++) {
-        VsFormantRow &r = rows[i];
+    for (VsFormantRow &r : ft.rows) {
         r.mu = op.preemph_hz > 0.0f ? std::exp(-2.0 * pi * (double)op.preemph_hz / r.fs) : 0.0;
-        auto it = std::find_if(win_at.begin(), win_at.end(), [&](const std::pair<uint32_t, uint32_t> &e) { return e.first == r.Nw; });
-        if (it == win_at.end()) {
-            win_at.push_back({r.Nw, (uint32_t)win.size()});
-            for (uint32_t m = 0; m < r.Nw; m++) win.push_back(0.54 - 0.46 * std::cos(2.0 * pi * (double)m / (double)(r.Nw - 1)));
-            it = win_at.end() - 1;
-        }
-        r.win_off = it->second;
         max_nw = std::max(max_nw, r.Nw);
-        frame0[i + 1] = frame0[i] + nfr[i];
     }
-    const Span span = place_rows(offsets, nsamp, rows);
-    const uint64_t F = frame0[n];
+    Scratch sc;
+    auto key = [](const VsFormantRow &r) { return r.Nw; };
+    ft.build(offsets, nsamp, &VsFormantRow::win_off, key, [](const VsFormantRow &r, std::vector<double> &win) {
+        for (uint32_t m = 0; m < r.Nw; m++) win.push_back(0.54 - 0.46 * std::cos(2.0 * pi * (double)m / (double)(r.Nw - 1)));
+    }, sc);
+    const uint64_t F = ft.frame0[n];
     VsFormantArgs a = {};
     a.n_rows = (uint32_t)n; a.order = op.order; a.nf = op.n_formants; a.max_nw = max_nw; a.n_frames = F; a.bmax = op.bmax_hz;
     for (uint32_t j = 0; j < op.order; j++) {
@@ -1163,31 +1206,25 @@ int vs_formant_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, c
         a.seed_im[j] = 0.9 * std::sin(t);
     }
 
-    /* scratch: rows | frame prefix | windows | per-frame found/flags | per-frame F, B | stats | frame records */
-    Scratch sc;
-    const size_t o_rows = sc.take(n * sizeof(VsFormantRow)), o_pre = sc.take((n + 1) * sizeof(uint64_t));
-    const size_t o_win = sc.take(win.size() * sizeof(double)), o_ff = sc.take(F * sizeof(uint32_t));
-    const size_t o_fb = sc.take(F * 2 * op.n_formants * sizeof(double)), o_st = sc.take(n * sizeof(vs_formant_stats));
-    const size_t o_fr = sc.take(frames ? F * sizeof(vs_formant_frame) : 0);
+    /* scratch, after the track's: per-frame found/flags | per-frame F, B | stats | frame records */
+    const size_t o_ff = sc.take(F * sizeof(uint32_t)), o_fb = sc.take(F * 2 * op.n_formants * sizeof(double));
+    const size_t o_st = sc.take(n * sizeof(vs_formant_stats)), o_fr = sc.take(frames ? F * sizeof(vs_formant_frame) : 0);
     DeviceGuard restore_device;
     PcmDev<const int16_t> d;
-    if ((rc = pcm_call_begin(ctx, pcm, span, sc.bytes, d))) return rc;
+    if ((rc = pcm_call_begin(ctx, pcm, ft.span, sc.bytes, d))) return rc;
     a.pcm = d.pcm;
-    a.rows = (const VsFormantRow *)(d.scratch + o_rows);
-    a.frame0 = (const uint64_t *)(d.scratch + o_pre);
-    a.win = (const double *)(d.scratch + o_win);
+    a.rows = (const VsFormantRow *)(d.scratch + ft.o_rows);
+    a.frame0 = (const uint64_t *)(d.scratch + ft.o_pre);
+    a.win = (const double *)(d.scratch + ft.o_tab);
     a.ff = (uint32_t *)(d.scratch + o_ff);
     a.fb = (double *)(d.scratch + o_fb);
     vs_formant_stats *d_stats = (vs_formant_stats *)(d.scratch + o_st);
     vs_formant_frame *d_frames = frames ? (vs_formant_frame *)(d.scratch + o_fr) : nullptr;
-    CU(cudaMemcpyAsync((void *)a.rows, rows.data(), n * sizeof(VsFormantRow), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.frame0, frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.win, win.data(), win.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
+    if ((rc = ft.upload(ctx, d))) return rc;
     CU(vs_launch_formants(a, d_stats, d_frames, d.st));
     CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_formant_stats), cudaMemcpyDeviceToHost, d.st));
-    /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
-    auto records = [&](size_t i) { return RowCopy{frame0[i], frame_offsets ? frame_offsets[i] : frame0[i], nfr[i]}; };
-    if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;
+    auto count = [&](size_t i) { return ft.nfr[i]; };
+    if (frames && (rc = records_home(ctx, frames, d_frames, ft.frame0.data(), frame_offsets, n, count, d.st))) return rc;
     CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are pageable host memory */
     return VS_OK;
 }
@@ -1211,10 +1248,9 @@ static int pitch_geometry(const vs_pitch_opts *in, const uint64_t *nsamp, const 
         if (!(tlo < thi)) return vs_error(err, VS_ERANGE, "stream %zu: lags %.0f..%.0f: fewer than two", i, tlo, thi);
         if (!(thi + 1.0 < nw) || nw > VS_PITCH_MAX_WIN)
             return vs_error(err, VS_ERANGE, "stream %zu: window of %.0f samples, needs %.0f..%d", i, nw, thi + 2.0, VS_PITCH_MAX_WIN);
-        if (!(hl >= 0.5 && hl < 2147483647.5)) return vs_error(err, VS_ERANGE, "stream %zu: frame step below 1 sample or above 2^31-1", i);
-        const uint64_t h = (uint64_t)std::lround(hl), w = (uint64_t)nw;
-        if (rows) rows[i] = {0, (uint32_t)w, (uint32_t)h, (uint32_t)tlo, (uint32_t)thi, 0, 0, (double)rate};
-        frames[i] = nsamp[i] >= w ? (nsamp[i] - w) / h + 1 : 0;
+        uint64_t h = 0;
+        if (const int rc = frame_step(err, i, hl, nsamp[i], (uint64_t)nw, h, frames[i])) return rc;
+        if (rows) rows[i] = {0, (uint32_t)nw, (uint32_t)h, (uint32_t)tlo, (uint32_t)thi, 0, 0, (double)rate};
         return VS_OK;
     });
 }
@@ -1226,80 +1262,60 @@ int vs_pitch_frames(const vs_pitch_opts *o, const uint64_t *nsamp, const int32_t
     return pitch_geometry(o, nsamp, fs, n, oo, nullptr, frames_out, nullptr);
 }
 
-/* the pitch track of vs_pitch_batch and vs_vowel_report_batch: the frame prefix, one table per distinct (Nw, tau_lo,
+/* the pitch track of vs_pitch_batch and vs_vowel_report_batch: the frame track with one table per distinct (Nw, tau_lo,
  * tau_hi) (host libm in double: the window w[0..Nw), then r_w(0) / r_w(tau) for tau = tau_lo-1 .. tau_hi+1, each r_w
- * summed in index order), the rows placed in the PCM, the kernels' arguments but for the device pointers, and their
- * scratch: rows | frame prefix | tables | per-frame candidates */
-struct PitchTrack {
-    std::vector<VsPitchRow> rows;
-    std::vector<uint64_t> nfr, frame0;
-    std::vector<double> tab;
-    Span span;
+ * summed in index order), the kernels' arguments but for the device pointers, and after the track's scratch the
+ * per-frame candidates */
+struct PitchTrack : FrameTrack<VsPitchRow> {
+    using FrameTrack::FrameTrack;
     VsPitchArgs a = {};
-    size_t o_rows, o_pre, o_tab, o_cand;
+    size_t o_cand = 0;
 };
 static int pitch_track(const vs_pitch_opts *o, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs, size_t n,
                        PitchTrack &p, Scratch &sc, std::string *err)
 {
     vs_pitch_opts op;
-    p.rows.resize(n);
-    p.nfr.resize(n);
     const int rc = pitch_geometry(o, nsamp, fs, n, op, p.rows.data(), p.nfr.data(), err);
     if (rc || n == 0) return rc;
-    const double pi = 3.14159265358979323846;
-    p.frame0.assign(n + 1, 0);
-    std::map<std::array<uint32_t, 3>, uint32_t> tab_at;
     uint32_t warp_doubles = 0;
-    for (size_t i = 0; i < n; i++) {
-        VsPitchRow &r = p.rows[i];
-        const auto ins = tab_at.insert({{r.Nw, r.tau_lo, r.tau_hi}, (uint32_t)p.tab.size()});
-        if (ins.second) {
-            std::vector<double> &tab = p.tab;
-            const size_t w0 = tab.size();
-            for (uint32_t m = 0; m < r.Nw; m++) tab.push_back(0.5 - 0.5 * std::cos(2.0 * pi * ((double)m + 0.5) / (double)r.Nw));
-            auto rw = [&](uint32_t tau) {
-                double s = 0.0;
-                for (uint32_t m = 0; m + tau < r.Nw; m++) s += tab[w0 + m] * tab[w0 + m + tau];
-                return s;
-            };
-            const double rw0 = rw(0);
-            for (uint32_t tau = r.tau_lo - 1; tau <= r.tau_hi + 1; tau++) tab.push_back(rw0 / rw(tau));
-        }
-        r.tab = ins.first->second;
-        warp_doubles = std::max(warp_doubles, (r.Nw + 32 + (r.tau_hi - r.tau_lo + 3) + 1) & ~1u);
-        p.frame0[i + 1] = p.frame0[i] + p.nfr[i];
-    }
-    p.span = place_rows(offsets, nsamp, p.rows);
+    for (const VsPitchRow &r : p.rows) warp_doubles = std::max(warp_doubles, (r.Nw + 32 + (r.tau_hi - r.tau_lo + 3) + 1) & ~1u);
+    auto key = [](const VsPitchRow &r) { return std::array<uint32_t, 3>{r.Nw, r.tau_lo, r.tau_hi}; };
+    p.build(offsets, nsamp, &VsPitchRow::tab, key, [](const VsPitchRow &r, std::vector<double> &tab) {
+        const size_t w0 = tab.size();
+        for (uint32_t m = 0; m < r.Nw; m++) tab.push_back(0.5 - 0.5 * std::cos(2.0 * pi * ((double)m + 0.5) / (double)r.Nw));
+        auto rw = [&](uint32_t tau) {
+            double s = 0.0;
+            for (uint32_t m = 0; m + tau < r.Nw; m++) s += tab[w0 + m] * tab[w0 + m + tau];
+            return s;
+        };
+        const double rw0 = rw(0);
+        for (uint32_t tau = r.tau_lo - 1; tau <= r.tau_hi + 1; tau++) tab.push_back(rw0 / rw(tau));
+    }, sc);
     VsPitchArgs &a = p.a;
     a.n_rows = (uint32_t)n; a.n_frames = p.frame0[n]; a.warp_doubles = warp_doubles;
     a.warps = (uint32_t)std::min<size_t>(4, (227 * 1024) / (warp_doubles * sizeof(double)));   /* the per-block cap of sm_100 */
     a.f_min = op.f_min_hz; a.voicing = op.voicing_threshold; a.silence = op.silence_threshold; a.octave_cost = op.octave_cost;
-    p.o_rows = sc.take(n * sizeof(VsPitchRow)); p.o_pre = sc.take((n + 1) * sizeof(uint64_t));
-    p.o_tab = sc.take(p.tab.size() * sizeof(double)); p.o_cand = sc.take(a.n_frames * sizeof(VsPitchCand));
+    p.o_cand = sc.take(a.n_frames * sizeof(VsPitchCand));
     return VS_OK;
 }
 
-/* points the pitch kernels' arguments into the call's scratch and uploads rows, frame prefix and tables */
+/* points the pitch kernels' arguments into the call's scratch and uploads the track */
 static int pitch_upload(vs_ctx *ctx, PitchTrack &p, const PcmDev<const int16_t> &d)
 {
-    const size_t n = p.rows.size();
     VsPitchArgs &a = p.a;
     a.pcm = d.pcm;
     a.rows = (const VsPitchRow *)(d.scratch + p.o_rows);
     a.frame0 = (const uint64_t *)(d.scratch + p.o_pre);
     a.tab = (const double *)(d.scratch + p.o_tab);
     a.cand = (VsPitchCand *)(d.scratch + p.o_cand);
-    CU(cudaMemcpyAsync((void *)a.rows, p.rows.data(), n * sizeof(VsPitchRow), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.frame0, p.frame0.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, d.st));
-    CU(cudaMemcpyAsync((void *)a.tab, p.tab.data(), p.tab.size() * sizeof(double), cudaMemcpyHostToDevice, d.st));
-    return VS_OK;
+    return p.upload(ctx, d);
 }
 
 int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, const uint64_t *nsamp, const int32_t *fs,
                    size_t n, const vs_pitch_opts *o, vs_pitch_stats *stats, vs_pitch_frame *frames, const uint64_t *frame_offsets)
 {
     if (!ctx || !pcm || !nsamp || !stats) return VS_EINVAL;
-    PitchTrack p;
+    PitchTrack p(n);
     Scratch sc;
     int rc = pitch_track(o, offsets, nsamp, fs, n, p, sc, &ctx->err);
     if (rc) return rc;
@@ -1315,9 +1331,8 @@ int vs_pitch_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offsets, con
     if ((rc = pitch_upload(ctx, p, d))) return rc;
     CU(vs_launch_pitch(p.a, d_stats, d_frames, d.st));
     CU(cudaMemcpyAsync(stats, d_stats, n * sizeof(vs_pitch_stats), cudaMemcpyDeviceToHost, d.st));
-    /* stream i's records: frame0[i] on the device, frame_offsets[i] (NULL: the same dense prefix) on the host */
-    auto records = [&](size_t i) { return RowCopy{p.frame0[i], frame_offsets ? frame_offsets[i] : p.frame0[i], p.nfr[i]}; };
-    if (frames && (rc = copy_rows_home(ctx, frames, d_frames, n, records, d.st))) return rc;
+    auto count = [&](size_t i) { return p.nfr[i]; };
+    if (frames && (rc = records_home(ctx, frames, d_frames, p.frame0.data(), frame_offsets, n, count, d.st))) return rc;
     CU(cudaStreamSynchronize(d.st));                          /* `rows` and the results are pageable host memory */
     return VS_OK;
 }
@@ -1349,7 +1364,7 @@ int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offse
                           size_t n, const vs_pitch_opts *o, vs_vowel_report *out, uint32_t *marks, const uint64_t *mark_offsets)
 {
     if (!ctx || !pcm || !nsamp || !out) return VS_EINVAL;
-    PitchTrack p;
+    PitchTrack p(n);
     Scratch sc;
     int rc = pitch_track(o, offsets, nsamp, fs, n, p, sc, &ctx->err);
     if (rc) return rc;
@@ -1359,12 +1374,12 @@ int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offse
      * period and the span of its candidates: lround(VS_MARK_STEP_MAX T) + lround(T) <= 2.25 T + 1 samples, with every
      * period a frame can publish below tau_hi + 1 */
     std::vector<VsAnalyzeRow> arows(n);
-    uint64_t slots = 0;
+    std::vector<uint64_t> slot0(n + 1, 0);
     uint32_t tau_max = 0;
     for (size_t i = 0; i < n; i++) {
         const uint64_t cap = mark_slots(nsamp[i], p.rows[i]);
-        arows[i] = {p.rows[i].off, slots, (uint32_t)nsamp[i], (uint32_t)cap, fs ? fs[i] : 22050, 0, 0};
-        slots += cap;
+        arows[i] = {p.rows[i].off, slot0[i], (uint32_t)nsamp[i], (uint32_t)cap, fs ? fs[i] : 22050, 0, 0};
+        slot0[i + 1] = slot0[i] + cap;
         tau_max = std::max(tau_max, p.rows[i].tau_hi);
     }
     const double t_hi = ((double)tau_max + 1.0) * (1.0 + 0x1p-20);
@@ -1372,7 +1387,7 @@ int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offse
 
     /* scratch, after the track's: pitch stats | frame records | report rows | mark counts | stats | marks | peaks |
      * reports | runs */
-    const uint64_t F = p.frame0[n];
+    const uint64_t F = p.frame0[n], slots = slot0[n];
     const size_t o_pst = sc.take(n * sizeof(vs_pitch_stats)), o_fr = sc.take(F * sizeof(vs_pitch_frame));
     const size_t o_rows = sc.take(n * sizeof(VsAnalyzeRow)), o_cnt = sc.take(n * sizeof(uint32_t));
     const size_t o_st = sc.take(n * sizeof(vs_flow_stats)), o_marks = sc.take(slots * sizeof(uint32_t));
@@ -1393,8 +1408,8 @@ int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offse
     CU(cudaMemcpyAsync(d.scratch + o_rows, arows.data(), n * sizeof(VsAnalyzeRow), cudaMemcpyHostToDevice, d.st));
     CU(vs_launch_pitch(p.a, (vs_pitch_stats *)(d.scratch + o_pst), (vs_pitch_frame *)(d.scratch + o_fr), d.st));
     CU(vs_launch_marks(m, d.st));
-    CU(vs_launch_report_onsets(d.pcm, m.arows, (uint32_t)n, m.marks, m.counts, (vs_flow_stats *)(d.scratch + o_st),
-                               (int32_t *)(d.scratch + o_peaks), d_rep, d.st));
+    CU(vs_launch_analyze(d.pcm, m.arows, (uint32_t)n, false, m.marks, m.counts, (vs_flow_stats *)(d.scratch + o_st),
+                         (int32_t *)(d.scratch + o_peaks), d_rep, d.st));
     /* the report and the run side by side in each 96-byte record */
     CU(cudaMemcpy2DAsync(out, sizeof(vs_vowel_report), d_rep, sizeof(vs_flow_report), sizeof(vs_flow_report), n,
                          cudaMemcpyDeviceToHost, d.st));
@@ -1402,11 +1417,8 @@ int vs_vowel_report_batch(vs_ctx *ctx, const int16_t *pcm, const uint64_t *offse
                          cudaMemcpyDeviceToHost, d.st));
     CU(cudaStreamSynchronize(d.st));                          /* the mark counts, `arows` and `out` are pageable host memory */
     if (marks) {
-        /* stream i's marks: its slots on the device, mark_offsets[i] (NULL: the same dense prefix) on the host */
-        auto rows = [&](size_t i) {
-            return RowCopy{arows[i].ons_off, mark_offsets ? mark_offsets[i] : arows[i].ons_off, std::min<uint64_t>(out[i].rep.base.onsets, arows[i].cap)};
-        };
-        if ((rc = copy_rows_home(ctx, marks, m.marks, n, rows, d.st))) return rc;
+        auto count = [&](size_t i) { return std::min<uint64_t>(out[i].rep.base.onsets, arows[i].cap); };
+        if ((rc = records_home(ctx, marks, m.marks, slot0.data(), mark_offsets, n, count, d.st))) return rc;
         CU(cudaStreamSynchronize(d.st));
     }
     return VS_OK;

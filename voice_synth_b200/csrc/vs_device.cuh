@@ -1,6 +1,7 @@
 /* vs_device.cuh -- device helpers shared by the plan kernels (vs_plan.cu) and the render kernel (vs_render.cu):
  * x86-64 conversion semantics, the constant-divisor division, glibc random() in its per-thread and
- * warp-cooperative forms, pulse / noise sample arithmetic and the reference quantiser. */
+ * warp-cooperative forms, pulse / noise sample arithmetic and the reference quantiser; and by the analysis
+ * kernels: warp reductions, the stream of a frame and the quiet NaNs. */
 #ifndef VS_DEVICE_CUH
 #define VS_DEVICE_CUH
 #include <cuda_runtime.h>
@@ -178,6 +179,65 @@ __device__ __forceinline__ int vs_round2int(double v)
     if (v > 32767.0) v = 32767.0;
     else if (v < -32767.0) v = -32767.0;
     return (int)vs_d2s(floor(v));
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * analysis kernels (vs_analyze.cu, vs_formants.cu, vs_pitch.cu, vs_marks.cu): warp reductions whose butterfly gives
+ * every lane the result, the stream of a frame, and the quiet NaN their records hold where a value is undefined
+ * ---------------------------------------------------------------------------------------------- */
+#define VS_QNAN_F __int_as_float(0x7fc00000)
+#define VS_QNAN_D __longlong_as_double(0x7ff8000000000000ll)
+
+template <class T>
+__device__ __forceinline__ T vs_warp_sum(T v)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(VS_FULL, v, o);
+    return v;
+}
+template <class T>
+__device__ __forceinline__ T vs_warp_max(T v)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(VS_FULL, v, o));
+    return v;
+}
+template <class T>
+__device__ __forceinline__ T vs_warp_min(T v)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(VS_FULL, v, o));
+    return v;
+}
+
+/* the stream of frame g: the last s with frame0[s] <= g (streams without frames have frame0[s] == frame0[s+1]) */
+__device__ __forceinline__ uint32_t vs_frame_stream(const uint64_t *frame0, uint32_t n_rows, uint64_t g)
+{
+    uint32_t lo = 0, hi = n_rows;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (frame0[mid] <= g) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+/* the launches of a frame-wise call (formants, pitch): the frame kernel, one warp per frame and `warps` of them per CTA
+ * with `smem` bytes of dynamic shared memory, when there are frames; then the stats kernel, one warp per stream in CTAs
+ * of stats_nt threads */
+template <class Args, class Stats, class Frame>
+cudaError_t vs_launch_frame_kernels(void (*frame_kernel)(Args), void (*stats_kernel)(Args, Stats *, Frame *), const Args &a,
+                                    uint32_t warps, size_t smem, uint32_t stats_nt, Stats *stats, Frame *frames, cudaStream_t s)
+{
+    if (a.n_frames) {
+        cudaError_t e = cudaFuncSetAttribute(frame_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        const uint64_t grid = (a.n_frames + warps - 1) / warps;
+        if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
+        frame_kernel<<<(unsigned)grid, 32 * warps, smem, s>>>(a);
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
+    stats_kernel<<<(a.n_rows + stats_nt / 32 - 1) / (stats_nt / 32), stats_nt, 0, s>>>(a, stats, frames);
+    return cudaGetLastError();
 }
 
 #endif

@@ -20,13 +20,6 @@
  * c[0..32] and the roots */
 __host__ __device__ inline size_t vs_fmt_warp_doubles(uint32_t max_nw) { return (size_t)max_nw + 32 + 33 + 33 + 64; }
 
-__device__ __forceinline__ double vs_fmt_warp_sum(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(VS_FULL, v, o);
-    return v;
-}
-
 /* (a + ib) / (c + id) */
 __device__ __forceinline__ void vs_cdiv(double a, double b, double c, double d, double &re, double &im)
 {
@@ -89,7 +82,7 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_frame_kernel(const __gri
 #pragma unroll
     for (int k = 0; k <= VS_FMT_MAX_ORDER; k++)
         if ((uint32_t)k <= p) {
-            const double s = vs_fmt_warp_sum(acc[k]);
+            const double s = vs_warp_sum(acc[k]);
             if (lane == 0) rr[k] = s;
         }
     __syncwarp();
@@ -104,7 +97,7 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_frame_kernel(const __gri
         double E = rr[0];
         const uint32_t j1 = (uint32_t)lane + 1;
         for (uint32_t i = 1; i <= p; i++) {
-            const double t = vs_fmt_warp_sum(j1 < i ? av * rr[i - j1] : 0.0);
+            const double t = vs_warp_sum(j1 < i ? av * rr[i - j1] : 0.0);
             const double k = -(rr[i] + t) / E;
             if (!(fabs(k) < 1.0)) { flags = VS_FRAME_SINGULAR; break; }
             const double partner = __shfl_sync(VS_FULL, av, (int)((i - j1 - 1) & 31));
@@ -186,7 +179,7 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_stats_kernel(const __gri
     if (s >= a.n_rows) return;
     const uint64_t g0 = a.frame0[s], g1 = a.frame0[s + 1];
     const uint32_t nf = a.nf;
-    const float qnan = __int_as_float(0x7fc00000);
+    const float qnan = VS_QNAN_F;
     uint32_t cnt[VS_MAX_FORMANTS], analysed = 0, unconv = 0;
     double sF[VS_MAX_FORMANTS], sB[VS_MAX_FORMANTS], sQ[VS_MAX_FORMANTS];
 #pragma unroll
@@ -216,8 +209,8 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_stats_kernel(const __gri
 #pragma unroll
     for (int k = 0; k < VS_MAX_FORMANTS; k++) {
         cnt[k] = __reduce_add_sync(VS_FULL, cnt[k]);
-        sF[k] = vs_fmt_warp_sum(sF[k]);
-        sB[k] = vs_fmt_warp_sum(sB[k]);
+        sF[k] = vs_warp_sum(sF[k]);
+        sB[k] = vs_warp_sum(sB[k]);
         mF[k] = cnt[k] ? sF[k] / (double)cnt[k] : 0.0;
     }
     analysed = __reduce_add_sync(VS_FULL, analysed);
@@ -230,7 +223,7 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_stats_kernel(const __gri
             if (!fl && (uint32_t)k < found) { const double d = fb[k] - mF[k]; sQ[k] += d * d; }
     }
 #pragma unroll
-    for (int k = 0; k < VS_MAX_FORMANTS; k++) sQ[k] = vs_fmt_warp_sum(sQ[k]);
+    for (int k = 0; k < VS_MAX_FORMANTS; k++) sQ[k] = vs_warp_sum(sQ[k]);
     if (lane == 0) {
         vs_formant_stats st;
         st.frames = (uint32_t)(g1 - g0);
@@ -250,15 +243,6 @@ __global__ void __launch_bounds__(VS_FMT_NT) vs_formant_stats_kernel(const __gri
 
 cudaError_t vs_launch_formants(const VsFormantArgs &a, vs_formant_stats *stats, vs_formant_frame *frames, cudaStream_t s)
 {
-    if (a.n_frames) {
-        const size_t smem = (VS_FMT_NT / 32) * vs_fmt_warp_doubles(a.max_nw) * sizeof(double);
-        cudaError_t e = cudaFuncSetAttribute(vs_formant_frame_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        const uint64_t grid = (a.n_frames + VS_FMT_NT / 32 - 1) / (VS_FMT_NT / 32);
-        if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-        vs_formant_frame_kernel<<<(unsigned)grid, VS_FMT_NT, smem, s>>>(a);
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    }
-    vs_formant_stats_kernel<<<(a.n_rows + VS_FMT_NT / 32 - 1) / (VS_FMT_NT / 32), VS_FMT_NT, 0, s>>>(a, stats, frames);
-    return cudaGetLastError();
+    const size_t smem = (VS_FMT_NT / 32) * vs_fmt_warp_doubles(a.max_nw) * sizeof(double);
+    return vs_launch_frame_kernels(vs_formant_frame_kernel, vs_formant_stats_kernel, a, VS_FMT_NT / 32, smem, VS_FMT_NT, stats, frames, s);
 }

@@ -44,8 +44,7 @@ __global__ void __launch_bounds__(VS_MARK_NT) vs_marks_kernel(const __grid_const
         if (v) best = max(best, ((uint64_t)len << 32) | (uint32_t)~f);
         cur = __shfl_sync(VS_FULL, len, 31);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) best = max(best, (uint64_t)__shfl_xor_sync(VS_FULL, (unsigned long long)best, o));
+    best = vs_warp_max(best);
     if (best == 0) {
         if (lane == 0) { a.counts[s] = 0; a.run[s] = VsMarkRun{0, 0, 0, 0}; }
         return;
@@ -72,8 +71,7 @@ __global__ void __launch_bounds__(VS_MARK_NT) vs_marks_kernel(const __grid_const
         const uint64_t a0 = c - L / 2;
         uint64_t key = 0;                                     /* |x| << 32 | ~j: the largest, then the first */
         for (uint32_t j = (uint32_t)lane; j < L; j += 32) key = max(key, ((uint64_t)abs((int)x[a0 + j]) << 32) | (uint32_t)~j);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) key = max(key, (uint64_t)__shfl_xor_sync(VS_FULL, (unsigned long long)key, o));
+        key = vs_warp_max(key);
         m = a0 + ~(uint32_t)key;
     }
 
@@ -93,9 +91,7 @@ __global__ void __launch_bounds__(VS_MARK_NT) vs_marks_kernel(const __grid_const
 
         long long e0 = 0;
         for (uint32_t j = (uint32_t)lane; j < (uint32_t)L; j += 32) { const int v = xs[j]; e0 += v * v; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) e0 += __shfl_xor_sync(VS_FULL, e0, o);
-        const double de0 = (double)e0;
+        const double de0 = (double)vs_warp_sum(e0);
 
         /* candidates d = m' - m_k, ascending per lane: a strict > keeps the smaller d of a tie */
         double br = -__longlong_as_double(0x7ff0000000000000ll);

@@ -16,25 +16,6 @@
 #define VS_PITCH_NT   128        /* threads per CTA of the stats kernel, and most of the frame kernel's    */
 #define VS_PITCH_KMAX 13         /* most lags per lane and pass (odd: see vs_pitch_lags)                   */
 
-__device__ __forceinline__ double vs_pitch_warp_sum(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(VS_FULL, v, o);
-    return v;
-}
-__device__ __forceinline__ double vs_pitch_warp_max(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(VS_FULL, v, o));
-    return v;
-}
-__device__ __forceinline__ double vs_pitch_warp_min(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(VS_FULL, v, o));
-    return v;
-}
-
 /* r_a(tau) for tau = t_first .. t_end-1 into rr[tau - t_first].  Lane l of a pass owns the K lags tl = t0 + l K ..
  * tl + K - 1 and walks m: per step one broadcast load of y[m] and one load of y[m + tl + K - 1] into a ring of K
  * registers feed K FMAs.  The ring index is a compile-time constant because the loop over m is unrolled K times.
@@ -72,14 +53,9 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_frame_kernel(const __gri
     const uint64_t g = (uint64_t)blockIdx.x * a.warps + (uint64_t)warp;
     if (g >= a.n_frames) return;
 
-    /* the stream: the last s with frame0[s] <= g (streams without frames have frame0[s] == frame0[s+1]) */
-    uint32_t lo = 0, hi = a.n_rows;
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (a.frame0[mid] <= g) lo = mid; else hi = mid;
-    }
-    const VsPitchRow r = a.rows[lo];
-    const int16_t *x = a.pcm + r.off + (g - a.frame0[lo]) * (uint64_t)r.H;
+    const uint32_t sid = vs_frame_stream(a.frame0, a.n_rows, g);
+    const VsPitchRow r = a.rows[sid];
+    const int16_t *x = a.pcm + r.off + (g - a.frame0[sid]) * (uint64_t)r.H;
     const uint32_t Nw = r.Nw, L = r.tau_hi - r.tau_lo + 3;
     const double *w = a.tab + r.tab, *cw = w + Nw;
     double *y = vs_pitch_smem + (size_t)warp * a.warp_doubles;
@@ -100,11 +76,10 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_frame_kernel(const __gri
         }
         y[m] = v;
     }
-    peak = vs_pitch_warp_max(peak);
-    e = vs_pitch_warp_sum(e);                                 /* the butterfly gives every lane the same sum */
-    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    peak = vs_warp_max(peak);
+    e = vs_warp_sum(e);                                       /* the butterfly gives every lane the same sum */
     if (e == 0.0) {
-        if (lane == 0) a.cand[g] = VsPitchCand{qnan, qnan, peak, VS_PITCH_SILENT, 0u};
+        if (lane == 0) a.cand[g] = VsPitchCand{VS_QNAN_D, VS_QNAN_D, peak, VS_PITCH_SILENT, 0u};
         return;
     }
     __syncwarp();
@@ -127,7 +102,7 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_frame_kernel(const __gri
     __syncwarp();
 
     /* candidates, lanes along tau in ascending order (a strict > keeps the smaller tau of a tie), then a warp argmax */
-    double bS = -__longlong_as_double(0x7ff0000000000000ll), bt = qnan, br = qnan;
+    double bS = -__longlong_as_double(0x7ff0000000000000ll), bt = VS_QNAN_D, br = VS_QNAN_D;
     uint32_t bi = 0xffffffffu;
     for (uint32_t t = r.tau_lo + (uint32_t)lane; t <= r.tau_hi; t += 32) {
         const uint32_t i = t - r.tau_lo + 1;
@@ -172,10 +147,10 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_stats_kernel(const __gri
     if (s >= a.n_rows) return;
     const uint64_t g0 = a.frame0[s], g1 = a.frame0[s + 1];
     const double fs = a.rows[s].fs;
-    const float qnan = __int_as_float(0x7fc00000);
+    const float qnan = VS_QNAN_F;
     double G = 0.0;
     for (uint64_t g = g0 + (uint64_t)lane; g < g1; g += 32) G = fmax(G, a.cand[g].peak);
-    const double quiet = a.silence * vs_pitch_warp_max(G);
+    const double quiet = a.silence * vs_warp_max(G);
 
     uint32_t periodic = 0, voiced = 0;
     double sf = 0.0, sh = 0.0, sr = 0.0, lo = __longlong_as_double(0x7ff0000000000000ll), hi = -lo;
@@ -196,11 +171,11 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_stats_kernel(const __gri
     }
     periodic = __reduce_add_sync(VS_FULL, periodic);
     voiced = __reduce_add_sync(VS_FULL, voiced);
-    sf = vs_pitch_warp_sum(sf);
-    sh = vs_pitch_warp_sum(sh);
-    sr = vs_pitch_warp_sum(sr);
-    lo = vs_pitch_warp_min(lo);
-    hi = vs_pitch_warp_max(hi);
+    sf = vs_warp_sum(sf);
+    sh = vs_warp_sum(sh);
+    sr = vs_warp_sum(sr);
+    lo = vs_warp_min(lo);
+    hi = vs_warp_max(hi);
     const double mf = voiced ? sf / (double)voiced : 0.0, mh = periodic ? sh / (double)periodic : 0.0;
     double qf = 0.0, qh = 0.0;
     for (uint64_t g = g0 + (uint64_t)lane; g < g1; g += 32) {
@@ -210,8 +185,8 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_stats_kernel(const __gri
         if (!fl || fl == VS_PITCH_VOICED) { const double d = hnr - mh; qh += d * d; }
         if (fl == VS_PITCH_VOICED) { const double d = f0 - mf; qf += d * d; }
     }
-    qf = vs_pitch_warp_sum(qf);
-    qh = vs_pitch_warp_sum(qh);
+    qf = vs_warp_sum(qf);
+    qh = vs_warp_sum(qh);
     if (lane == 0) {
         vs_pitch_stats st;
         st.frames = (uint32_t)(g1 - g0);
@@ -231,15 +206,6 @@ __global__ void __launch_bounds__(VS_PITCH_NT) vs_pitch_stats_kernel(const __gri
 
 cudaError_t vs_launch_pitch(const VsPitchArgs &a, vs_pitch_stats *stats, vs_pitch_frame *frames, cudaStream_t s)
 {
-    if (a.n_frames) {
-        const size_t smem = (size_t)a.warps * a.warp_doubles * sizeof(double);
-        cudaError_t e = cudaFuncSetAttribute(vs_pitch_frame_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        const uint64_t grid = (a.n_frames + a.warps - 1) / a.warps;
-        if (grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-        vs_pitch_frame_kernel<<<(unsigned)grid, 32 * a.warps, smem, s>>>(a);
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    }
-    vs_pitch_stats_kernel<<<(a.n_rows + VS_PITCH_NT / 32 - 1) / (VS_PITCH_NT / 32), VS_PITCH_NT, 0, s>>>(a, stats, frames);
-    return cudaGetLastError();
+    const size_t smem = (size_t)a.warps * a.warp_doubles * sizeof(double);
+    return vs_launch_frame_kernels(vs_pitch_frame_kernel, vs_pitch_stats_kernel, a, a.warps, smem, VS_PITCH_NT, stats, frames, s);
 }
